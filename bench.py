@@ -13,7 +13,11 @@ them: `generate` (configs[2]: `NeuralMarionette.generate`, clips sharded over th
 D-FAUST-shape training step - fwd + bwd + Adam - data-parallel with the NCCL gradient all-reduce over NVLink).
 `--workload generate|train` makes one of them the headline of the line instead.
 
+`--dump-outputs DIR` writes what the headline's last timed step returned (rank 0's clips) as DIR/<name>.npy: inputs,
+weights and the roll-out noise are seeded, so two builds run with the same arguments can be compared array for array.
+
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload detector|generate|train]
+                    [--dump-outputs DIR]
 """
 from __future__ import annotations
 
@@ -34,6 +38,7 @@ sys.path.insert(0, ROOT)
 # algorithmic conv FLOPs (2*MAC) at G = 64, SURVEY.md §8(d) / BASELINE.md §5
 GF_ENC_FRAME, GF_ST_CLIP, GF_DEC_FRAME = 27.848, 93.815, 65.434
 METRIC = "voxel frames/sec keypoint detection"
+DUMP_BYTES = 64 << 20
 
 
 def parse():
@@ -53,7 +58,14 @@ def parse():
     ap.add_argument("--workload", default="detector", choices=["detector", "generate", "train"],
                     help="detector = configs[1] (default, the headline); generate = configs[2] shape "
                          "(NeuralMarionette.generate); train = configs[3] shape (training step, T = 10, 24 clips per GPU)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the arrays the headline's last timed step returned to DIR/<name>.npy (float32 / float64, "
+                         f"at most {DUMP_BYTES >> 20} MB in all; larger outputs as a fixed, seeded sample of their elements)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs is not None and a.impl == "reference":
+        ap.error("--dump-outputs writes the GPU arm's outputs; it does not apply to --impl reference")
     train = a.workload == "train"
     a.clips = a.clips if a.clips is not None else (24 if train else 64)
     a.frames = a.frames if a.frames is not None else (10 if train else 20)
@@ -134,6 +146,32 @@ def synthetic_raw(seed0, B, T, N):
     for b in range(B):       # 8 distinct clips, re-posed by a random rigid offset/scale: distinct occupancy per clip
         out[b] = base[b % len(base)] * np.float32(rng.uniform(0.8, 1.2)) + rng.uniform(-0.2, 0.2, size=3).astype(np.float32)
     return out
+
+
+def sample_outputs(out: dict) -> dict:
+    """The tensors of a step's result as host arrays (float64 stays float64 and integers become float64, everything else
+    float32), DUMP_BYTES at most in all.  An array larger than its equal share of that budget keeps a seeded choice of
+    its elements, flattened: the same positions for the same shape, so that two builds compare element for element.
+    name -> (full shape, array)."""
+    tensors = {k: v.detach() for k, v in sorted(out.items()) if isinstance(v, torch.Tensor)}
+    share = DUMP_BYTES // (8 * max(1, len(tensors)))
+    res = {}
+    for name, t in tensors.items():
+        wide = t.dtype == torch.float64 or not (t.dtype.is_floating_point or t.dtype == torch.bool)
+        a = t.to(torch.float64 if wide else torch.float32)
+        if a.numel() > share:
+            pick = np.sort(np.random.default_rng(0).choice(a.numel(), share, replace=False))
+            a = a.reshape(-1)[torch.from_numpy(pick).to(a.device)]
+        res[name] = (list(t.shape), a.cpu().numpy())
+    return res
+
+
+def write_outputs(path: str, arrays: dict) -> dict:
+    os.makedirs(path, exist_ok=True)
+    for name, (_, a) in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), a)
+    return {"dir": os.path.abspath(path),
+            "arrays": {name: {"shape": shape, "saved": int(a.size)} for name, (shape, a) in arrays.items()}}
 
 
 # ------------------------------------------------------------------ the CPU arm
@@ -227,7 +265,7 @@ def reference_arm(args):
     """`--impl reference`: the reference's CPU implementation of the workload on this box's host cores.  The line reports
     exactly what ran: `steps` / `warmup` executed and the ONE-clip sample each step processes."""
     frames = max(2, args.cpu_baseline_frames)
-    steps, warmup = max(1, min(args.steps, 6)), max(1, min(args.warmup, 2))
+    steps, warmup = args.steps, max(1, min(args.warmup, 2))
     fps, t, cores, kind = cpu_reference_run(args, steps, warmup, frames)
     what = {"detector": "KyptDetector.forward", "generate": "NeuralMarionette.generate",
             "train": "KyptDetector fwd + bwd + Adam"}[args.workload]
@@ -288,6 +326,7 @@ class Bench:
         self.world = int(os.environ.get("WORLD_SIZE", 1))
         self.local = int(os.environ.get("LOCAL_RANK", 0))
         assert torch.cuda.is_available(), "bench.py needs a GPU (no CPU fallback); use --impl reference for the CPU arm"
+        torch.manual_seed(0)                # the roll-out noise of `generate`: the same every run
         torch.cuda.set_device(self.local)
         self.dev = torch.device("cuda", self.local)
         if self.world > 1:
@@ -304,19 +343,23 @@ class Bench:
         net.anneal(1)
         return net, hp
 
-    def timed(self, fn, steps):
+    def timed(self, fn, steps, keep_last=False):
+        """Device time per call of `fn` over `steps` calls (slowest rank); with keep_last, (time, what the last call
+        returned)."""
         from neural_marionette_b200.parallel import barrier, max_over_ranks
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        for _ in range(steps):
+        for _ in range(steps - 1):
             fn()
+        last = fn()
         e1.record()
         barrier()
-        return max_over_ranks(e0.elapsed_time(e1), self.dev) / steps      # device time, slowest rank
+        ms = max_over_ranks(e0.elapsed_time(e1), self.dev) / steps      # device time, slowest rank
+        return (ms, last) if keep_last else ms
 
     # ---- configs[1] / configs[2]: inference
-    def run_inference(self, workload, B, T, N, steps, warmup, want_roofline):
+    def run_inference(self, workload, B, T, N, steps, warmup, want_roofline, keep_outputs=False):
         ops, G, dev = self.ops, self.G, self.dev
         net, hp = self.model()
         net.eval()
@@ -350,10 +393,12 @@ class Bench:
             sampler.start()
             calls0 = self.lib.CALLS
             ops.PROFILE = {} if want_roofline else None
-            ms = self.timed(step_resident, steps)
+            ms, out = self.timed(step_resident, steps, keep_last=True)
             prof, ops.PROFILE = ops.PROFILE, None
             res["launches"] = self.lib.CALLS - calls0
             res["clocks"] = sampler.result()
+            res["outputs"] = sample_outputs(out) if keep_outputs else None
+            del out
             step_e2e()
             ms_e2e = self.timed(step_e2e, steps)
             if workload == "detector" and want_roofline:
@@ -378,7 +423,7 @@ class Bench:
         return res
 
     # ---- configs[3]: the training step
-    def run_train(self, B, T, N, steps, warmup):
+    def run_train(self, B, T, N, steps, warmup, keep_outputs=False):
         """fwd + bwd of the stage-1 loss sum (train.py:173-181 weights) + Adam (train.py:380-409) on B clips x T frames
         per GPU (dataset/config.py:4-12: T = 10, batch 24); gradients all-reduced over the ranks in 4 buckets launched
         from the backward (parallel.GradientBuckets, NCCL)."""
@@ -416,10 +461,12 @@ class Bench:
         sampler = ClockSampler(self.local)
         sampler.start()
         calls0 = self.lib.CALLS
-        ms = self.timed(lambda: step(raw_dev), steps)
+        ms, out = self.timed(lambda: step(raw_dev), steps, keep_last=True)
         launches = self.lib.CALLS - calls0
         clocks = sampler.result()
         torch.cuda.synchronize()
+        outputs = sample_outputs(out) if keep_outputs else None
+        del out
         # per-launch CUDA events of the tensor-core convs / weight gradients over two more steps (kept out of `ms`)
         ops.PROFILE = {}
         prof_ms = self.timed(lambda: step(raw_dev), 2)
@@ -462,7 +509,7 @@ class Bench:
                    h2d=int(raw_host.numel() * 4), d2h=4, launches=launches,
                    grad_bytes=int(opt.buckets.flat.numel() * 4), buckets=len(opt.buckets.bounds), exposed_ms=exposed,
                    allreduce_alone_ms=ar_ms, skipped=opt.skipped, peak_gib=torch.cuda.max_memory_allocated() / 2 ** 30,
-                   grad_scale=ops.grad_scale(), clocks=clocks, prof=prof, prof_ms=prof_ms)
+                   grad_scale=ops.grad_scale(), clocks=clocks, prof=prof, prof_ms=prof_ms, outputs=outputs)
         if G == 64:   # training ~ 3x the forward's conv FLOPs (fwd + dgrad + wgrad)
             res["model_tflops"] = 3 * self.world * B * (GF_ST_CLIP + T * (GF_ENC_FRAME + GF_DEC_FRAME)) / (ms / 1e3) / 1e3
         del net, opt
@@ -543,8 +590,9 @@ def main():
     line = {"metric": METRIC, "unit": "frames/s", "n_gpus": world, "steps": steps, "warmup": warmup,
             "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "fp16", "data": "synthetic",
             "config": config}
+    dump = args.dump_outputs is not None
     if args.workload == "train":
-        r = be.run_train(B, T, N, steps, warmup)
+        r = be.run_train(B, T, N, steps, warmup, keep_outputs=dump)
         rec = be.train_record(r, B, T)
         be.training_profile = True
         line.update(value=r["value"], ms_per_step=r["ms"], e2e=rec["e2e"], gpu_launches=int(r["launches"]),
@@ -552,7 +600,7 @@ def main():
                     clocks=r["clocks"])
         line["e2e"]["note"] = "host points -> device every step; the step's loss read back"
     else:
-        r = be.run_inference(args.workload, B, T, N, steps, warmup, want_roofline=True)
+        r = be.run_inference(args.workload, B, T, N, steps, warmup, want_roofline=True, keep_outputs=dump)
         line.update(value=r["value"], ms_per_step=r["ms"], clocks=r["clocks"],
                     e2e={"value": r["e2e"], "unit": "frames/s", "h2d_bytes_per_step": r["h2d"], "d2h_bytes_per_step": r["d2h"],
                          "ms_per_step": r["ms_e2e"],
@@ -580,6 +628,8 @@ def main():
         line["cpu_baseline"] = {"value": fps, "unit": "frames/s", "cores": cores, "kind": kind,
                                 "sample": f"1 clip x {args.cpu_baseline_frames} frames (voxelize + {args.workload}), "
                                           f"1 warm-up + 2 timed reps of {t:.1f} s; same per-frame work as the GPU arm"}
+    if rank == 0 and dump:
+        line["outputs"] = write_outputs(args.dump_outputs, r["outputs"])
     if rank == 0:
         print(json.dumps(line))
     if world > 1:

@@ -392,6 +392,8 @@ class KyptDetector(nn.Module):
             first_feature=det["first_feature"])
 
     def forward(self, seq, Tcond=None):
+        if not seq.is_cuda:
+            raise ops.L.NmError("KyptDetector needs CUDA tensors (there is no CPU fallback)")
         if _training(self):
             return self.forward_train(seq)
         B, T = seq.shape[:2]
