@@ -612,11 +612,18 @@ constexpr int kSlab3XformWarps = 6;   // max extra warps (only launched when the
 constexpr int kLoRing = 4;
 constexpr int kLoRows = 10 * 6;              // low-resolution box: 10 (h) x 6 (w) rows of 64 channels
 constexpr int kLoBytes = kLoRows * 128;      // 7680
+constexpr int kUpWarps = 4;                  // up-sampling producer warps launched (3 working)
 
 // ACC: split-K second launch - the epilogue adds the partial sum already in `out`.
-template <int BK, int PN, bool UP = false, bool ACC = false>
+// DEPI (with UP): the depth part of the up-sampling is applied to the accumulators instead of the operand.  Everything
+// after the input transform is linear and trilinear x2 is separable, so the producer builds one halo slice per
+// LOW-resolution plane (h / w interpolation only), the MMAs run over D/2 slices, and the epilogue forms every output
+// slice as a fixed combination of the TMEM groups P(i-1), P(i), P(i+1) (coefficients at the epilogue).  Half the MMAs,
+// half the operand traffic; the depth border (clamp + zero padding) stays exact and is blended in fp32.
+template <int BK, int PN, bool UP = false, bool ACC = false, bool DEPI = false>
 __global__ void __launch_bounds__(kSlab3Threads + 32 * kSlab3XformWarps, 1)
 conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
+  static_assert(!DEPI || (UP && PN == 32), "the depth epilogue belongs to the up-sampling variant");
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
   constexpr int w_tile_bytes = PN * BK * 2;                            // one (tap, k-chunk)
@@ -640,6 +647,7 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
   float* s_ab = reinterpret_cast<float*>(tmem_slot + 4);   // [2][Cin] scale | shift of the current sample
   const bool xform = UP || p.in_scale != nullptr;
   const int nxw = ((int)blockDim.x - kSlab3Threads) >> 5;   // transform / producer warps launched (0, 4 or 6)
+  const int n_sl = DEPI ? p.D >> 1 : p.D;                   // operand slices (= TMEM groups) per column
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int n_cols = p.N * p.nh * p.nw;
@@ -681,7 +689,7 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
     // 16-byte channel chunk c): 24 plane loads -> depth + h blends for the 6 box columns -> the 10 halo columns of
     // that row, written at the TMA-128B-swizzle position.  Rows / columns outside the tensor are the conv's zero
     // padding.  With a fused prologue the producer's GroupNorm scale/shift (+LeakyReLU) is applied to each plane
-    // in place when it lands.
+    // in place when it lands.  DEPI: operand slice d is low-res plane d blended in h and w only (near = far = d).
     const int tid = threadIdx.x - 32 * (2 + kSlab3EpiWarps);
     const bool fused = p.in_scale != nullptr;
     const int Dl = p.D >> 1, Hl = p.H >> 1;
@@ -732,8 +740,8 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
         cur_n = n;
       }
       int landed = 0;                                     // planes of this column already waited for
-      for (int d = 0; d < p.D; d++, fill++) {
-        const int pn = d >> 1, pf = min(max(pn + ((d & 1) ? 1 : -1), 0), Dl - 1);
+      for (int d = 0; d < n_sl; d++, fill++) {
+        const int pn = DEPI ? d : d >> 1, pf = DEPI ? d : min(max(pn + ((d & 1) ? 1 : -1), 0), Dl - 1);
         const int need = max(pn, pf);
         while (landed <= need) {
           const uint32_t g = planes + landed;
@@ -792,8 +800,13 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
             uint4 va[NW], vb[NW];                                    // depth-blended low-res rows m and m+1
 #pragma unroll
             for (int w = 0; w < NW; w++) {
-              va[w] = lerp(lds128(lo_n + oa + (W0 + w) * 128), lds128(lo_f + oa + (W0 + w) * 128));
-              vb[w] = lerp(lds128(lo_n + ob + (W0 + w) * 128), lds128(lo_f + ob + (W0 + w) * 128));
+              if constexpr (DEPI) {
+                va[w] = lds128(lo_n + oa + (W0 + w) * 128);
+                vb[w] = lds128(lo_n + ob + (W0 + w) * 128);
+              } else {
+                va[w] = lerp(lds128(lo_n + oa + (W0 + w) * 128), lds128(lo_f + oa + (W0 + w) * 128));
+                vb[w] = lerp(lds128(lo_n + ob + (W0 + w) * 128), lds128(lo_f + ob + (W0 + w) * 128));
+              }
             }
 #pragma unroll
             for (int r2 = 0; r2 < 2; r2++) {
@@ -836,9 +849,13 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
         __syncwarp();
         if (lane == 0) {
           mbar_arrive(&ready[slot]);
-          // plane x is last read by slice min(2x + 2, D - 1)
-          if (d >= 2 && !(d & 1)) mbar_arrive(&empty_lo[(planes + ((d - 2) >> 1)) % kLoRing]);
-          if (d == p.D - 1) mbar_arrive(&empty_lo[(planes + Dl - 1) % kLoRing]);
+          if (DEPI) {
+            mbar_arrive(&empty_lo[(planes + d) % kLoRing]);
+          } else {
+            // plane x is last read by slice min(2x + 2, D - 1)
+            if (d >= 2 && !(d & 1)) mbar_arrive(&empty_lo[(planes + ((d - 2) >> 1)) % kLoRing]);
+            if (d == p.D - 1) mbar_arrive(&empty_lo[(planes + Dl - 1) % kLoRing]);
+          }
         }
       }
     }
@@ -975,7 +992,7 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
       mbar_wait(wfull, 0);
       uint32_t q = 0;                                    // global slice counter (ring + P-group position)
       for (int col = col0; col < n_cols; col += col_step) {
-        for (int sl = 0; sl < p.D; sl++, q++) {
+        for (int sl = 0; sl < n_sl; sl++, q++) {
           mbar_wait(&ready[q % ring], (q / ring) & 1);
           mbar_wait(&pempty[q % kPGroups], ((q / kPGroups) & 1) ^ 1);
           tc_fence_after();
@@ -1067,12 +1084,21 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
     const int row = quad * 32 + lane;
     const uint32_t lane_addr = ((uint32_t)(quad * 32) << 16) + (uint32_t)(chalf * CW);
     float bias[CW];
+    // DEPI: the bias is read from shared memory (broadcast), which keeps that epilogue within 128 registers; it sits
+    // behind the scale / shift (UP: Cin = 64, well inside the 2 x 256 floats reserved for them)
+    float* s_bias = s_ab + 2 * p.cin;
+    if constexpr (DEPI) {
+      const int e = threadIdx.x - 64;
+      if (e < PN) s_bias[e] = (p.bias && part * PN + e < p.cout) ? __ldg(p.bias + part * PN + e) : 0.f;
+      named_bar_sync(1, 32 * kSlab3EpiWarps);
+    } else {
 #pragma unroll
-    for (int j = 0; j < CW; j++) {
-      const int ch = part * PN + chalf * CW + j;
-      bias[j] = (p.bias && ch < p.cout) ? __ldg(p.bias + ch) : 0.f;
+      for (int j = 0; j < CW; j++) {
+        const int ch = part * PN + chalf * CW + j;
+        bias[j] = (p.bias && ch < p.cout) ? __ldg(p.bias + ch) : 0.f;
+      }
     }
-    uint32_t q0 = 0;                                     // global index of slice 0 of the current column
+    uint32_t q0 = 0;                                    // global index of slice 0 of the current column
     uint32_t n_out = 0;                                  // output tiles staged so far (staging buffer parity)
     const bool is_issuer = warp == 2 && lane == 0;       // the thread that owns the TMA-store bulk groups
     // this thread's 16-byte chunks in the staging tile (swizzled like the store tensor map): constant per thread
@@ -1084,7 +1110,7 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
       st_off[c8] = off ^ (((off >> 7) & (row_b == 64 ? 3u : 1u)) << 4);
     }
     const uint32_t s_out_u32 = smem_u32(s_out);
-    for (int col = col0; col < n_cols; col += col_step, q0 += p.D) {
+    for (int col = col0; col < n_cols; col += col_step, q0 += n_sl) {
       int t = col;
       const int iw = t % p.nw; t /= p.nw;
       const int ih = t % p.nh; t /= p.nh;
@@ -1100,23 +1126,24 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
       // touched 16 cache lines per warp instruction and ran at ~1 TB/s)
       // split-K second launch: the partial sum the first launch left in `out` (fp16) is added; its loads are issued
       // one output slice ahead
-      uint4 pvq[ACC ? CW / 8 : 1];
-      auto load_prev = [&](int od) {
+      using PrevT = uint4[ACC ? CW / 8 : 1];
+      PrevT pvq, pvq1;
+      auto load_prev = [&](PrevT& pv, int od) {
         const act_t* prev = p.out + ((((long long)n * p.D + od) * p.H + ih * 16 + (row >> 3)) * p.W + iw * 8 + (row & 7)) * p.cout +
                             part * PN + chalf * CW;
 #pragma unroll
-        for (int c8 = 0; c8 < (ACC ? CW / 8 : 0); c8++) pvq[c8] = *reinterpret_cast<const uint4*>(prev + c8 * 8);
+        for (int c8 = 0; c8 < (ACC ? CW / 8 : 0); c8++) pv[c8] = *reinterpret_cast<const uint4*>(prev + c8 * 8);
       };
-      auto emit = [&](float (&f)[CW], int od) {
+      auto emit = [&](float (&f)[CW], int od, const PrevT& pv) {
         if constexpr (ACC) {
 #pragma unroll
           for (int c8 = 0; c8 < CW / 8; c8++) {
-            float pv[8];
-            nm_unpack8(*reinterpret_cast<const half8*>(&pvq[c8]), pv);
+            float pf[8];
+            nm_unpack8(*reinterpret_cast<const half8*>(&pv[c8]), pf);
 #pragma unroll
-            for (int k = 0; k < 8; k++) f[c8 * 8 + k] += pv[k];
+            for (int k = 0; k < 8; k++) f[c8 * 8 + k] += pf[k];
           }
-          if (od + 1 < p.D) load_prev(od + 1);           // for the next output slice: a whole slice period ahead
+          if (!DEPI && od + 1 < p.D) load_prev(pvq, od + 1);   // for the next output slice: a whole slice period ahead
         }
 #pragma unroll
         for (int c = 0; c < CW; c++) { ssum[c] += f[c]; ssq[c] = fmaf(f[c], f[c], ssq[c]); }
@@ -1136,50 +1163,131 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
         }
         n_out++;
       };
-      if (ACC) load_prev(0);
-      for (int sl = 0; sl < p.D; sl++) {
-        const uint32_t q = q0 + sl;
-        // with producer warps in the CTA the eight epilogue warps back off between polls (isolated launch of the
-        // fused 32->32 layer: 5.97 -> 5.12 ms; inside the full step the effect is within run-to-run noise)
-        if (xform) mbar_wait_backoff(&pfull[q % kPGroups], (q / kPGroups) & 1, 100u);
-        else mbar_wait(&pfull[q % kPGroups], (q / kPGroups) & 1);
-        tc_fence_after();
-        const uint32_t g_cur = lane_addr + (q % kPGroups) * (3 * PN);
-        const uint32_t g_prev = lane_addr + ((q + kPGroups - 1) % kPGroups) * (3 * PN);
-        uint32_t ra[CW], rb[CW], rc[CW];
-        if (sl >= 1 && !(p.debug & 24)) {
-          if constexpr (CW == 16) { tmem_ld16(g_cur + 2 * PN, ra); tmem_ld16(g_prev, rc); }
-          else { tmem_ld8(g_cur + 2 * PN, ra); tmem_ld8(g_prev, rc); }
-        } else {
+      if constexpr (DEPI) {
+        // Event s = "group P(s) complete", P(s)[kd] = W(kd) x(s) with x(s) = low-res plane s up-sampled in h and w.  The
+        // depth-up-sampled input is h(2i) = 0.75 x(i) + 0.25 x(max(i-1, 0)), h(2i+1) = 0.75 x(i) + 0.25 x(min(i+1, Dl-1)),
+        // h(-1) = h(2 Dl) = 0 (conv padding), and out(m) = sum_kd W(kd) h(m+kd-1):
+        //   out(2i)   = 0.75 P(i-1)[0] + 0.25 P(i)[0] + 0.25 P(i-1)[1] + 0.75 P(i)[1] + 0.75 P(i)[2] + 0.25 P(i+1)[2]
+        //   out(2i+1) = 0.25 P(i-1)[0] + 0.75 P(i)[0] + 0.75 P(i)[1] + 0.25 P(i+1)[1] + 0.25 P(i)[2] + 0.75 P(i+1)[2]
+        // At the first and last slice the clamp and the zero padding only change coefficients.  Event s adds the P(s)
+        // terms of pair s-1 and emits it, then starts pair s from P(s-1) and P(s) (P(s-1) is dead after that) and, at
+        // the last slice, emits it too.  TMEM blocks are loaded two at a time: the register budget of the 8 warps.
+        static_assert(CW == 16, "DEPI epilogue: 16 columns per warp");
+        float part0[CW], part1[CW];                      // out(2i), out(2i+1) of the pair in flight
+        for (int s = 0; s < n_sl; s++) {
+          const uint32_t q = q0 + s;
+          const bool first = s == 0, last = s == n_sl - 1;
+          if (ACC && !first) { load_prev(pvq, 2 * s - 2); load_prev(pvq1, 2 * s - 1); }   // in flight during the wait
+          mbar_wait_backoff(&pfull[q % kPGroups], (q / kPGroups) & 1, 100u);
+          tc_fence_after();
+          const uint32_t g_cur = lane_addr + (q % kPGroups) * (3 * PN);
+          const uint32_t g_prev = lane_addr + ((q + kPGroups - 1) % kPGroups) * (3 * PN);
+          uint32_t ra[CW], rb[CW];
+          if (!first) {
+            tmem_ld16(g_cur + PN, ra);
+            tmem_ld16(g_cur + 2 * PN, rb);
+            tmem_ld_wait();
 #pragma unroll
-          for (int c = 0; c < CW; c++) { ra[c] = 0u; rc[c] = 0u; }
-        }
-        if (!(p.debug & 8)) {
-          if constexpr (CW == 16) tmem_ld16(g_cur + PN, rb);
-          else tmem_ld8(g_cur + PN, rb);
-        } else {
+            for (int c = 0; c < CW; c++) {
+              part0[c] = fmaf(0.25f, __uint_as_float(rb[c]), part0[c]);
+              part1[c] = fmaf(0.75f, __uint_as_float(rb[c]), fmaf(0.25f, __uint_as_float(ra[c]), part1[c]));
+            }
+            emit(part0, 2 * s - 2, pvq);
+            emit(part1, 2 * s - 1, pvq1);
+          }
+          tmem_ld16(g_cur, ra);
+          tmem_ld16(g_cur + PN, rb);
+          tmem_ld_wait();
+          {
+            const float a0 = first ? 0.f : 0.25f, a1 = first ? 1.f : 0.75f;
+            const float e0 = first ? 1.f : 0.75f, e1 = last ? 1.f : 0.75f;
 #pragma unroll
-          for (int c = 0; c < CW; c++) rb[c] = 0u;
-        }
-        tmem_ld_wait();
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) {
-          if (sl >= 1) mbar_arrive(&pempty[(q + kPGroups - 1) % kPGroups]);
-          if (sl == p.D - 1) mbar_arrive(&pempty[q % kPGroups]);
-        }
-        if (p.debug & 128) continue;                     // ablation: handshakes only
-        // out(sl-1) is complete now; out(D-1) completes together with the last event
-        if (sl >= 1) {
-          float f[CW];
+            for (int c = 0; c < CW; c++) {
+              const float b = s_bias[chalf * CW + c];
+              part0[c] = fmaf(a1, __uint_as_float(rb[c]), fmaf(a0, __uint_as_float(ra[c]), b));
+              part1[c] = fmaf(e1, __uint_as_float(rb[c]), fmaf(e0, __uint_as_float(ra[c]), b));
+            }
+          }
+          tmem_ld16(g_cur + 2 * PN, ra);
+          if (!first) tmem_ld16(g_prev, rb);
+          tmem_ld_wait();
+          {
+            const float a2 = last ? 1.f : 0.75f, e2 = last ? 0.f : 0.25f;
 #pragma unroll
-          for (int c = 0; c < CW; c++) f[c] = partial[c] + __uint_as_float(ra[c]);
-          emit(f, sl - 1);
-        }
+            for (int c = 0; c < CW; c++) {
+              part0[c] = fmaf(a2, __uint_as_float(ra[c]), part0[c]);
+              part1[c] = fmaf(e2, __uint_as_float(ra[c]), part1[c]);
+            }
+          }
+          if (!first) {
 #pragma unroll
-        for (int c = 0; c < CW; c++) partial[c] = (__uint_as_float(rb[c]) + __uint_as_float(rc[c])) + bias[c];
-        if (sl == p.D - 1) {
-          emit(partial, sl);
+            for (int c = 0; c < CW; c++) {
+              part0[c] = fmaf(0.75f, __uint_as_float(rb[c]), part0[c]);
+              part1[c] = fmaf(0.25f, __uint_as_float(rb[c]), part1[c]);
+            }
+            tmem_ld16(g_prev + PN, ra);
+            tmem_ld_wait();
+#pragma unroll
+            for (int c = 0; c < CW; c++) part0[c] = fmaf(0.25f, __uint_as_float(ra[c]), part0[c]);
+          }
+          tc_fence_before();
+          __syncwarp();
+          if (lane == 0) {
+            if (!first) mbar_arrive(&pempty[(q + kPGroups - 1) % kPGroups]);
+            if (last) mbar_arrive(&pempty[q % kPGroups]);
+          }
+          if (last) {
+            if (ACC) { load_prev(pvq, 2 * s); load_prev(pvq1, 2 * s + 1); }
+            emit(part0, 2 * s, pvq);
+            emit(part1, 2 * s + 1, pvq1);
+          }
+        }
+      } else {
+        if (ACC) load_prev(pvq, 0);
+        for (int sl = 0; sl < p.D; sl++) {
+          const uint32_t q = q0 + sl;
+          // with producer warps in the CTA the eight epilogue warps back off between polls (isolated launch of the
+          // fused 32->32 layer: 5.97 -> 5.12 ms; inside the full step the effect is within run-to-run noise)
+          if (xform) mbar_wait_backoff(&pfull[q % kPGroups], (q / kPGroups) & 1, 100u);
+          else mbar_wait(&pfull[q % kPGroups], (q / kPGroups) & 1);
+          tc_fence_after();
+          const uint32_t g_cur = lane_addr + (q % kPGroups) * (3 * PN);
+          const uint32_t g_prev = lane_addr + ((q + kPGroups - 1) % kPGroups) * (3 * PN);
+          uint32_t ra[CW], rb[CW], rc[CW];
+          if (sl >= 1 && !(p.debug & 24)) {
+            if constexpr (CW == 16) { tmem_ld16(g_cur + 2 * PN, ra); tmem_ld16(g_prev, rc); }
+            else { tmem_ld8(g_cur + 2 * PN, ra); tmem_ld8(g_prev, rc); }
+          } else {
+#pragma unroll
+            for (int c = 0; c < CW; c++) { ra[c] = 0u; rc[c] = 0u; }
+          }
+          if (!(p.debug & 8)) {
+            if constexpr (CW == 16) tmem_ld16(g_cur + PN, rb);
+            else tmem_ld8(g_cur + PN, rb);
+          } else {
+#pragma unroll
+            for (int c = 0; c < CW; c++) rb[c] = 0u;
+          }
+          tmem_ld_wait();
+          tc_fence_before();
+          __syncwarp();
+          if (lane == 0) {
+            if (sl >= 1) mbar_arrive(&pempty[(q + kPGroups - 1) % kPGroups]);
+            if (sl == p.D - 1) mbar_arrive(&pempty[q % kPGroups]);
+          }
+          if (p.debug & 128) continue;                     // ablation: handshakes only
+          // out(sl-1) is complete now; out(D-1) completes together with the last event
+          if (sl >= 1) {
+            float f[CW];
+#pragma unroll
+            for (int c = 0; c < CW; c++) f[c] = partial[c] + __uint_as_float(ra[c]);
+            emit(f, sl - 1, pvq);
+          }
+#pragma unroll
+          for (int c = 0; c < CW; c++) partial[c] = (__uint_as_float(rb[c]) + __uint_as_float(rc[c])) + bias[c];
+          if (sl == p.D - 1) {
+            emit(partial, sl, pvq);
+          }
         }
       }
       if (p.stats) {
@@ -1482,18 +1590,25 @@ int conv3d_tc_impl(const void* x, const void* packed_w, const float* bias, void*
           NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab3_kernel<64, 32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
           NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab3_kernel<64, 32, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
           NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab3_kernel<64, 32, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+          NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab3_kernel<64, 32, true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+          NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab3_kernel<64, 32, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
         });
         static int xw_env = -1;
         if (xw_env < 0) { const char* e = getenv("NM_XFORM_WARPS"); xw_env = e ? atoi(e) : 6; if (xw_env != 4) xw_env = 6; }
         // the up-sampling producer runs on 4 warps (3 working): with 6 (5 working, 144 finer items) dec.8 got slower
         // [measured, same GPU: 20.4 -> 24.6 ms per 640 frames] - more producer threads take issue slots and shared-memory
         // bandwidth from the MMA / epilogue warps; the in-place transform gains from 6 (13.2 -> 11.6 ms)
-        const int threads3 = kSlab3Threads + (up ? 32 * 4 : (in_scale ? 32 * xw_env : 0));
+        const int threads3 = kSlab3Threads + (up ? 32 * kUpWarps : (in_scale ? 32 * xw_env : 0));
+        // NM_UP_DEPTH_EPI=0: the up-sampling producer blends two planes per output slice (A/B switch, read per call)
+        const char* depi_env = getenv("NM_UP_DEPTH_EPI");
+        const bool depi = up && !(depi_env && strcmp(depi_env, "0") == 0);
         if (accum) {
           NM_CHECK_ARG(bk == 64 && pn == 32 && !in_scale, "nm_conv3d_tc: split-K accumulation needs slab3<64, 32>");
-          if (up) conv3d_slab3_kernel<64, 32, true, true><<<grid, threads3, need, (cudaStream_t)stream>>>(q);
+          if (depi) conv3d_slab3_kernel<64, 32, true, true, true><<<grid, threads3, need, (cudaStream_t)stream>>>(q);
+          else if (up) conv3d_slab3_kernel<64, 32, true, true><<<grid, threads3, need, (cudaStream_t)stream>>>(q);
           else conv3d_slab3_kernel<64, 32, false, true><<<grid, threads3, need, (cudaStream_t)stream>>>(q);
-        } else if (up) conv3d_slab3_kernel<64, 32, true><<<grid, threads3, need, (cudaStream_t)stream>>>(q);
+        } else if (depi) conv3d_slab3_kernel<64, 32, true, false, true><<<grid, threads3, need, (cudaStream_t)stream>>>(q);
+        else if (up) conv3d_slab3_kernel<64, 32, true><<<grid, threads3, need, (cudaStream_t)stream>>>(q);
         else if (pn == 16) conv3d_slab3_kernel<64, 16><<<grid, threads3, need, (cudaStream_t)stream>>>(q);
         else if (bk == 64) conv3d_slab3_kernel<64, 32><<<grid, threads3, need, (cudaStream_t)stream>>>(q);
         else conv3d_slab3_kernel<32, 32><<<grid, threads3, need, (cudaStream_t)stream>>>(q);

@@ -5,6 +5,7 @@ from __future__ import annotations
 
 import ctypes
 import math
+import os
 from typing import Optional, Tuple
 
 import torch
@@ -537,7 +538,11 @@ def conv3d_up2x(x_lo: torch.Tensor, conv: torch.nn.Conv3d, gn: Optional[torch.nn
            L.ptr(ia[0]), L.ptr(ia[1]), int(ia[2]), L.ptr(partial), L.stream())
     if PROFILE is not None:
         e1.record()
+        # what the tensor cores execute: the depth half of the up-sampling is applied to the accumulators (MMAs over
+        # the D low-resolution slices), unless NM_UP_DEPTH_EPI=0 selects the two-plane operand producer
         flops = 2.0 * n * 8 * D * H * W * Cout * Cin * 27
+        if os.environ.get("NM_UP_DEPTH_EPI", "1") != "0":
+            flops /= 2
         PROFILE.setdefault(("conv", n, 2 * D, Cin, Cout, 3, 1, flops), []).append((e0, e1))
     if gn is None:
         return out
