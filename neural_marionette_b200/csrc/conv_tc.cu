@@ -16,9 +16,7 @@
 #include "common.cuh"
 #include "../../include/nm_b200.h"   // the definitions below must match the public declarations
 #include <cuda.h>
-#include <stdlib.h>
 #include <string.h>
-#include <type_traits>
 
 namespace {
 
@@ -383,209 +381,36 @@ conv3d_tc_kernel(const __grid_constant__ ConvTcParams p) {
   }
 }
 
-// ------------------------------------------------------------------ slab-walking variant (k3, small Cout)
+// ------------------------------------------------------------------ slab-walking kernel (k3, Cout <= 128)
 // For Cout <= 64 the tap-streaming kernel above is bound by operand delivery: every tap re-fetches its
 // 128 x Cin A tile from L2 (27x re-read; ncu: 7 TB/s L2->SM, tensor pipe 8 %).  Here a CTA owns a column of
 // output tiles (16 h x 8 w voxels) and walks it along d: each input slice (18 x 10 halo rows) is fetched ONCE
-// by TMA into a 4-slot ring and reused by all 27 taps - a tap is just a different start address / the same
+// by TMA into a ring of slots and reused by all 27 taps - a tap is just a different start address / the same
 // 8-row-group stride (10 rows) in the A descriptor (the 128B/64B swizzle is a function of the absolute
 // shared-memory address, so a row-shifted start stays consistent with what TMA wrote; verified on B200).
 // The weights of all taps stay resident in shared memory.
 struct ConvSlabParams {
   CUtensorMap tmap_a;     // (C, W, H, D, N) box (BK, 10, 18, 1, 1)
-  CUtensorMap tmap_b;     // (Cin, Cout, 27) box (BK, n_tile, 1)
-  CUtensorMap tmap_o;     // slab3: output (Cout, W, H, D, N) box (PN, 8, 16, 1, 1) for the TMA-store epilogue
+  CUtensorMap tmap_b;     // (Cin, Cout, 27) box (BK, PN, 1)
+  CUtensorMap tmap_o;     // output (Cout, W, H, D, N) box (PN, 8, 16, 1, 1) for the TMA-store epilogue
   int kchunks, block_k, n_tile, cout;
   int nw, nh;             // tiles per (w, h); columns = N * nh * nw
   int D, H, W, N;
   int slot_bytes;         // bytes of one ring slot (kchunks chunks)
   int chunk_bytes;        // bytes of one (slice, k-chunk) = 180 rows, padded to 1 KiB
-  int ring;               // slab3: ring slots actually used (2..4)
-  int debug;              // NM_SLAB_DEBUG bit mask (profiling experiments only): 1 no stores, 2 no MMAs, 4 no A loads
-  float* stats;           // slab3: optional GroupNorm partials [n][nh*nw*4][Cout][2] (sum, sum of squares)
-  const float* in_scale;  // slab3: optional fused input transform x <- act(x * in_scale[n][c] + in_shift[n][c]),
-  const float* in_shift;  //        i.e. the GroupNorm (+LeakyReLU) of the producing layer applied on the halo
-  int in_act;             //        slice in shared memory (zero padding preserved); (n, Cin) fp32 each
+  int ring;               // ring slots actually used (2..8)
+  float* stats;           // optional GroupNorm partials [n][nh*nw*4][Cout][2] (sum, sum of squares)
+  const float* in_scale;  // optional fused input transform x <- act(x * in_scale[n][c] + in_shift[n][c]),
+  const float* in_shift;  // i.e. the GroupNorm (+LeakyReLU) of the producing layer applied on the halo
+  int in_act;             // slice in shared memory (zero padding preserved); (n, Cin) fp32 each
   int cin;
-  int cin_off;            // slab3: first input channel of this launch (split-K over two launches: Cin = 128)
-  int accum;              // slab3: add the existing contents of `out` (the partial sum of the previous launch)
+  int cin_off;            // first input channel of this launch (split-K over two launches: Cin = 128)
+  int accum;              // add the existing contents of `out` (the partial sum of the previous launch)
   const float* bias;      // may be null (second split-K launch)
   act_t* out;
 };
 
-constexpr int kSlabRing = 4;
 constexpr int kHaloW = 10, kHaloH = 18;
-
-template <int BK>
-__global__ void __launch_bounds__(192, 1)
-conv3d_slab_kernel(const __grid_constant__ ConvSlabParams p) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-  const int w_tile_bytes = p.n_tile * BK * 2;                         // one (tap, k-chunk) weight tile
-  const int w_bytes = 27 * p.kchunks * w_tile_bytes;
-  uint8_t* s_w = smem;
-  uint8_t* s_ring = smem + w_bytes;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(s_ring + (size_t)kSlabRing * p.slot_bytes);
-  uint64_t* full = bars;                 // [ring]
-  uint64_t* empty = bars + kSlabRing;    // [ring]
-  uint64_t* tfull = empty + kSlabRing;   // [2]
-  uint64_t* tempty = tfull + 2;          // [2]
-  uint64_t* wfull = tempty + 2;          // [1] weights landed
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(wfull + 1);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int n_cols = p.N * p.nh * p.nw;
-  uint32_t tmem_cols = 32;
-  while ((int)tmem_cols < 2 * p.n_tile) tmem_cols <<= 1;
-
-  if (warp == 0 && lane == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&p.tmap_a) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&p.tmap_b) : "memory");
-    for (int s = 0; s < kSlabRing; s++) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
-    for (int s = 0; s < 2; s++) { mbar_init(&tfull[s], 1); mbar_init(&tempty[s], 4); }
-    mbar_init(wfull, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(tmem_cols)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  // One CTA per SM and a single allocation: the allocator hands out column 0.  Treating the base as the
-  // literal 0 keeps every TMEM address a warp-uniform value (uniform registers), which removes an
-  // ELECT / R2UR.BROADCAST / branch sequence in front of every UTCHMMA in the issue loop.
-  if (*tmem_slot != 0u) {
-    printf("nm_conv3d_tc(slab): unexpected TMEM base %u\n", *tmem_slot);
-    __trap();
-  }
-  constexpr uint32_t tmem_base = 0u;
-
-  if (warp == 0) {
-    // ===================== TMA producer =====================
-    if (lane == 0) {
-      // resident weights: 27 * kchunks tiles, one barrier
-      mbar_expect_tx(wfull, (uint32_t)w_bytes);
-      for (int tap = 0; tap < 27; tap++)
-        for (int kc = 0; kc < p.kchunks; kc++)
-          tma_load_3d(s_w + (size_t)(tap * p.kchunks + kc) * w_tile_bytes, &p.tmap_b, wfull, kc * BK, 0, tap);
-      uint32_t fill = 0;                                  // running count of slice fills (ring position)
-      const uint32_t slice_tx = (uint32_t)(kHaloW * kHaloH * BK * 2 * p.kchunks);
-      for (int col = blockIdx.x; col < n_cols; col += gridDim.x) {
-        int t = col;
-        const int iw = t % p.nw; t /= p.nw;
-        const int ih = t % p.nh; t /= p.nh;
-        const int n = t;
-        for (int dz = -1; dz <= p.D; dz++, fill++) {
-          const int slot = fill % kSlabRing;
-          mbar_wait(&empty[slot], ((fill / kSlabRing) & 1) ^ 1);
-          mbar_expect_tx(&full[slot], slice_tx);
-          for (int kc = 0; kc < p.kchunks; kc++)
-            tma_load_5d(s_ring + (size_t)slot * p.slot_bytes + (size_t)kc * p.chunk_bytes, &p.tmap_a, &full[slot],
-                        kc * BK, iw * 8 - 1, ih * 16 - 1, dz, n);
-        }
-      }
-    }
-  } else if (warp == 1) {
-    // ===================== MMA issuer =====================
-    const uint32_t idesc = (1u << 4) | ((uint32_t)(p.n_tile >> 3) << 17) | ((uint32_t)(kTileM >> 4) << 24);
-    constexpr uint32_t row_bytes = BK * 2;
-    constexpr uint32_t layout = row_bytes == 128 ? 2u : 4u;
-    // A: next 8-row group = next h row of the halo slice (10 rows further); B: dense 8-row groups
-    const uint32_t hi_a = desc_hi(kHaloW * row_bytes, layout), hi_b = desc_hi(8 * row_bytes, layout);
-    const uint32_t ring_lo = desc_lo(smem_u32(s_ring)), w_lo = desc_lo(smem_u32(s_w));
-    const uint32_t slot_step = (uint32_t)p.slot_bytes >> 4, chunk_step = (uint32_t)p.chunk_bytes >> 4;
-    const uint32_t w_step = (uint32_t)w_tile_bytes >> 4;
-    mbar_wait(wfull, 0);
-    uint32_t fill = 0;                                   // index of the next slice fill to wait for
-    int acc = 0;
-    uint32_t acc_phase = 0;
-    for (int col = blockIdx.x; col < n_cols; col += gridDim.x) {
-      // slices -1 and 0 of this column
-      for (int pre = 0; pre < 2; pre++, fill++) mbar_wait(&full[fill % kSlabRing], (fill / kSlabRing) & 1);
-      for (int d = 0; d < p.D; d++) {
-        mbar_wait(&full[fill % kSlabRing], (fill / kSlabRing) & 1);   // slice d + 1
-        fill++;
-        mbar_wait(&tempty[acc], acc_phase ^ 1);
-        tc_fence_after();
-        __syncwarp();
-        if (elect_one()) {
-          const uint32_t tmem_d = tmem_base + (uint32_t)(acc * p.n_tile);
-          const uint32_t first_fill = fill - 3;          // fill index of slice d - 1
-          uint32_t blo = w_lo;
-#pragma unroll 1
-          for (int kd = 0; kd < 3; kd++) {
-            const uint32_t slot_lo = ring_lo + ((first_fill + kd) % kSlabRing) * slot_step;
-#pragma unroll
-            for (int t9 = 0; t9 < 9; t9++) {
-              const uint32_t tap_lo = slot_lo + (uint32_t)(((t9 / 3) * kHaloW + (t9 % 3)) * (BK * 2 / 16));
-#pragma unroll 1
-              for (int kc = 0; kc < p.kchunks; kc++) {
-                const uint32_t alo = tap_lo + kc * chunk_step;
-                if (kd == 0 && t9 == 0 && kc == 0) umma_f16(tmem_d, desc64(hi_a, alo), desc64(hi_b, blo), idesc, 0u);
-                else umma_f16_acc(tmem_d, desc64(hi_a, alo), desc64(hi_b, blo), idesc);
-#pragma unroll
-                for (int k = 1; k < BK / 16; k++)
-                  umma_f16_acc(tmem_d, desc64(hi_a, alo + 2 * k), desc64(hi_b, blo + 2 * k), idesc);
-                blo += w_step;
-              }
-            }
-          }
-          umma_commit(&empty[first_fill % kSlabRing]);   // slice d - 1 is dead once these MMAs retire
-          umma_commit(&tfull[acc]);
-          if (d == p.D - 1) {                            // column done: slices D-1 and D are dead too
-            umma_commit(&empty[(first_fill + 1) % kSlabRing]);
-            umma_commit(&empty[(first_fill + 2) % kSlabRing]);
-          }
-        }
-        __syncwarp();
-        if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-      }
-    }
-  } else {
-    // ===================== epilogue (warps 2..5) =====================
-    const int quad = warp & 3;
-    const int row = quad * 32 + lane;
-    const int rx = row & 7, ry = row >> 3;               // row = h * 8 + w inside the 16 x 8 tile
-    int acc = 0;
-    uint32_t acc_phase = 0;
-    for (int col = blockIdx.x; col < n_cols; col += gridDim.x) {
-      int t = col;
-      const int iw = t % p.nw; t /= p.nw;
-      const int ih = t % p.nh; t /= p.nh;
-      const int n = t;
-      const int ow = iw * 8 + rx, oh = ih * 16 + ry;
-      for (int d = 0; d < p.D; d++) {
-        act_t* dst = p.out + ((((long long)n * p.D + d) * p.H + oh) * p.W + ow) * (long long)p.cout;
-        mbar_wait(&tfull[acc], acc_phase);
-        tc_fence_after();
-        const uint32_t taddr = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(acc * p.n_tile);
-        for (int c0 = 0; c0 < p.n_tile; c0 += 16) {
-          uint32_t r[16];
-          tmem_ld16(taddr + c0, r);
-          tmem_ld_wait();
-          float f[16];
-#pragma unroll
-          for (int j = 0; j < 16; j++) f[j] = __uint_as_float(r[j]) + ((c0 + j < p.cout) ? __ldg(p.bias + c0 + j) : 0.f);
-          if (c0 + 8 <= p.cout) *reinterpret_cast<half8*>(dst + c0) = nm_pack8(f);
-          if (c0 + 16 <= p.cout) *reinterpret_cast<half8*>(dst + c0 + 8) = nm_pack8(f + 8);
-        }
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&tempty[acc]);
-        if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) {
-    tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(tmem_cols) : "memory");
-  }
-}
 
 // ------------------------------------------------------------------ slab kernel, 3 depth-taps per MMA (Cout = 32)
 // With N = Cout = 32 an MMA is 16 tensor-pipe cycles but costs ~70 cycles to issue from a single thread and
@@ -606,24 +431,23 @@ constexpr int kSlab3XformWarps = 6;   // max extra warps (only launched when the
                                       // number actually launched comes from blockDim (512 threads x 128 registers)
 
 // UP: the conv input is the 2x trilinear up-sampling (align_corners = False) of a low-resolution tensor that is
-// never materialised: TMA brings (10 x 6)-row low-resolution planes into a small ring and the transform warps
-// interpolate every halo slice from two planes directly into the swizzled operand layout (tmap_a then describes the
-// low-resolution tensor; BK = 64, one k-chunk).
+// never materialised (tmap_a then describes the low-resolution tensor; BK = 64, one k-chunk).  Everything after the
+// input transform is linear and trilinear x2 is separable, so the depth part of the up-sampling is applied to the
+// accumulators instead of the operand: TMA brings (10 x 6)-row low-resolution planes into a small ring, the transform
+// warps build one halo slice per LOW-resolution plane (h / w interpolation only) directly in the swizzled operand
+// layout, the MMAs run over D/2 slices, and the epilogue forms every output slice as a fixed combination of the TMEM
+// groups P(i-1), P(i), P(i+1).  Half the MMAs, half the operand traffic; the depth border (clamp + zero padding)
+// stays exact and is blended in fp32.
 constexpr int kLoRing = 4;
 constexpr int kLoRows = 10 * 6;              // low-resolution box: 10 (h) x 6 (w) rows of 64 channels
 constexpr int kLoBytes = kLoRows * 128;      // 7680
 constexpr int kUpWarps = 4;                  // up-sampling producer warps launched (3 working)
 
 // ACC: split-K second launch - the epilogue adds the partial sum already in `out`.
-// DEPI (with UP): the depth part of the up-sampling is applied to the accumulators instead of the operand.  Everything
-// after the input transform is linear and trilinear x2 is separable, so the producer builds one halo slice per
-// LOW-resolution plane (h / w interpolation only), the MMAs run over D/2 slices, and the epilogue forms every output
-// slice as a fixed combination of the TMEM groups P(i-1), P(i), P(i+1) (coefficients at the epilogue).  Half the MMAs,
-// half the operand traffic; the depth border (clamp + zero padding) stays exact and is blended in fp32.
-template <int BK, int PN, bool UP = false, bool ACC = false, bool DEPI = false>
+template <int BK, int PN, bool UP = false, bool ACC = false>
 __global__ void __launch_bounds__(kSlab3Threads + 32 * kSlab3XformWarps, 1)
 conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
-  static_assert(!DEPI || (UP && PN == 32), "the depth epilogue belongs to the up-sampling variant");
+  static_assert(!UP || PN == 32, "the up-sampling epilogue serves 32-channel parts");
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
   constexpr int w_tile_bytes = PN * BK * 2;                            // one (tap, k-chunk)
@@ -647,7 +471,7 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
   float* s_ab = reinterpret_cast<float*>(tmem_slot + 4);   // [2][Cin] scale | shift of the current sample
   const bool xform = UP || p.in_scale != nullptr;
   const int nxw = ((int)blockDim.x - kSlab3Threads) >> 5;   // transform / producer warps launched (0, 4 or 6)
-  const int n_sl = DEPI ? p.D >> 1 : p.D;                   // operand slices (= TMEM groups) per column
+  const int n_sl = UP ? p.D >> 1 : p.D;                     // operand slices (= TMEM groups) per column
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int n_cols = p.N * p.nh * p.nw;
@@ -684,15 +508,16 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
 
   if (UP && warp >= 2 + kSlab3EpiWarps) {
     // ===================== up-sampling operand producer (warps 10..13) =====================
-    // Output slice d blends the low-res planes near = d>>1 and far = near -/+ 1 (clamped) with weights 0.75 / 0.25
-    // (PyTorch trilinear, align_corners = False); the same rule applies along h and w.  Work item = (halo row hh,
-    // 16-byte channel chunk c): 24 plane loads -> depth + h blends for the 6 box columns -> the 10 halo columns of
-    // that row, written at the TMA-128B-swizzle position.  Rows / columns outside the tensor are the conv's zero
-    // padding.  With a fused prologue the producer's GroupNorm scale/shift (+LeakyReLU) is applied to each plane
-    // in place when it lands.  DEPI: operand slice d is low-res plane d blended in h and w only (near = far = d).
+    // Operand slice d is low-res plane d up-sampled along h and w (the depth part is applied in the epilogue): a
+    // full-resolution row blends the low-res rows near and far = near -/+ 1 (clamped) with weights 0.75 / 0.25
+    // (PyTorch trilinear, align_corners = False), and the same rule applies along w.  Work item = (pair of halo rows,
+    // 16-byte channel chunk c): 12 plane loads -> h blends for the 6 box columns -> the 10 halo columns of both rows,
+    // written at the TMA-128B-swizzle position.  Rows / columns outside the tensor are the conv's zero padding.  With
+    // a fused prologue the producer's GroupNorm scale/shift (+LeakyReLU) is applied to each plane in place when it
+    // lands.
     const int tid = threadIdx.x - 32 * (2 + kSlab3EpiWarps);
     const bool fused = p.in_scale != nullptr;
-    const int Dl = p.D >> 1, Hl = p.H >> 1;
+    const int Hl = p.H >> 1;
     const __half2 q25 = __float2half2_rn(0.25f);
     auto lerp = [&](const uint4& a, const uint4& b) -> uint4 {      // a + 0.25 (b - a)
       uint4 r;
@@ -725,7 +550,7 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
     uint32_t planes = 0;                                  // global index of plane 0 of the current column
     int cur_n = -1;
     const uint32_t lo_base = smem_u32(s_lo), ring_base = smem_u32(s_ring);
-    for (int col = col0; col < n_cols; col += col_step, planes += Dl) {
+    for (int col = col0; col < n_cols; col += col_step, planes += n_sl) {
       int t = col;
       const int iw = t % p.nw; t /= p.nw;
       const int ih = t % p.nh; t /= p.nh;
@@ -739,123 +564,85 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
         named_bar_sync(2, 32 * nxw);
         cur_n = n;
       }
-      int landed = 0;                                     // planes of this column already waited for
       for (int d = 0; d < n_sl; d++, fill++) {
-        const int pn = DEPI ? d : d >> 1, pf = DEPI ? d : min(max(pn + ((d & 1) ? 1 : -1), 0), Dl - 1);
-        const int need = max(pn, pf);
-        while (landed <= need) {
-          const uint32_t g = planes + landed;
-          mbar_wait(&full_lo[g % kLoRing], (g / kLoRing) & 1);
-          if (fused) {
-            const uint32_t pb = lo_base + (g % kLoRing) * kLoBytes;
-            for (int i = tid; i < kLoRows * 8; i += 32 * nxw) {
-              const int c = i & 7;
-              const uint32_t addr = pb + i * 16;
-              const uint4 raw = lds128(addr);
-              const uint32_t in[4] = {raw.x, raw.y, raw.z, raw.w};
-              uint32_t o[4];
+        const uint32_t g = planes + d;                    // global index of low-res plane d
+        const uint32_t lo = lo_base + (g % kLoRing) * kLoBytes;
+        mbar_wait(&full_lo[g % kLoRing], (g / kLoRing) & 1);
+        if (fused) {
+          for (int i = tid; i < kLoRows * 8; i += 32 * nxw) {
+            const int c = i & 7;
+            const uint32_t addr = lo + i * 16;
+            const uint4 raw = lds128(addr);
+            const uint32_t in[4] = {raw.x, raw.y, raw.z, raw.w};
+            uint32_t o[4];
 #pragma unroll
-              for (int k = 0; k < 4; k++) {
-                const float2 f = __half22float2(*reinterpret_cast<const __half2*>(&in[k]));
-                __half2 hv = __floats2half2_rn(fmaf(f.x, s_ab[c * 8 + 2 * k], s_ab[p.cin + c * 8 + 2 * k]),
-                                               fmaf(f.y, s_ab[c * 8 + 2 * k + 1], s_ab[p.cin + c * 8 + 2 * k + 1]));
-                if (p.in_act) hv = __hmax2(hv, __hmul2(hv, __float2half2_rn(0.01f)));
-                o[k] = *reinterpret_cast<uint32_t*>(&hv);
-              }
-              sts128(addr, make_uint4(o[0], o[1], o[2], o[3]));
+            for (int k = 0; k < 4; k++) {
+              const float2 f = __half22float2(*reinterpret_cast<const __half2*>(&in[k]));
+              __half2 hv = __floats2half2_rn(fmaf(f.x, s_ab[c * 8 + 2 * k], s_ab[p.cin + c * 8 + 2 * k]),
+                                             fmaf(f.y, s_ab[c * 8 + 2 * k + 1], s_ab[p.cin + c * 8 + 2 * k + 1]));
+              if (p.in_act) hv = __hmax2(hv, __hmul2(hv, __float2half2_rn(0.01f)));
+              o[k] = *reinterpret_cast<uint32_t*>(&hv);
             }
-            named_bar_sync(2, 32 * nxw);
+            sts128(addr, make_uint4(o[0], o[1], o[2], o[3]));
           }
-          landed++;
+          named_bar_sync(2, 32 * nxw);
         }
         const int slot = fill % ring;
         mbar_wait(&empty[slot], ((fill / ring) & 1) ^ 1);
         const uint32_t sbase = ring_base + (uint32_t)slot * p.slot_bytes;
-        const uint32_t lo_n = lo_base + ((planes + pn) % kLoRing) * kLoBytes;
-        const uint32_t lo_f = lo_base + ((planes + pf) % kLoRing) * kLoBytes;
         // item = (pair of halo rows 2j, 2j+1, chunk c): h = ih*16 - 1 + 2j is odd (= 2m+1) and h + 1 = 2m+2, so both
-        // rows interpolate between the same low-res rows m and m+1 (near / far swapped): the 24 plane loads and the
-        // 12 depth blends are shared
-        // Work split: with 4 producer warps, 72 (pair, chunk) items on the first three; with 6 warps, 144 (pair, chunk,
-        // half of the 10 halo columns) items on five.  The warp that shares its SM sub-partition with the MMA-issuing
-        // warp (producer warp 3 = warp 13) only takes part in the barriers, so that it does not compete for issue slots.
-        const int pw = tid >> 5;                                     // producer warp index
-        const int wtid = pw < 3 ? tid : (pw == 3 ? -1 : tid - 32);   // worker thread id, -1: idle warp
-        const bool split = nxw >= 6;
-        const int n_items = split ? (kHaloH / 2) * 16 : (kHaloH / 2) * 8;
-        const int n_workers = split ? 160 : 96;
-        for (int item = (wtid >= 0 && !(p.debug & 512)) ? wtid : 99999; item < n_items; item += n_workers) {   // 512: ablation, no interpolation
-          const int j = split ? item >> 4 : item >> 3, c = split ? (item >> 1) & 7 : item & 7;
-          const int half = split ? item & 1 : 2;                     // 0: columns 0..4, 1: 5..9, 2: all ten
+        // rows interpolate between the same low-res rows m and m+1 (near / far swapped): the 12 plane loads are shared.
+        // The 72 items go to the first three producer warps.  The fourth (warp 13) shares its SM sub-partition with
+        // the MMA-issuing warp and only takes part in the barriers, so that it does not compete for issue slots.
+        if (tid < (kHaloH / 2) * 8) {
+          const int j = tid >> 3, c = tid & 7;
           const int h0 = ih * 16 - 1 + 2 * j;                        // first row of the pair (may be -1)
           const int m = (h0 + 1) / 2 - 1;                            // h0 = 2m + 1
           const int ma = min(max(m, 0), Hl - 1), mb = min(m + 1, Hl - 1);
           const uint32_t oa = (uint32_t)((ma - (ih * 8 - 1)) * 6) * 128 + c * 16;
           const uint32_t ob = (uint32_t)((mb - (ih * 8 - 1)) * 6) * 128 + c * 16;
           const uint4 zero = make_uint4(0, 0, 0, 0);
-          // W0 .. W0+NW-1: box columns needed; WW0 .. WW0+NWW-1: halo columns produced
-          auto run = [&](auto W0c, auto NWc, auto WW0c, auto NWWc) {
-            constexpr int W0 = decltype(W0c)::value, NW = decltype(NWc)::value, WW0 = decltype(WW0c)::value,
-                          NWW = decltype(NWWc)::value;
-            uint4 va[NW], vb[NW];                                    // depth-blended low-res rows m and m+1
+          constexpr int NW = 6;                                      // box columns
+          uint4 va[NW], vb[NW];                                      // low-res rows m and m+1
 #pragma unroll
-            for (int w = 0; w < NW; w++) {
-              if constexpr (DEPI) {
-                va[w] = lds128(lo_n + oa + (W0 + w) * 128);
-                vb[w] = lds128(lo_n + ob + (W0 + w) * 128);
-              } else {
-                va[w] = lerp(lds128(lo_n + oa + (W0 + w) * 128), lds128(lo_f + oa + (W0 + w) * 128));
-                vb[w] = lerp(lds128(lo_n + ob + (W0 + w) * 128), lds128(lo_f + ob + (W0 + w) * 128));
-              }
+          for (int w = 0; w < NW; w++) {
+            va[w] = lds128(lo + oa + w * 128);
+            vb[w] = lds128(lo + ob + w * 128);
+          }
+#pragma unroll
+          for (int r2 = 0; r2 < 2; r2++) {
+            const int hh = 2 * j + r2, hf = h0 + r2;
+            const uint32_t orow = sbase + (uint32_t)(hh * kHaloW) * 128;
+            if ((unsigned)hf >= (unsigned)p.H) {                     // conv padding row
+#pragma unroll
+              for (int ww = 0; ww < kHaloW; ww++) sts128(orow + ww * 128 + ((c ^ ((hh * kHaloW + ww) & 7)) << 4), zero);
+              continue;
             }
+            uint4 v[NW];                                             // row 2m+1: near m, far m+1; row 2m+2: near m+1, far m
 #pragma unroll
-            for (int r2 = 0; r2 < 2; r2++) {
-              const int hh = 2 * j + r2, hf = h0 + r2;
-              const uint32_t orow = sbase + (uint32_t)(hh * kHaloW) * 128;
-              if ((unsigned)hf >= (unsigned)p.H) {                   // conv padding row
+            for (int w = 0; w < NW; w++) v[w] = r2 == 0 ? lerp(va[w], vb[w]) : lerp(vb[w], va[w]);
+            // along w every box column is the near operand of two halo columns and the far operand of up to two:
+            // 0.75 v and 0.25 v once per column, then one add per output (22 instead of 40 half2 ops per channel pair)
+            uint4 t75[NW], t25[NW];
 #pragma unroll
-                for (int k = 0; k < NWW; k++) sts128(orow + (WW0 + k) * 128 + ((c ^ ((hh * kHaloW + WW0 + k) & 7)) << 4), zero);
-                continue;
-              }
-              uint4 v[NW];                                           // row 2m+1: near m, far m+1; row 2m+2: near m+1, far m
+            for (int w = 0; w < NW; w++) { t75[w] = scale4(v[w], q75); t25[w] = scale4(v[w], q25); }
 #pragma unroll
-              for (int w = 0; w < NW; w++) v[w] = r2 == 0 ? lerp(va[w], vb[w]) : lerp(vb[w], va[w]);
-              // along w every box column is the near operand of two halo columns and the far operand of up to two:
-              // 0.75 v and 0.25 v once per column, then one add per output (22 instead of 40 half2 ops per channel pair)
-              uint4 t75[NW], t25[NW];
-#pragma unroll
-              for (int w = 0; w < NW; w++) { t75[w] = scale4(v[w], q75); t25[w] = scale4(v[w], q25); }
-#pragma unroll
-              for (int k = 0; k < NWW; k++) {
-                // halo column ww <-> w = iw*8 - 1 + ww: near box column (ww+1)>>1, far = near +1 (ww even) / -1 (ww odd)
-                const int ww = WW0 + k;
-                const int nr = ((ww + 1) >> 1) - W0, fr = (ww & 1) ? nr - 1 : nr + 1;
-                uint4 o;
-                if ((ww == 0 && iw == 0) || (ww == kHaloW - 1 && iw == p.nw - 1)) o = zero;             // conv padding
-                else if ((ww == 1 && iw == 0) || (ww == kHaloW - 2 && iw == p.nw - 1)) o = v[nr];        // clamped far
-                else o = add4(t75[nr], t25[fr]);
-                sts128(orow + ww * 128 + ((c ^ ((hh * kHaloW + ww) & 7)) << 4), o);
-              }
+            for (int ww = 0; ww < kHaloW; ww++) {
+              // halo column ww <-> w = iw*8 - 1 + ww: near box column (ww+1)>>1, far = near +1 (ww even) / -1 (ww odd)
+              const int nr = (ww + 1) >> 1, fr = (ww & 1) ? nr - 1 : nr + 1;
+              uint4 o;
+              if ((ww == 0 && iw == 0) || (ww == kHaloW - 1 && iw == p.nw - 1)) o = zero;             // conv padding
+              else if ((ww == 1 && iw == 0) || (ww == kHaloW - 2 && iw == p.nw - 1)) o = v[nr];        // clamped far
+              else o = add4(t75[nr], t25[fr]);
+              sts128(orow + ww * 128 + ((c ^ ((hh * kHaloW + ww) & 7)) << 4), o);
             }
-          };
-          using I0 = std::integral_constant<int, 0>; using I2 = std::integral_constant<int, 2>;
-          using I4 = std::integral_constant<int, 4>; using I5 = std::integral_constant<int, 5>;
-          using I6 = std::integral_constant<int, 6>; using I10 = std::integral_constant<int, 10>;
-          if (half == 0) run(I0{}, I4{}, I0{}, I5{});                // halo columns 0..4 use box columns 0..3
-          else if (half == 1) run(I2{}, I4{}, I5{}, I5{});           // halo columns 5..9 use box columns 2..5
-          else run(I0{}, I6{}, I0{}, I10{});
+          }
         }
         fence_async_smem();                              // generic-proxy writes -> visible to the UMMA reads
         __syncwarp();
         if (lane == 0) {
           mbar_arrive(&ready[slot]);
-          if (DEPI) {
-            mbar_arrive(&empty_lo[(planes + d) % kLoRing]);
-          } else {
-            // plane x is last read by slice min(2x + 2, D - 1)
-            if (d >= 2 && !(d & 1)) mbar_arrive(&empty_lo[(planes + ((d - 2) >> 1)) % kLoRing]);
-            if (d == p.D - 1) mbar_arrive(&empty_lo[(planes + Dl - 1) % kLoRing]);
-          }
+          mbar_arrive(&empty_lo[g % kLoRing]);
         }
       }
     }
@@ -968,7 +755,6 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
         for (int dz = 0; dz < p.D; dz++, fill++) {
           const int slot = fill % ring;
           mbar_wait(&empty[slot], ((fill / ring) & 1) ^ 1);
-          if (p.debug & 4) { mbar_arrive(&full[slot]); continue; }
           mbar_expect_tx(&full[slot], slice_tx);
           for (int kc = 0; kc < p.kchunks; kc++)
             tma_load_5d(s_ring + (size_t)slot * p.slot_bytes + (size_t)kc * p.chunk_bytes, &p.tmap_a, &full[slot],
@@ -1001,7 +787,6 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
             const uint32_t tmem_d = (q % kPGroups) * (3 * PN);
             const uint32_t slot_lo = ring_lo + (q % ring) * slot_step;
             uint32_t blo = w_lo;
-            if (!(p.debug & 2))
 #pragma unroll
             for (int t9 = 0; t9 < 9; t9++) {
               const uint32_t tap_lo = slot_lo + (uint32_t)(((t9 / 3) * kHaloW + (t9 % 3)) * (BK * 2 / 16));
@@ -1031,7 +816,7 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
       uint32_t q = 0;                                    // global slice counter (ring + P-group position)
       auto wait_slice = [&](uint32_t qq) {
         mbar_wait(&full[qq % ring], (qq / ring) & 1);
-        if (!(p.debug & 256)) mbar_wait(&pempty[qq % kPGroups], ((qq / kPGroups) & 1) ^ 1);
+        mbar_wait(&pempty[qq % kPGroups], ((qq / kPGroups) & 1) ^ 1);
         tc_fence_after();
       };
       auto issue_tap = [&](int t9, uint32_t tmem_d, uint32_t slot_lo, uint32_t& blo) {
@@ -1050,7 +835,7 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
       // non-blocking variant: true when both barriers of slice qq have already completed
       auto try_slice = [&](uint32_t qq) -> bool {
         if (!mbar_try_wait(&full[qq % ring], (qq / ring) & 1)) return false;
-        if (!(p.debug & 256) && !mbar_try_wait(&pempty[qq % kPGroups], ((qq / kPGroups) & 1) ^ 1)) return false;
+        if (!mbar_try_wait(&pempty[qq % kPGroups], ((qq / kPGroups) & 1) ^ 1)) return false;
         tc_fence_after();
         return true;
       };
@@ -1062,12 +847,10 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
           const uint32_t slot_lo = ring_lo + (q % ring) * slot_step;
           uint32_t blo = w_lo;
           const bool has_next = sl + 1 < p.D || col + col_step < n_cols;
-          if (!(p.debug & 2)) {
 #pragma unroll
-            for (int t9 = 0; t9 < 8; t9++) issue_tap(t9, tmem_d, slot_lo, blo);
-          }
+          for (int t9 = 0; t9 < 8; t9++) issue_tap(t9, tmem_d, slot_lo, blo);
           ready_now = has_next && try_slice(q + 1);      // if it is not there yet, block after this slice's commits
-          if (!(p.debug & 2)) issue_tap(8, tmem_d, slot_lo, blo);
+          issue_tap(8, tmem_d, slot_lo, blo);
           umma_commit(&empty[q % ring]);
           umma_commit(&pfull[q % kPGroups]);
         }
@@ -1084,10 +867,10 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
     const int row = quad * 32 + lane;
     const uint32_t lane_addr = ((uint32_t)(quad * 32) << 16) + (uint32_t)(chalf * CW);
     float bias[CW];
-    // DEPI: the bias is read from shared memory (broadcast), which keeps that epilogue within 128 registers; it sits
-    // behind the scale / shift (UP: Cin = 64, well inside the 2 x 256 floats reserved for them)
+    // UP: the bias is read from shared memory (broadcast), which keeps that epilogue within 128 registers; it sits
+    // behind the scale / shift (Cin = 64, well inside the 2 x 256 floats reserved for them)
     float* s_bias = s_ab + 2 * p.cin;
-    if constexpr (DEPI) {
+    if constexpr (UP) {
       const int e = threadIdx.x - 64;
       if (e < PN) s_bias[e] = (p.bias && part * PN + e < p.cout) ? __ldg(p.bias + part * PN + e) : 0.f;
       named_bar_sync(1, 32 * kSlab3EpiWarps);
@@ -1143,7 +926,7 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
 #pragma unroll
             for (int k = 0; k < 8; k++) f[c8 * 8 + k] += pf[k];
           }
-          if (!DEPI && od + 1 < p.D) load_prev(pvq, od + 1);   // for the next output slice: a whole slice period ahead
+          if (!UP && od + 1 < p.D) load_prev(pvq, od + 1);   // for the next output slice: a whole slice period ahead
         }
 #pragma unroll
         for (int c = 0; c < CW; c++) { ssum[c] += f[c]; ssq[c] = fmaf(f[c], f[c], ssq[c]); }
@@ -1157,13 +940,13 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
         }
         fence_async_smem();
         named_bar_sync(1, 32 * kSlab3EpiWarps);
-        if (is_issuer && !(p.debug & 1)) {
+        if (is_issuer) {
           tma_store_5d(&p.tmap_o, s_out + boff, part * PN, iw * 8, ih * 16, od, n);
           bulk_commit();
         }
         n_out++;
       };
-      if constexpr (DEPI) {
+      if constexpr (UP) {
         // Event s = "group P(s) complete", P(s)[kd] = W(kd) x(s) with x(s) = low-res plane s up-sampled in h and w.  The
         // depth-up-sampled input is h(2i) = 0.75 x(i) + 0.25 x(max(i-1, 0)), h(2i+1) = 0.75 x(i) + 0.25 x(min(i+1, Dl-1)),
         // h(-1) = h(2 Dl) = 0 (conv padding), and out(m) = sum_kd W(kd) h(m+kd-1):
@@ -1172,7 +955,7 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
         // At the first and last slice the clamp and the zero padding only change coefficients.  Event s adds the P(s)
         // terms of pair s-1 and emits it, then starts pair s from P(s-1) and P(s) (P(s-1) is dead after that) and, at
         // the last slice, emits it too.  TMEM blocks are loaded two at a time: the register budget of the 8 warps.
-        static_assert(CW == 16, "DEPI epilogue: 16 columns per warp");
+        static_assert(CW == 16, "UP epilogue: 16 columns per warp");
         float part0[CW], part1[CW];                      // out(2i), out(2i+1) of the pair in flight
         for (int s = 0; s < n_sl; s++) {
           const uint32_t q = q0 + s;
@@ -1254,20 +1037,15 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
           const uint32_t g_cur = lane_addr + (q % kPGroups) * (3 * PN);
           const uint32_t g_prev = lane_addr + ((q + kPGroups - 1) % kPGroups) * (3 * PN);
           uint32_t ra[CW], rb[CW], rc[CW];
-          if (sl >= 1 && !(p.debug & 24)) {
+          if (sl >= 1) {
             if constexpr (CW == 16) { tmem_ld16(g_cur + 2 * PN, ra); tmem_ld16(g_prev, rc); }
             else { tmem_ld8(g_cur + 2 * PN, ra); tmem_ld8(g_prev, rc); }
           } else {
 #pragma unroll
             for (int c = 0; c < CW; c++) { ra[c] = 0u; rc[c] = 0u; }
           }
-          if (!(p.debug & 8)) {
-            if constexpr (CW == 16) tmem_ld16(g_cur + PN, rb);
-            else tmem_ld8(g_cur + PN, rb);
-          } else {
-#pragma unroll
-            for (int c = 0; c < CW; c++) rb[c] = 0u;
-          }
+          if constexpr (CW == 16) tmem_ld16(g_cur + PN, rb);
+          else tmem_ld8(g_cur + PN, rb);
           tmem_ld_wait();
           tc_fence_before();
           __syncwarp();
@@ -1275,7 +1053,6 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
             if (sl >= 1) mbar_arrive(&pempty[(q + kPGroups - 1) % kPGroups]);
             if (sl == p.D - 1) mbar_arrive(&pempty[q % kPGroups]);
           }
-          if (p.debug & 128) continue;                     // ablation: handshakes only
           // out(sl-1) is complete now; out(D-1) completes together with the last event
           if (sl >= 1) {
             float f[CW];
@@ -1364,41 +1141,31 @@ extern "C" int nm_pack_conv_weights(const float* weight, void* packed, int Cout,
 // x: (n, D, H, W, Cin) fp16; packed_w: [k^3][Cout][Cin] fp16; out: (n, OD, OH, OW, Cout) fp16.
 // Supported: (k=1|3, stride 1, pad (k-1)/2) and (k=2, stride 2, pad 0); Cin, Cout multiples of 8; Cout <= 256.
 namespace {
-int slab_mode_env() {
-  static int slab_mode = -1;
-  if (slab_mode < 0) {
-    const char* e = getenv("NM_CONV_SLAB");   // A/B switch for profiling: 0 = tap-streaming kernel only, 1 = no slab3
-    slab_mode = e ? atoi(e) : 2;
-  }
-  return slab_mode;
-}
-// Which kernel serves this conv, and how many GroupNorm partial chunks per sample it can emit (0 = none).
-struct ConvPlan { bool slab, use3; int bk, kch, ntile, pn, ring, chunk_bytes; size_t need, w_bytes, extra; int stats_chunks; };
+// Which kernel serves this conv (slab3: conv3d_slab3_kernel, else conv3d_tc_kernel), and how many GroupNorm partial
+// chunks per sample it can emit (0 = none).
+struct ConvPlan { bool slab3; int bk, kch, ntile, pn, ring, chunk_bytes; size_t need, w_bytes, extra; int stats_chunks; };
 ConvPlan plan_conv(int n, int D, int H, int W, int Cin, int Cout, int k, int stride) {
   ConvPlan pl;
   memset(&pl, 0, sizeof(pl));
-  const int slab_mode = slab_mode_env();
   pl.bk = Cin >= 64 ? 64 : 32;
   pl.kch = (Cin + pl.bk - 1) / pl.bk;
   pl.ntile = ((Cout + 15) / 16) * 16;
   pl.pn = pl.kch == 1 ? 32 : 16;
-  pl.use3 = slab_mode >= 2 && pl.kch <= 2 && Cout % pl.pn == 0 && Cout <= 128;
-  const size_t w_bytes = (size_t)27 * pl.kch * (pl.use3 ? pl.pn : pl.ntile) * pl.bk * 2;
+  const size_t w_bytes = (size_t)27 * pl.kch * pl.pn * pl.bk * 2;
   pl.chunk_bytes = ((kHaloW * kHaloH * pl.bk * 2 + 1023) / 1024) * 1024;
-  pl.ring = pl.use3 ? kSlab3Ring : kSlabRing;
-  const size_t extra = 1024 + 48 * 8 + 16 + 2 * 256 * 4 + (pl.use3 ? (size_t)2 * kTileM * pl.pn * 2 : 0);
-  if (pl.use3)
-    while (pl.ring > 2 && w_bytes + (size_t)pl.ring * pl.kch * pl.chunk_bytes + extra > 227 * 1024) pl.ring--;
+  pl.ring = kSlab3Ring;
+  const size_t extra = 1024 + 48 * 8 + 16 + 2 * 256 * 4 + (size_t)2 * kTileM * pl.pn * 2;
+  while (pl.ring > 2 && w_bytes + (size_t)pl.ring * pl.kch * pl.chunk_bytes + extra > 227 * 1024) pl.ring--;
   pl.need = w_bytes + (size_t)pl.ring * pl.kch * pl.chunk_bytes + extra;
   pl.w_bytes = w_bytes; pl.extra = extra;
   // Measured (B200, 320 frames): with N = Cout >= 128 the tap-streaming kernel amortises the shared-memory A-operand
   // read over a wide MMA and wins over 16-channel slab3 parts: 128->128 @16^3 1.17 vs 1.32 ms, @32^3 (64 clips) 1.87
   // vs 2.11 ms.  (128->64: 8.0 vs 5.1 ms, 64->128: 0.63 vs 0.51 ms - those stay on slab3.)
   const bool wide = Cin >= 128 && Cout >= 128;
-  pl.slab = slab_mode && !wide && k == 3 && stride == 1 && Cin >= 32 && Cin % pl.bk == 0 && W % 8 == 0 && H % 16 == 0 &&
-            pl.need <= 227 * 1024;
-  if (pl.slab) {
-    pl.stats_chunks = pl.use3 ? (H / 16) * (W / 8) * 4 : 0;
+  pl.slab3 = pl.kch <= 2 && Cout % pl.pn == 0 && Cout <= 128 && !wide && k == 3 && stride == 1 && Cin >= 32 &&
+             Cin % pl.bk == 0 && W % 8 == 0 && H % 16 == 0 && pl.need <= 227 * 1024;
+  if (pl.slab3) {
+    pl.stats_chunks = (H / 16) * (W / 8) * 4;
   } else {
     const int OD = D / stride, OH = H / stride, OW = W / stride;
     const int tw = OW < 8 ? OW : 8, th = OH < 4 ? OH : 4, td = OD < 4 ? OD : 4;
@@ -1422,8 +1189,8 @@ extern "C" int nm_conv3d_can_fuse_input(int n, int D, int H, int W, int Cin, int
   // output-channel parts: 32->32 @64^3 4.95 ms plain + 2.23 ms affine pass vs 5.59 ms fused; 64->64 @32^3 1.95 + 0.69 vs
   // 2.05.  For Cin = 128 (8 parts of 16 channels) the separate HBM-bound affine pass is faster.
   const ConvPlan pl = plan_conv(n, D, H, W, Cin, Cout, k, stride);
-  if (pl.slab && pl.use3 && pl.kch == 1 && pl.bk == 32 && Cout <= 32) return 1;
-  return pl.slab && pl.use3 && pl.kch == 1 && pl.bk == 64 && Cout <= 64 ? 1 : 0;
+  if (pl.slab3 && pl.kch == 1 && pl.bk == 32 && Cout <= 32) return 1;
+  return pl.slab3 && pl.kch == 1 && pl.bk == 64 && Cout <= 64 ? 1 : 0;
 }
 
 extern "C" int nm_conv3d_tc_fused(const void* x, const void* packed_w, const float* bias, void* out, int n, int D,
@@ -1445,7 +1212,7 @@ bool up2x_ok(int n, int D, int H, int W, int Cin, int Cout) {
   if ((D | H | W) & 1) return false;
   if (Cin == 128) Cin = 64;   // split-K: two launches over 64-channel slices of the low-resolution tensor
   const ConvPlan pl = plan_conv(n, D, H, W, Cin, Cout, 3, 1);
-  return pl.slab && pl.use3 && pl.bk == 64 && pl.kch == 1 && pl.pn == 32 &&
+  return pl.slab3 && pl.bk == 64 && pl.kch == 1 && pl.pn == 32 &&
          pl.w_bytes + (size_t)3 * pl.chunk_bytes + kLoRing * kLoBytes + pl.extra <= 227 * 1024;
 }
 }  // namespace
@@ -1494,10 +1261,9 @@ int conv3d_tc_impl(const void* x, const void* packed_w, const float* bias, void*
   // resident a CTA can only serve 16 output channels (N = 48 per MMA, 58 cycles for 24 cycles of tensor work); one
   // chunk at a time allows 32-channel parts (N = 96, 92 cycles for 48).  The second launch adds the fp16 partial sum
   // the first one left in `out`; GroupNorm statistics come from the second.
-  if (!up && !in_scale && cin_total == Cin && Cin == 128 && Cout % 32 == 0 && Cout <= 64 && k == 3 && stride == 1 && n > 0 &&
-      !getenv("NM_NO_SPLITK")) {
+  if (!up && !in_scale && cin_total == Cin && Cin == 128 && Cout % 32 == 0 && Cout <= 64 && k == 3 && stride == 1 && n > 0) {
     const ConvPlan half = plan_conv(n, D, H, W, 64, Cout, k, stride);
-    if (half.slab && half.use3 && half.pn == 32) {
+    if (half.slab3 && half.pn == 32) {
       const int rc = conv3d_tc_impl(x, packed_w, bias, out, n, D, H, W, 64, Cout, k, stride, nullptr, nullptr, 0, nullptr,
                                     stream, false, 128, 0, 0);
       if (rc != NM_OK) return rc;
@@ -1516,7 +1282,7 @@ int conv3d_tc_impl(const void* x, const void* packed_w, const float* bias, void*
     nm_set_error("nm_conv3d_tc: cuTensorMapEncodeTiled entry point not available");
     return NM_ERR_DRIVER;
   }
-  // ---- slab-walking kernels: k3, weights resident in smem
+  // ---- slab-walking kernel: k3, weights resident in smem
   ConvPlan pl = plan_conv(n, D, H, W, Cin, Cout, k, stride);
   if (up) {
     pl.ring = 3;
@@ -1524,100 +1290,77 @@ int conv3d_tc_impl(const void* x, const void* packed_w, const float* bias, void*
   }
   NM_CHECK_ARG(!stats_partial || pl.stats_chunks > 0, "nm_conv3d_tc: this shape cannot fuse GroupNorm statistics");
   NM_CHECK_ARG((in_scale == nullptr) == (in_shift == nullptr), "nm_conv3d_tc: in_scale and in_shift go together");
-  NM_CHECK_ARG(!in_scale || (pl.slab && pl.use3 && Cin <= 256),
+  NM_CHECK_ARG(!in_scale || (pl.slab3 && Cin <= 256),
                "nm_conv3d_tc: this shape cannot fuse the input transform (see nm_conv3d_can_fuse_input)");
-  {
+  if (pl.slab3) {
     const int bk = pl.bk, kch = pl.kch, ntile = pl.ntile, pn = pl.pn, ring = pl.ring, chunk_bytes = pl.chunk_bytes;
-    const bool use3 = pl.use3;
     const size_t need = pl.need;
-    if (pl.slab) {
-      ConvSlabParams q;
-      memset(&q, 0, sizeof(q));
-      q.kchunks = kch; q.block_k = bk; q.n_tile = ntile; q.cout = Cout;
-      q.nw = W / 8; q.nh = H / 16; q.D = D; q.H = H; q.W = W; q.N = n;
-      q.chunk_bytes = chunk_bytes; q.slot_bytes = kch * chunk_bytes; q.ring = ring;
-      { const char* dbg = getenv("NM_SLAB_DEBUG"); q.debug = dbg ? atoi(dbg) : 0; }
-      q.bias = bias; q.out = (act_t*)out; q.stats = use3 ? stats_partial : nullptr;
-      q.in_scale = in_scale; q.in_shift = in_shift; q.in_act = in_act; q.cin = Cin;
-      q.cin_off = cin_off; q.accum = accum;
-      NM_CHECK_ARG(cin_total == Cin || use3, "nm_conv3d_tc: split-K needs the slab3 kernel");
-      const CUtensorMapSwizzle swz = bk == 64 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B;
-      const cuuint64_t ct = (cuuint64_t)cin_total;
-      cuuint64_t dims[5] = {ct, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)D, (cuuint64_t)n};
-      cuuint64_t strides[4] = {ct * 2, (cuuint64_t)W * ct * 2, (cuuint64_t)H * W * ct * 2, (cuuint64_t)D * H * W * ct * 2};
-      cuuint32_t box[5] = {(cuuint32_t)bk, kHaloW, kHaloH, 1, 1};
-      cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-      if (up) {   // the low-resolution tensor, (10 x 6)-row planes, linear rows (read by the transform warps)
-        dims[1] = W / 2; dims[2] = H / 2; dims[3] = D / 2;
-        strides[1] = (cuuint64_t)(W / 2) * ct * 2; strides[2] = (cuuint64_t)(H / 2) * (W / 2) * ct * 2;
-        strides[3] = (cuuint64_t)(D / 2) * (H / 2) * (W / 2) * ct * 2;
-        box[1] = 6; box[2] = 10;
-      }
-      CUresult r = encode(&q.tmap_a, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 5, (void*)x, dims, strides, box, estr,
-                          CU_TENSOR_MAP_INTERLEAVE_NONE, up ? CU_TENSOR_MAP_SWIZZLE_NONE : swz,
-                          CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-      if (r != CUDA_SUCCESS) { nm_set_error("nm_conv3d_tc(slab): cuTensorMapEncodeTiled(A) failed with %d", (int)r); return NM_ERR_DRIVER; }
-      cuuint64_t wdims[3] = {ct, (cuuint64_t)Cout, 27};
-      cuuint64_t wstrides[2] = {ct * 2, ct * Cout * 2};
-      cuuint32_t wbox[3] = {(cuuint32_t)bk, (cuuint32_t)(use3 ? pn : ntile), 1};
-      cuuint32_t westr[3] = {1, 1, 1};
-      r = encode(&q.tmap_b, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, (void*)packed_w, wdims, wstrides, wbox, westr,
-                 CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-      if (r != CUDA_SUCCESS) { nm_set_error("nm_conv3d_tc(slab): cuTensorMapEncodeTiled(W) failed with %d", (int)r); return NM_ERR_DRIVER; }
-      if (use3) {
-        cuuint64_t odims[5] = {(cuuint64_t)Cout, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)D, (cuuint64_t)n};
-        cuuint64_t ostrides[4] = {(cuuint64_t)Cout * 2, (cuuint64_t)W * Cout * 2, (cuuint64_t)H * W * Cout * 2,
-                                  (cuuint64_t)D * H * W * Cout * 2};
-        cuuint32_t obox[5] = {(cuuint32_t)pn, 8, 16, 1, 1};
-        r = encode(&q.tmap_o, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 5, out, odims, ostrides, obox, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, pn == 32 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B,
-                   CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) { nm_set_error("nm_conv3d_tc(slab3): cuTensorMapEncodeTiled(out) failed with %d", (int)r); return NM_ERR_DRIVER; }
-      }
-      NM_PER_DEVICE_ONCE({
-        NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-        NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-      });
-      const int cols = n * q.nh * q.nw;
-      int grid = cols < nm_num_sms() ? cols : nm_num_sms();
-      if (use3) {
-        const int parts = ntile / pn;
-        grid = cols * parts < nm_num_sms() ? cols * parts : (nm_num_sms() / parts) * parts;
-        NM_PER_DEVICE_ONCE({
-          NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab3_kernel<64, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-          NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab3_kernel<32, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-          NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab3_kernel<64, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-          NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab3_kernel<64, 32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-          NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab3_kernel<64, 32, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-          NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab3_kernel<64, 32, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-          NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab3_kernel<64, 32, true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-          NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab3_kernel<64, 32, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-        });
-        static int xw_env = -1;
-        if (xw_env < 0) { const char* e = getenv("NM_XFORM_WARPS"); xw_env = e ? atoi(e) : 6; if (xw_env != 4) xw_env = 6; }
-        // the up-sampling producer runs on 4 warps (3 working): with 6 (5 working, 144 finer items) dec.8 got slower
-        // [measured, same GPU: 20.4 -> 24.6 ms per 640 frames] - more producer threads take issue slots and shared-memory
-        // bandwidth from the MMA / epilogue warps; the in-place transform gains from 6 (13.2 -> 11.6 ms)
-        const int threads3 = kSlab3Threads + (up ? 32 * kUpWarps : (in_scale ? 32 * xw_env : 0));
-        // NM_UP_DEPTH_EPI=0: the up-sampling producer blends two planes per output slice (A/B switch, read per call)
-        const char* depi_env = getenv("NM_UP_DEPTH_EPI");
-        const bool depi = up && !(depi_env && strcmp(depi_env, "0") == 0);
-        if (accum) {
-          NM_CHECK_ARG(bk == 64 && pn == 32 && !in_scale, "nm_conv3d_tc: split-K accumulation needs slab3<64, 32>");
-          if (depi) conv3d_slab3_kernel<64, 32, true, true, true><<<grid, threads3, need, (cudaStream_t)stream>>>(q);
-          else if (up) conv3d_slab3_kernel<64, 32, true, true><<<grid, threads3, need, (cudaStream_t)stream>>>(q);
-          else conv3d_slab3_kernel<64, 32, false, true><<<grid, threads3, need, (cudaStream_t)stream>>>(q);
-        } else if (depi) conv3d_slab3_kernel<64, 32, true, false, true><<<grid, threads3, need, (cudaStream_t)stream>>>(q);
-        else if (up) conv3d_slab3_kernel<64, 32, true><<<grid, threads3, need, (cudaStream_t)stream>>>(q);
-        else if (pn == 16) conv3d_slab3_kernel<64, 16><<<grid, threads3, need, (cudaStream_t)stream>>>(q);
-        else if (bk == 64) conv3d_slab3_kernel<64, 32><<<grid, threads3, need, (cudaStream_t)stream>>>(q);
-        else conv3d_slab3_kernel<32, 32><<<grid, threads3, need, (cudaStream_t)stream>>>(q);
-      } else if (bk == 64) conv3d_slab_kernel<64><<<grid, 192, need, (cudaStream_t)stream>>>(q);
-      else conv3d_slab_kernel<32><<<grid, 192, need, (cudaStream_t)stream>>>(q);
-      NM_CHECK_LAUNCH("conv3d_slab");
-      return NM_OK;
+    ConvSlabParams q;
+    memset(&q, 0, sizeof(q));
+    q.kchunks = kch; q.block_k = bk; q.n_tile = ntile; q.cout = Cout;
+    q.nw = W / 8; q.nh = H / 16; q.D = D; q.H = H; q.W = W; q.N = n;
+    q.chunk_bytes = chunk_bytes; q.slot_bytes = kch * chunk_bytes; q.ring = ring;
+    q.bias = bias; q.out = (act_t*)out; q.stats = stats_partial;
+    q.in_scale = in_scale; q.in_shift = in_shift; q.in_act = in_act; q.cin = Cin;
+    q.cin_off = cin_off; q.accum = accum;
+    const CUtensorMapSwizzle swz = bk == 64 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B;
+    const cuuint64_t ct = (cuuint64_t)cin_total;
+    cuuint64_t dims[5] = {ct, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)D, (cuuint64_t)n};
+    cuuint64_t strides[4] = {ct * 2, (cuuint64_t)W * ct * 2, (cuuint64_t)H * W * ct * 2, (cuuint64_t)D * H * W * ct * 2};
+    cuuint32_t box[5] = {(cuuint32_t)bk, kHaloW, kHaloH, 1, 1};
+    cuuint32_t estr[5] = {1, 1, 1, 1, 1};
+    if (up) {   // the low-resolution tensor, (10 x 6)-row planes, linear rows (read by the transform warps)
+      dims[1] = W / 2; dims[2] = H / 2; dims[3] = D / 2;
+      strides[1] = (cuuint64_t)(W / 2) * ct * 2; strides[2] = (cuuint64_t)(H / 2) * (W / 2) * ct * 2;
+      strides[3] = (cuuint64_t)(D / 2) * (H / 2) * (W / 2) * ct * 2;
+      box[1] = 6; box[2] = 10;
     }
+    CUresult r = encode(&q.tmap_a, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 5, (void*)x, dims, strides, box, estr,
+                        CU_TENSOR_MAP_INTERLEAVE_NONE, up ? CU_TENSOR_MAP_SWIZZLE_NONE : swz,
+                        CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS) { nm_set_error("nm_conv3d_tc(slab3): cuTensorMapEncodeTiled(A) failed with %d", (int)r); return NM_ERR_DRIVER; }
+    cuuint64_t wdims[3] = {ct, (cuuint64_t)Cout, 27};
+    cuuint64_t wstrides[2] = {ct * 2, ct * Cout * 2};
+    cuuint32_t wbox[3] = {(cuuint32_t)bk, (cuuint32_t)pn, 1};
+    cuuint32_t westr[3] = {1, 1, 1};
+    r = encode(&q.tmap_b, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, (void*)packed_w, wdims, wstrides, wbox, westr,
+               CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS) { nm_set_error("nm_conv3d_tc(slab3): cuTensorMapEncodeTiled(W) failed with %d", (int)r); return NM_ERR_DRIVER; }
+    cuuint64_t odims[5] = {(cuuint64_t)Cout, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)D, (cuuint64_t)n};
+    cuuint64_t ostrides[4] = {(cuuint64_t)Cout * 2, (cuuint64_t)W * Cout * 2, (cuuint64_t)H * W * Cout * 2,
+                              (cuuint64_t)D * H * W * Cout * 2};
+    cuuint32_t obox[5] = {(cuuint32_t)pn, 8, 16, 1, 1};
+    r = encode(&q.tmap_o, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 5, out, odims, ostrides, obox, estr,
+               CU_TENSOR_MAP_INTERLEAVE_NONE, pn == 32 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B,
+               CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS) { nm_set_error("nm_conv3d_tc(slab3): cuTensorMapEncodeTiled(out) failed with %d", (int)r); return NM_ERR_DRIVER; }
+    const int cols = n * q.nh * q.nw;
+    const int parts = ntile / pn;
+    const int grid = cols * parts < nm_num_sms() ? cols * parts : (nm_num_sms() / parts) * parts;
+    NM_PER_DEVICE_ONCE({
+      NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab3_kernel<64, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+      NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab3_kernel<32, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+      NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab3_kernel<64, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+      NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab3_kernel<64, 32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+      NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab3_kernel<64, 32, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+      NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab3_kernel<64, 32, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+    });
+    // the up-sampling producer runs on 4 warps (3 working): with 6 (5 working, 144 finer items) dec.8 got slower
+    // [measured, same GPU: 20.4 -> 24.6 ms per 640 frames] - more producer threads take issue slots and shared-memory
+    // bandwidth from the MMA / epilogue warps; the in-place transform gains from 6 (13.2 -> 11.6 ms)
+    const int threads3 = kSlab3Threads + (up ? 32 * kUpWarps : (in_scale ? 32 * kSlab3XformWarps : 0));
+    if (accum) {
+      NM_CHECK_ARG(bk == 64 && pn == 32 && !in_scale, "nm_conv3d_tc: split-K accumulation needs slab3<64, 32>");
+      if (up) conv3d_slab3_kernel<64, 32, true, true><<<grid, threads3, need, (cudaStream_t)stream>>>(q);
+      else conv3d_slab3_kernel<64, 32, false, true><<<grid, threads3, need, (cudaStream_t)stream>>>(q);
+    } else if (up) conv3d_slab3_kernel<64, 32, true><<<grid, threads3, need, (cudaStream_t)stream>>>(q);
+    else if (pn == 16) conv3d_slab3_kernel<64, 16><<<grid, threads3, need, (cudaStream_t)stream>>>(q);
+    else if (bk == 64) conv3d_slab3_kernel<64, 32><<<grid, threads3, need, (cudaStream_t)stream>>>(q);
+    else conv3d_slab3_kernel<32, 32><<<grid, threads3, need, (cudaStream_t)stream>>>(q);
+    NM_CHECK_LAUNCH("conv3d_slab3");
+    return NM_OK;
   }
+  NM_CHECK_ARG(cin_total == Cin, "nm_conv3d_tc: split-K needs the slab3 kernel");
   ConvTcParams p;
   memset(&p, 0, sizeof(p));
   const int pad = stride == 1 ? (k - 1) / 2 : 0;

@@ -13,7 +13,6 @@
 // discrete decision; keep it as close to the reference arithmetic as possible).
 #include "common.cuh"
 #include "../../include/nm_b200.h"
-#include <stdlib.h>
 
 namespace {
 
@@ -729,9 +728,8 @@ extern "C" int nm_hsvrnn_step(const nm_hsvrnn_weights* w, const float* h_in, con
   a.B = B; a.K = K; a.S = S; a.posterior = posterior;
   cudaStream_t st = (cudaStream_t)stream;
   // small and medium batches: a cluster of 8 CTAs per element (weights split over the ranks, DSMEM broadcasts)
-  static const bool use_cluster = []() { const char* e = getenv("NM_HSVRNN_CLUSTER"); return !(e && atoi(e) == 0); }();
-  // measured (tools/time_rollout.py, us per step): B = 1: 30 vs 216, B = 16: 59 vs 228, B = 64: 144 vs 235, B = 256: 510 vs 240
-  if (use_cluster && S <= 10 && B <= 96) {
+  // measured, cluster vs one-CTA-per-element kernel (us per step): B = 1: 30 vs 216, B = 16: 59 vs 228, B = 64: 144 vs 235, B = 256: 510 vs 240
+  if (S <= 10 && B <= 96) {
     const int SV = S == 1 ? 1 : 10;
     const size_t smem = (size_t)cl_layout(SV).total * sizeof(float);
     if (SV == 1) {

@@ -40,8 +40,6 @@ def frames_per_pass(grid_size: int) -> int:
     return max(1, FRAME_CHUNK * 64 ** 3 // grid_size ** 3)
 # Run the once-per-clip spatio-temporal branch on an auxiliary stream next to the per-frame encoder (0 disables).
 ST_OVERLAP = __import__("os").environ.get("NM_ST_OVERLAP", "1") != "0"
-# Interpolate the first decoder up-sampling inside the dec.1 conv as well (0: separate up-sampling kernel).
-UP_DEC1 = __import__("os").environ.get("NM_UP_DEC1", "1") != "0"
 
 
 def _training(module) -> bool:
@@ -248,7 +246,7 @@ class KyptToVoxNet(nn.Module):
                 gs = gaussians[b0:b1].float().contiguous().view(n, K, g, g, g) if keypoints is None else None
                 x = ops.decoder_adjust(first_feature_act[b0:b1], self.adjust_combined_representation[0], T, g, K,
                                        sigma, keypoints=kp, gaussians=gs)
-                if UP_DEC1 and ops.can_conv_up2x(x, dec[1]):
+                if ops.can_conv_up2x(x, dec[1]):
                     raw, a, b = ops.conv3d_up2x(x, dec[1], dec[2])     # up-sampling inside the conv's operand path
                 else:
                     raw, a, b = ops.conv3d(ops.upsample2x(x), dec[1], dec[2])

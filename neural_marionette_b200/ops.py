@@ -5,7 +5,6 @@ from __future__ import annotations
 
 import ctypes
 import math
-import os
 from typing import Optional, Tuple
 
 import torch
@@ -311,9 +310,6 @@ def _slab_wgrad_ok(x, Cout) -> bool:
     return Cin % 32 == 0 and Cout % 32 == 0 and Cin <= 256 and Cout <= 256 and W in (16, 32, 48, 64)
 
 
-WGRAD_TC = __import__("os").environ.get("NM_WGRAD_TC", "1") != "0"
-
-
 def conv3d_weight_grad(x: torch.Tensor, grad_out: torch.Tensor, k: int = 3, stride: int = 1,
                        out_scale: float = 1.0, force_gather: bool = False, impl: Optional[str] = None) -> torch.Tensor:
     """dL/dW of an nn.Conv3d ((k, stride) in {(1, 1), (3, 1), (2, 2)}): x act (n, D, H, W, Cin), grad_out act
@@ -328,7 +324,7 @@ def conv3d_weight_grad(x: torch.Tensor, grad_out: torch.Tensor, k: int = 3, stri
     if force_gather:
         impl = "gather"
     tc_ok = k == 3 and stride == 1 and bool(L.query("nm_conv3d_k3_wgrad_tc_supported", n, D, H, W, Cin, Cout))
-    if impl == "tc" or (impl is None and WGRAD_TC and tc_ok):
+    if impl == "tc" or (impl is None and tc_ok):
         nbytes = L.query("nm_conv3d_k3_wgrad_tc_workspace_bytes", n, D, H, W, Cin, Cout)
         ws = workspace(max(nbytes, 16), x.device, "wgrad")
         if PROFILE is not None:
@@ -539,10 +535,8 @@ def conv3d_up2x(x_lo: torch.Tensor, conv: torch.nn.Conv3d, gn: Optional[torch.nn
     if PROFILE is not None:
         e1.record()
         # what the tensor cores execute: the depth half of the up-sampling is applied to the accumulators (MMAs over
-        # the D low-resolution slices), unless NM_UP_DEPTH_EPI=0 selects the two-plane operand producer
-        flops = 2.0 * n * 8 * D * H * W * Cout * Cin * 27
-        if os.environ.get("NM_UP_DEPTH_EPI", "1") != "0":
-            flops /= 2
+        # the D low-resolution slices)
+        flops = 2.0 * n * 8 * D * H * W * Cout * Cin * 27 / 2
         PROFILE.setdefault(("conv", n, 2 * D, Cin, Cout, 3, 1, flops), []).append((e0, e1))
     if gn is None:
         return out

@@ -101,6 +101,7 @@ CONV_CASES = [
     (1, 16, 128, 64, 3, 1), (1, 8, 128, 256, 3, 1), (1, 8, 256, 256, 1, 1), (3, 4, 48, 48, 3, 1),
     (5, 2, 72, 72, 3, 1), (20, 2, 48, 72, 3, 1), (2, 16, 32, 32, 2, 2), (2, 8, 64, 64, 2, 2),
     (3, 4, 48, 48, 2, 2), (1, 32, 32, 32, 3, 1), (2, 8, 32, 64, 1, 1), (3, 2, 48, 48, 2, 2),
+    (2, 16, 32, 48, 3, 1), (1, 16, 64, 16, 3, 1),   # k3 at 16^3, Cout not a multiple of 32: conv3d_tc_kernel
 ]
 
 

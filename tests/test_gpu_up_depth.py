@@ -1,8 +1,7 @@
 """conv3d_k3(upsample2x(x)) with the depth half of the up-sampling applied to the accumulators (nm_conv3d_tc_up2x):
 the MMAs run over the low-resolution depth and the epilogue blends the TMEM groups of neighbouring slices.  Checked
-against torch (F.interpolate trilinear + F.conv3d on fp16-rounded weights), against the two-plane operand producer
-(NM_UP_DEPTH_EPI=0), for the GroupNorm statistics of the epilogue and for run-to-run bit identity.  Shapes are the
-decoder's dec.8 (64 -> 32) and dec.1 (128 -> 64, split-K) channel counts, plus depths where every slice is a border
+against torch (F.interpolate trilinear + F.conv3d on fp16-rounded weights), for the GroupNorm statistics of the
+epilogue and for run-to-run bit identity.  Shapes are the decoder's dec.8 (64 -> 32) and dec.1 (128 -> 64, split-K) channel counts, plus depths where every slice is a border
 slice (low-resolution depth 1 and 2)."""
 import pytest
 import torch
@@ -56,7 +55,7 @@ def _setup(n, dl, hl, wl, cin, cout, seed):
 
 
 @pytest.mark.parametrize("n,dl,hl,wl,cin,cout,fused", CASES)
-def test_up2x_depth_epilogue(ops, monkeypatch, n, dl, hl, wl, cin, cout, fused):
+def test_up2x_depth_epilogue(ops, n, dl, hl, wl, cin, cout, fused):
     conv, gn_out, raw, a, b = _setup(n, dl, hl, wl, cin, cout, seed=dl * 7 + hl + cin + cout)
     assert ops.can_conv_up2x(raw, conv)
     ia = (a, b, True) if fused else None
@@ -67,16 +66,12 @@ def test_up2x_depth_epilogue(ops, monkeypatch, n, dl, hl, wl, cin, cout, fused):
         torch.cuda.synchronize()
         return out.clone(), ga.clone(), gb.clone()
 
-    monkeypatch.setenv("NM_UP_DEPTH_EPI", "1")
     got, ga, gb = run()
     again, ga2, gb2 = run()
-    monkeypatch.setenv("NM_UP_DEPTH_EPI", "0")
-    old, _, _ = run()
 
     ref = F.conv3d(F.interpolate(from_act(act), scale_factor=2.0, mode="trilinear", align_corners=False),
                    conv.weight.detach().cpu().half().float(), conv.bias.detach().cpu(), padding=1)
     assert rel_err(from_act(got), ref) < 3e-3
-    assert rel_err(from_act(got), from_act(old)) < 3e-3
     # the epilogue's GroupNorm statistics describe the tensor it wrote
     ta, tb = ops.gn_scale_shift(got, gn_out)
     assert (ga - ta).abs().max() <= 3e-3 * ta.abs().max() and (gb - tb).abs().max() <= 3e-3 * (1 + tb.abs().max())
@@ -84,18 +79,16 @@ def test_up2x_depth_epilogue(ops, monkeypatch, n, dl, hl, wl, cin, cout, fused):
     assert torch.equal(got, again) and torch.equal(ga, ga2) and torch.equal(gb, gb2)
 
 
-def test_up2x_profile_counts_executed_flops(ops, monkeypatch):
+def test_up2x_profile_counts_halved_flops(ops):
     """The profiling record carries the FLOPs the tensor cores execute (half of the up-sampled conv's count with the
     depth epilogue), so a layer's rate stays a hardware rate."""
     conv, _, raw, _, _ = _setup(1, 4, 8, 8, 64, 32, seed=3)
     full = 2.0 * 8 * 4 * 8 * 8 * 32 * 64 * 27
     prev = ops.PROFILE
     try:
-        for env, flops in (("1", full / 2), ("0", full)):
-            monkeypatch.setenv("NM_UP_DEPTH_EPI", env)
-            ops.PROFILE = {}
-            ops.conv3d_up2x(raw, conv)
-            torch.cuda.synchronize()
-            assert [k[-1] for k in ops.PROFILE] == [flops]
+        ops.PROFILE = {}
+        ops.conv3d_up2x(raw, conv)
+        torch.cuda.synchronize()
+        assert [k[-1] for k in ops.PROFILE] == [full / 2]
     finally:
         ops.PROFILE = prev

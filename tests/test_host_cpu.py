@@ -154,6 +154,16 @@ def test_product_never_imports_the_oracle():
                 assert "oracle" not in src.replace("the oracle", ""), f"{f} references oracle/"
 
 
+def test_kernel_choice_ignores_the_environment():
+    """Which kernel runs, and what it computes, follows from the arguments alone: no CUDA source reads an environment variable."""
+    csrc = os.path.join(ROOT, "neural_marionette_b200", "csrc")
+    for base, _, files in os.walk(csrc):
+        for f in files:
+            if f.endswith((".cu", ".cuh")):
+                src = open(os.path.join(base, f)).read()
+                assert not re.search(r"\bgetenv\s*\(", src), f"{f} calls getenv"
+
+
 def test_new_entry_points_reject_cpu_tensors():
     """No CPU fallback anywhere: the §8f#4 consumers and the backward bricks raise on CPU tensors."""
     import numpy as np

@@ -1,5 +1,5 @@
-"""Device time of the HSVRNN roll-out (5 conditioned + 15 generated steps) at several batch sizes, with the cluster
-kernel and (NM_HSVRNN_CLUSTER=0) the one-CTA-per-element kernel: CUDA events around `HSVRNNBVH.generate`, and the same
+"""Device time of the HSVRNN roll-out (5 conditioned + 15 generated steps) at several batch sizes (the cluster kernel
+serves B <= 96, the one-CTA-per-element kernel B = 256): CUDA events around `HSVRNNBVH.generate`, and the same
 roll-out replayed as a CUDA graph (what a latency-bound caller would do; the draws are injected so the graph is static)."""
 import os
 import sys
