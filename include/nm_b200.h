@@ -195,6 +195,43 @@ typedef struct nm_hsvrnn_weights {
 int nm_hsvrnn_step(const nm_hsvrnn_weights* w, const float* h_in, const float* kp, const float* eps, const float* offset,
                    const int* order, const int* parents, int B, int K, int S, int posterior, float* h_out,
                    float* kp_out, float* z_out, float* R_out, float* post_out, float* prior_out, void* stream);
+/* nm_hsvrnn_step that also records, in pick_out (B) int32 (nullable), which of the S samples each element fed to the GRU.
+ * The arithmetic is that of nm_hsvrnn_step. */
+int nm_hsvrnn_step_record(const nm_hsvrnn_weights* w, const float* h_in, const float* kp, const float* eps,
+                          const float* offset, const int* order, const int* parents, int B, int K, int S, int posterior,
+                          float* h_out, float* kp_out, float* z_out, float* R_out, float* post_out, float* prior_out,
+                          int* pick_out, void* stream);
+/* ---- stage-2 training: backward of HSVRNNBVH.encode (hsvrnn_bvh.py:67-156), one call per step from t = T-1 down to 0.
+ * wt: the weights as for nm_hsvrnn_step ([in][out]); w: the same struct pointing at the fp32 parameters in their own
+ * [out][in] layout (nn.Linear.weight, GRUCell.weight_ih / weight_hh).  Saved from the forward of step t: h (B,512) = h_t,
+ * kp (B,4K), eps (S,B,128), pick (B) from nm_hsvrnn_step_record, f (B,4K) / z (B,128) / R (B,K,9) the step's kp_out /
+ * z_out / R_out, offset (B,K,3).  Incoming gradients: dh_next (B,512) of h_{t+1}, already including the external gradient
+ * of h_{t+1}; nullable: dh_ext (B,512) the external gradient of h_t, df (B,4K), dR (B,K,9), dz (B,128), dpost / dprior
+ * (B,256) of (mean | std).  Outputs: dh_out (B,512) the full gradient of h_t; doffset (B,K,3) is ACCUMULATED into; rows
+ * (B x nm_hsvrnn_backward_workspace_bytes(1, 1) bytes) is this step's slice of the workspace, read later by
+ * nm_hsvrnn_weight_grads.  No gradient flows to kp. */
+size_t nm_hsvrnn_backward_workspace_bytes(int B, int T);
+int nm_hsvrnn_step_backward(const nm_hsvrnn_weights* wt, const nm_hsvrnn_weights* w, const float* h, const float* kp,
+                            const float* eps, const int* pick, const float* f, const float* z, const float* R,
+                            const float* offset, const int* order, const int* parents, int B, int K, int S,
+                            const float* dh_next, const float* dh_ext, const float* df, const float* dR, const float* dz,
+                            const float* dpost, const float* dprior, float* dh_out, float* doffset, float* rows,
+                            void* stream);
+/* Gradients of the parameters in their own layouts ([out][in] weights), fully overwritten. */
+typedef struct nm_hsvrnn_grads {
+  float *post0_w, *post0_b, *post2_w, *post2_b, *prior0_w, *prior0_b, *prior2_w, *prior2_b;
+  float *root0_w, *root0_b, *root2_w, *root2_b, *joint0_w, *joint0_b, *joint2_w, *joint2_b;
+  float *gru_ih_w, *gru_hh_w, *gru_ih_b, *gru_hh_b;
+  float* init_state;     /* (512): sum over b of dh_0 */
+  float* offset_param;   /* (K,3) or null (offset_param frozen) */
+} nm_hsvrnn_grads;
+/* After the reverse loop: one launch computes every weight / bias gradient over the T*B rows (r = t*B + b) of `rows`
+ * (the whole workspace) in a fixed order - no atomics, bit-reproducible - plus the init-state gradient from dh0 (B,512)
+ * and, when g->offset_param is set, the offset_param gradient from offset / doffset (B,K,3) and offset_param (K,3).
+ * h (T+1,B,512) or at least its first T*B rows, kp / f (T,B,4K), z (T,B,128): the forward's per-step tensors. */
+int nm_hsvrnn_weight_grads(const float* rows, const float* h, const float* kp, const float* f, const float* z,
+                           const float* dh0, const float* offset, const float* doffset, const float* offset_param, int B,
+                           int T, int K, const nm_hsvrnn_grads* g, void* stream);
 /* extract_kypt_from_latent_and_state (hsvrnn_bvh.py:255-286): dec_in (B, 640) -> flat (B, 4K), R (B, K, 9) */
 int nm_hsvrnn_decode_pose(const nm_hsvrnn_weights* w, const float* dec_in, const float* offset, const int* order,
                           const int* parents, int B, int K, float* flat_out, float* R_out, void* stream);

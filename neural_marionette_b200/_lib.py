@@ -27,6 +27,13 @@ class HsvrnnWeights(C.Structure):
         "gru_ih_wt", "gru_hh_wt", "gru_ih_b", "gru_hh_b")]
 
 
+class HsvrnnGrads(C.Structure):
+    _fields_ = [(n, _vp) for n in (
+        "post0_w", "post0_b", "post2_w", "post2_b", "prior0_w", "prior0_b", "prior2_w", "prior2_b",
+        "root0_w", "root0_b", "root2_w", "root2_b", "joint0_w", "joint0_b", "joint2_w", "joint2_b",
+        "gru_ih_w", "gru_hh_w", "gru_ih_b", "gru_hh_b", "init_state", "offset_param")]
+
+
 # name -> (restype, argtypes); every symbol declared in include/nm_b200.h
 PROTOTYPES = {
     "nm_last_error": (C.c_char_p, []),
@@ -78,6 +85,12 @@ PROTOTYPES = {
     "nm_decoder_adjust": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _f, _vp, _vp, _vp]),
     "nm_hsvrnn_step": (_i, [C.POINTER(HsvrnnWeights), _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i,
                             _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "nm_hsvrnn_step_record": (_i, [C.POINTER(HsvrnnWeights), _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i,
+                                   _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "nm_hsvrnn_backward_workspace_bytes": (_sz, [_i, _i]),
+    "nm_hsvrnn_step_backward": (_i, [C.POINTER(HsvrnnWeights), C.POINTER(HsvrnnWeights)] + [_vp] * 10 + [_i, _i, _i] +
+                                [_vp] * 11),
+    "nm_hsvrnn_weight_grads": (_i, [_vp] * 9 + [_i, _i, _i, C.POINTER(HsvrnnGrads), _vp]),
     "nm_hsvrnn_decode_pose": (_i, [C.POINTER(HsvrnnWeights), _vp, _vp, _vp, _vp, _i, _i, _vp, _vp, _vp]),
     "nm_hsvrnn_bone_offsets": (_i, [_vp, _vp, _vp, _i, _i, _i, _vp, _vp]),
     "nm_voxel_chamfer_workspace_bytes": (_sz, [_i, _i]),

@@ -13,6 +13,10 @@ has it divided out again, so `param.grad` holds true values as with the referenc
   Upsample2x         nn.Upsample(scale 2, trilinear)                              kypt_detector.py:427,441
   ConvGNFinalRecon   last 3x3x3 conv + GN + LReLU + 1x1 conv + sigmoid/tanh + BCE kypt_detector.py:450-457,410,91-92
   ChamferVolFit      get_volume_fitting_loss('chamfer')                           utils/kypt_detector_utils.py:141-157
+
+and, for stage 2 (training the dynamics module, reference train.py:146-147), fp32 throughout with no loss scale:
+
+  HSVRNNEncode       the conditioned roll-out of HSVRNNBVH.encode                 model/hsvrnn_bvh.py:67-156
 """
 from __future__ import annotations
 
@@ -251,6 +255,66 @@ class ChamferVolFit(torch.autograd.Function):
     def backward(ctx, dout):
         frames, kp = ctx.saved_tensors
         return None, ops.chamfer_vol_fit_backward(frames, kp, _c(dout.float()))
+
+
+class HSVRNNEncode(torch.autograd.Function):
+    """The T recorded steps of `HSVRNNBVH.encode` (the eval loop, plus the pick of every element) -> per-step tensors
+    f (B, T, K, 4), R (B, T, K, 3, 3), z (B, T, Z), h (B, T+1, H), post / prior (T, B, 2Z) = mean | std.  The backward
+    runs `nm_hsvrnn_step_backward` from t = T-1 down to 0, then `nm_hsvrnn_weight_grads` once.  `params` are
+    `ops.hsvrnn_params(mod)`, so autograd routes their gradients into `param.grad`; keypoints get none."""
+
+    @staticmethod
+    def forward(ctx, kp, eps, mod, *params):
+        B, T, K, _ = kp.shape
+        S, Z, H = eps.shape[1], mod.nlatent_kypt, mod.nhidden_kypt
+        dev = kp.device
+        order, parents = mod._tree(dev)
+        w = ops.hsvrnn_weight_struct(mod)
+        offset = ops.hsvrnn_bone_offsets(kp, parents, ops.f32(mod, "offset_param"))
+        kpt = kp.transpose(0, 1).reshape(T, B, 4 * K).contiguous()
+        hs = torch.empty(T + 1, B, H, dtype=torch.float32, device=dev)
+        hs[0] = mod.init_kypt_rnn_state.detach().float().expand(B, -1)
+        fs = torch.empty(T, B, 4 * K, dtype=torch.float32, device=dev)
+        zs = torch.empty(T, B, Z, dtype=torch.float32, device=dev)
+        Rs = torch.empty(T, B, K, 3, 3, dtype=torch.float32, device=dev)
+        post = torch.empty(T, B, 2 * Z, dtype=torch.float32, device=dev)
+        prior = torch.empty(T, B, 2 * Z, dtype=torch.float32, device=dev)
+        pick = torch.empty(T, B, dtype=torch.int32, device=dev)
+        for t in range(T):
+            ops.hsvrnn_step_record(w, hs[t], kpt[t], eps[t], offset, order, parents, K, hs[t + 1], fs[t], zs[t], Rs[t],
+                                   post[t], prior[t], pick[t])
+        ctx.save_for_backward(hs, kpt, fs, zs, Rs, eps, pick, offset)
+        ctx.mod = mod
+        return (fs.view(T, B, K, 4).transpose(0, 1).contiguous(), Rs.transpose(0, 1).contiguous(),
+                zs.transpose(0, 1).contiguous(), hs.transpose(0, 1).contiguous(), post, prior)
+
+    @staticmethod
+    def backward(ctx, dF, dR, dZ, dH, dpost, dprior):
+        hs, kpt, fs, zs, Rs, eps, pick, offset = ctx.saved_tensors
+        mod = ctx.mod
+        T, B = fs.shape[:2]
+        K = fs.shape[-1] // 4
+        order, parents = mod._tree(hs.device)
+        wt, w = ops.hsvrnn_weight_struct(mod), ops.hsvrnn_weight_struct(mod, transposed=False)
+        dF = dF.float().transpose(0, 1).reshape(T, B, 4 * K).contiguous()
+        dR = dR.float().transpose(0, 1).reshape(T, B, K * 9).contiguous()
+        dZ = dZ.float().transpose(0, 1).contiguous()
+        dH = dH.float().transpose(0, 1).contiguous()
+        dpost, dprior = _c(dpost.float()), _c(dprior.float())
+        rows = ops.hsvrnn_backward_workspace(B, T, hs.device)
+        doff = torch.zeros_like(offset)
+        carry, nxt = dH[T].clone(), torch.empty_like(dH[T])
+        for t in range(T - 1, -1, -1):
+            ops.hsvrnn_step_backward(wt, w, hs[t], kpt[t], eps[t], pick[t], fs[t], zs[t], Rs[t], offset, order, parents, K,
+                                     carry, dH[t], dF[t], dR[t], dZ[t], dpost[t], dprior[t], nxt, doff, rows[t])
+            carry, nxt = nxt, carry
+        params = ops.hsvrnn_params(mod)
+        want_op = ctx.needs_input_grad[3 + len(params) - 1]
+        grads = [torch.empty(p.shape, dtype=torch.float32, device=p.device) for p in params[:-1]]
+        grads.append(torch.empty(params[-1].shape, dtype=torch.float32, device=hs.device) if want_op else None)
+        ops.hsvrnn_weight_grads(rows, hs, kpt, fs, zs, carry, offset, doff,
+                                ops.f32(mod, "offset_param") if want_op else None, grads)
+        return (None, None, None) + tuple(g if need else None for g, need in zip(grads, ctx.needs_input_grad[3:]))
 
 
 # ------------------------------------------------------------------ module-level helpers used by the training path

@@ -110,6 +110,7 @@ struct StepArgs {
   float* R_out;           // (B, K, 9) or null
   float* post_out;        // (B, 256) posterior mean | std, or null
   float* prior_out;       // (B, 256) prior mean | std, or null
+  int* pick_out;          // (B) index of the sample fed to the GRU, or null
   int B, K, S, posterior;
 };
 
@@ -230,6 +231,7 @@ hsvrnn_step_kernel(const StepArgs a) {
       }
     }
     s_best[v] = best;
+    if (a.pick_out) a.pick_out[b0 + v] = best;
   }
   __syncthreads();
   for (int i = threadIdx.x; i < nb * (K4 + Z); i += kThreads) {
@@ -608,6 +610,7 @@ hsvrnn_step_cluster_kernel(const StepArgs a) {
       }
     }
     s_tree[2 * KP_MAX] = best;
+    if (rank == 0 && a.pick_out) a.pick_out[b] = best;
   }
   __syncthreads();
   const int best = s_tree[2 * KP_MAX];
@@ -713,10 +716,10 @@ __global__ void bone_offset_kernel(const float* __restrict__ kp /* (B,T,K,4) */,
 
 }  // namespace
 
-extern "C" int nm_hsvrnn_step(const nm_hsvrnn_weights* w, const float* h_in, const float* kp, const float* eps,
-                              const float* offset, const int* order, const int* parents, int B, int K, int S,
-                              int posterior, float* h_out, float* kp_out, float* z_out, float* R_out,
-                              float* post_out, float* prior_out, void* stream) {
+static int hsvrnn_step_impl(const nm_hsvrnn_weights* w, const float* h_in, const float* kp, const float* eps,
+                            const float* offset, const int* order, const int* parents, int B, int K, int S, int posterior,
+                            float* h_out, float* kp_out, float* z_out, float* R_out, float* post_out, float* prior_out,
+                            int* pick_out, void* stream) {
   NM_CHECK_ARG(w && h_in && eps && offset && order && parents && h_out && kp_out, "nm_hsvrnn_step: null pointer");
   NM_CHECK_ARG(!posterior || kp, "nm_hsvrnn_step: posterior step needs detected keypoints");
   NM_CHECK_ARG(K > 0 && K <= KP_MAX && S >= 1 && S <= 16, "nm_hsvrnn_step: K=%d S=%d unsupported", K, S);
@@ -725,6 +728,7 @@ extern "C" int nm_hsvrnn_step(const nm_hsvrnn_weights* w, const float* h_in, con
   StepArgs a;
   a.w = *w; a.h_in = h_in; a.kp = kp; a.eps = eps; a.offset = offset; a.order = order; a.parents = parents;
   a.h_out = h_out; a.kp_out = kp_out; a.z_out = z_out; a.R_out = R_out; a.post_out = post_out; a.prior_out = prior_out;
+  a.pick_out = pick_out;
   a.B = B; a.K = K; a.S = S; a.posterior = posterior;
   cudaStream_t st = (cudaStream_t)stream;
   // small and medium batches: a cluster of 8 CTAs per element (weights split over the ranks, DSMEM broadcasts)
@@ -755,6 +759,22 @@ extern "C" int nm_hsvrnn_step(const nm_hsvrnn_weights* w, const float* h_in, con
   return NM_OK;
 }
 
+extern "C" int nm_hsvrnn_step(const nm_hsvrnn_weights* w, const float* h_in, const float* kp, const float* eps,
+                              const float* offset, const int* order, const int* parents, int B, int K, int S,
+                              int posterior, float* h_out, float* kp_out, float* z_out, float* R_out,
+                              float* post_out, float* prior_out, void* stream) {
+  return hsvrnn_step_impl(w, h_in, kp, eps, offset, order, parents, B, K, S, posterior, h_out, kp_out, z_out, R_out,
+                          post_out, prior_out, nullptr, stream);
+}
+
+extern "C" int nm_hsvrnn_step_record(const nm_hsvrnn_weights* w, const float* h_in, const float* kp, const float* eps,
+                                     const float* offset, const int* order, const int* parents, int B, int K, int S,
+                                     int posterior, float* h_out, float* kp_out, float* z_out, float* R_out,
+                                     float* post_out, float* prior_out, int* pick_out, void* stream) {
+  return hsvrnn_step_impl(w, h_in, kp, eps, offset, order, parents, B, K, S, posterior, h_out, kp_out, z_out, R_out,
+                          post_out, prior_out, pick_out, stream);
+}
+
 extern "C" int nm_hsvrnn_decode_pose(const nm_hsvrnn_weights* w, const float* dec_in, const float* offset,
                                      const int* order, const int* parents, int B, int K, float* flat_out,
                                      float* R_out, void* stream) {
@@ -773,5 +793,506 @@ extern "C" int nm_hsvrnn_bone_offsets(const float* keypoints, const int* parents
   if (B == 0) return NM_OK;
   bone_offset_kernel<<<nm_cdiv(B * K, 128), 128, 0, (cudaStream_t)stream>>>(keypoints, parents, offset_param, B, T, K, out);
   NM_CHECK_LAUNCH("hsvrnn_bone_offsets");
+  return NM_OK;
+}
+
+// ================================================================== stage-2 training: backward of a conditioned step
+// The reverse loop launches nm_hsvrnn_step_backward once per step, t = T-1 .. 0.  Only the picked sample of each
+// element feeds anything downstream (the other S-1 decodes do not), so the backward decodes one pose per element.  It
+// saves nothing from the forward beyond the pick: the hidden layers, the decoder outputs and the GRU gates are recomputed
+// from h_t, kp_t and the picked (z, f) that encode() already returns.  The work is a chain of small batched mat-vecs over
+// all B elements at once; every one of them splits its output columns over CTAs (32 columns x 16 elements per CTA, the
+// reduction split 32 ways inside the CTA), so the 6.1 MB of weights stream through many SMs whatever B is.  Forward
+// recomputes read the cached [in][out] copies, the transposed products dx = W^T dy read the fp32 parameters in their own
+// [out][in] layout: both are coalesced along the output columns.  Every reduction runs in a fixed order.
+namespace {
+
+// Per-(t, b) row record (floats): forward recomputes, then every d pre-activation the weight gradients need.
+enum : int {
+  RW_AP = 0, RW_AQ = RW_AP + HID, RW_AR = RW_AQ + HID, RW_AJ = RW_AR + HID,       // first-layer pre-activations
+  RW_GI = RW_AJ + HID, RW_GH = RW_GI + 3 * H,                                      // W_ih x + b_ih, W_hh h + b_hh
+  RW_OP = RW_GH + 3 * H, RW_OQ = RW_OP + 2 * Z,                                    // prior / posterior raw outputs
+  RW_OR = RW_OQ + 2 * Z, RW_OJ = RW_OR + 32,                                       // tanh(root) (3+K), joint 6-D (6K)
+  RW_DGI = RW_OJ + 6 * KP_MAX, RW_DGH = RW_DGI + 3 * H,                            // d gates (input / hidden side)
+  RW_DXG = RW_DGH + 3 * H, RW_DH1 = RW_DXG + 4 * KP_MAX + Z,                       // W_ih^T dgi (then df | dz), W_hh^T dgh
+  RW_DOR = RW_DH1 + H, RW_DOJ = RW_DOR + 32,                                       // d pre-tanh root, d joint 6-D
+  RW_DAR = RW_DOJ + 6 * KP_MAX, RW_DAJ = RW_DAR + HID,                             // d first-layer pre-activations
+  RW_DXDR = RW_DAJ + HID, RW_DXDJ = RW_DXDR + H + Z,                               // W0^T da of the decoders ([h | z])
+  RW_DOP = RW_DXDJ + H + Z, RW_DOQ = RW_DOP + 2 * Z,                               // d prior / posterior raw outputs
+  RW_DAP = RW_DOQ + 2 * Z, RW_DAQ = RW_DAP + HID,
+  RW_DXP = RW_DAQ + HID, RW_DXQ = RW_DXP + H, RW_DHD = RW_DXQ + H,                 // h parts; GRU's direct dh' * z
+  RW = RW_DHD + H
+};
+
+constexpr int GR = 16;        // elements per CTA
+constexpr int GC = 32;        // output columns per CTA (8 quads)
+constexpr int GKS = 32;       // reduction slices per CTA (4 per warp)
+constexpr int kMaxGemmJobs = 6;
+
+// Y[b][c] = epi(sum_k X[b][k] M[k][c]),  X[b] = [x0[b][0:k0] | x1[b][0:K-k0]] (LeakyReLU applied on load when xlrelu),
+// M[k][c] = m[k * ldm + c]; epi: + bias[c], then tanh, then * LeakyReLU'(gate[b][c]) - each optional.
+struct GemmJob {
+  const float* x0; const float* x1; const float* m; const float* bias; const float* gate; float* y;
+  int ldx0, ldx1, k0, K, ldm, N, ldgate, ldy, xlrelu, tanh_out;
+};
+struct GemmJobs {
+  GemmJob j[kMaxGemmJobs];
+  int tile_end[kMaxGemmJobs];
+  int n, B;
+};
+
+__global__ void __launch_bounds__(kThreads)
+rows_gemm_kernel(const __grid_constant__ GemmJobs js) {
+  extern __shared__ float sm[];
+  int tile = blockIdx.x, ji = 0;
+  while (tile >= js.tile_end[ji]) ji++;
+  const GemmJob& J = js.j[ji];
+  const int c0 = (tile - (ji ? js.tile_end[ji - 1] : 0)) * GC;
+  const int b0 = blockIdx.y * GR, nb = min(GR, js.B - b0);
+  const int K = J.K;
+  float* sx = sm;                 // [GR][K]
+  float* sred = sm + GR * K;      // [8 warps][GR][GC]
+  for (int i = threadIdx.x; i < GR * K; i += kThreads) {
+    const int r = i / K, k = i % K;
+    float v = 0.f;
+    if (r < nb) {
+      v = k < J.k0 ? J.x0[(long long)(b0 + r) * J.ldx0 + k] : J.x1[(long long)(b0 + r) * J.ldx1 + (k - J.k0)];
+      if (J.xlrelu) v = nm_lrelu(v);
+    }
+    sx[i] = v;
+  }
+  __syncthreads();
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int q = lane & 7, s = lane >> 3, ks = warp * 4 + s;
+  const int col = c0 + q * 4;
+  const int per = (K + GKS - 1) / GKS;
+  const int klo = min(K, ks * per), khi = min(K, klo + per);
+  float acc[GR][4];
+#pragma unroll
+  for (int r = 0; r < GR; r++) acc[r][0] = acc[r][1] = acc[r][2] = acc[r][3] = 0.f;
+#pragma unroll 4
+  for (int k = klo; k < khi; k++) {      // four rows of weight loads in flight
+    const float* mr = J.m + (long long)k * J.ldm;
+    float w[4];
+#pragma unroll
+    for (int e = 0; e < 4; e++) w[e] = col + e < J.N ? __ldg(mr + col + e) : 0.f;
+    const float* xk = sx + k;
+#pragma unroll
+    for (int r = 0; r < GR; r++) {
+      const float xv = xk[r * K];
+#pragma unroll
+      for (int e = 0; e < 4; e++) acc[r][e] = fmaf(w[e], xv, acc[r][e]);
+    }
+  }
+#pragma unroll
+  for (int r = 0; r < GR; r++)
+#pragma unroll
+    for (int e = 0; e < 4; e++) {
+      float v = acc[r][e];
+      v += __shfl_xor_sync(0xffffffffu, v, 8);
+      v += __shfl_xor_sync(0xffffffffu, v, 16);
+      acc[r][e] = v;
+    }
+  if (s == 0)
+#pragma unroll
+    for (int r = 0; r < GR; r++)
+#pragma unroll
+      for (int e = 0; e < 4; e++) sred[(warp * GR + r) * GC + q * 4 + e] = acc[r][e];
+  __syncthreads();
+  for (int i = threadIdx.x; i < GR * GC; i += kThreads) {
+    const int r = i / GC, c = i % GC;
+    if (r >= nb || c0 + c >= J.N) continue;
+    float v = 0.f;
+#pragma unroll
+    for (int w = 0; w < 8; w++) v += sred[(w * GR + r) * GC + c];
+    if (J.bias) v += J.bias[c0 + c];
+    if (J.tanh_out) v = tanhf(v);
+    if (J.gate) v *= J.gate[(long long)(b0 + r) * J.ldgate + c0 + c] > 0.f ? 1.f : 0.01f;
+    J.y[(long long)(b0 + r) * J.ldy + c0 + c] = v;
+  }
+}
+
+__device__ __forceinline__ float ld_or0(const float* p, long long i) { return p ? p[i] : 0.f; }
+// d softplus(x) / dx with torch's threshold (softplus(x) = x above 20)
+__device__ __forceinline__ float dsoftplus_d(float x) { return x > 20.f ? 1.f : sigmoid_d(x); }
+
+// GRU cell backward (gate order r, z, n): dgi, dgh and the direct part dh' * z of dh.  One CTA per element.
+__global__ void __launch_bounds__(kThreads)
+gru_bwd_kernel(const float* __restrict__ h, const float* __restrict__ dh_next, float* __restrict__ rows) {
+  const int b = blockIdx.x;
+  float* rec = rows + (long long)b * RW;
+  for (int j = threadIdx.x; j < H; j += kThreads) {
+    const float* gi = rec + RW_GI;
+    const float* gh = rec + RW_GH;
+    const float r = sigmoid_d(gi[j] + gh[j]);
+    const float zg = sigmoid_d(gi[H + j] + gh[H + j]);
+    const float ghn = gh[2 * H + j];
+    const float n = tanhf(gi[2 * H + j] + r * ghn);
+    const float d = dh_next[(long long)b * H + j];
+    const float dan = d * (1.f - zg) * (1.f - n * n);
+    const float dar = dan * ghn * r * (1.f - r);
+    const float daz = d * (h[(long long)b * H + j] - n) * zg * (1.f - zg);
+    rec[RW_DGI + j] = dar; rec[RW_DGI + H + j] = daz; rec[RW_DGI + 2 * H + j] = dan;
+    rec[RW_DGH + j] = dar; rec[RW_DGH + H + j] = daz; rec[RW_DGH + 2 * H + j] = dan * r;
+    rec[RW_DHD + j] = d * zg;
+  }
+}
+
+// 6-D -> rotation backward: dR (row-major 3x3, columns x, y, z) -> dp (6)
+__device__ void rot6d_bwd(const float* p, const float* dR, float* dp) {
+  const float a0 = p[0], a1 = p[1], a2 = p[2], b0 = p[3], b1 = p[4], b2 = p[5];
+  const float la = sqrtf(a0 * a0 + a1 * a1 + a2 * a2), na = la + 1e-10f;
+  const float x0 = a0 / na, x1 = a1 / na, x2 = a2 / na;
+  const float c0 = x1 * b2 - x2 * b1, c1 = x2 * b0 - x0 * b2, c2 = x0 * b1 - x1 * b0;
+  const float lc = sqrtf(c0 * c0 + c1 * c1 + c2 * c2), nc = lc + 1e-10f;
+  const float z0 = c0 / nc, z1 = c1 / nc, z2 = c2 / nc;
+  float dx0 = dR[0], dx1 = dR[3], dx2 = dR[6];
+  const float dy0 = dR[1], dy1 = dR[4], dy2 = dR[7];
+  float dz0 = dR[2], dz1 = dR[5], dz2 = dR[8];
+  // y = z x x
+  dz0 += x1 * dy2 - x2 * dy1; dz1 += x2 * dy0 - x0 * dy2; dz2 += x0 * dy1 - x1 * dy0;
+  dx0 += dy1 * z2 - dy2 * z1; dx1 += dy2 * z0 - dy0 * z2; dx2 += dy0 * z1 - dy1 * z0;
+  // z = c / (|c| + 1e-10)
+  const float cdz = (c0 * dz0 + c1 * dz1 + c2 * dz2) / (lc > 0.f ? lc * nc * nc : 1.f);
+  const float dc0 = dz0 / nc - c0 * cdz, dc1 = dz1 / nc - c1 * cdz, dc2 = dz2 / nc - c2 * cdz;
+  // c = x x b
+  dx0 += b1 * dc2 - b2 * dc1; dx1 += b2 * dc0 - b0 * dc2; dx2 += b0 * dc1 - b1 * dc0;
+  dp[3] = dc1 * x2 - dc2 * x1; dp[4] = dc2 * x0 - dc0 * x2; dp[5] = dc0 * x1 - dc1 * x0;
+  // x = a / (|a| + 1e-10)
+  const float adx = (a0 * dx0 + a1 * dx1 + a2 * dx2) / (la > 0.f ? la * na * na : 1.f);
+  dp[0] = dx0 / na - a0 * adx; dp[1] = dx1 / na - a1 * adx; dp[2] = dx2 / na - a2 * adx;
+}
+
+// Pose backward of the picked decode: forward kinematics down `order` in reverse, then the 6-D rotations and the tanh.
+// df = W_ih^T dgi [:4K] + external d kypt_recon; dR external d R; accumulates d offset.  One CTA of 64 threads per element.
+__global__ void __launch_bounds__(64)
+pose_bwd_kernel(const float* __restrict__ Rg_all /* (B, K, 9) */, const float* __restrict__ offset, const int* __restrict__ order,
+                const int* __restrict__ parents, const float* __restrict__ df_ext, const float* __restrict__ dR_ext,
+                const float* __restrict__ dz_ext, int K, float* __restrict__ doffset, float* __restrict__ rows) {
+  __shared__ float s_rl[KP_MAX * 9], s_drg[KP_MAX * 9], s_dpos[KP_MAX * 3], s_doff[KP_MAX * 3], s_dint[KP_MAX];
+  const int b = blockIdx.x, K4 = 4 * K;
+  float* rec = rows + (long long)b * RW;
+  const float* Rg = Rg_all + (long long)b * K * 9;
+  for (int k = threadIdx.x; k < K; k += 64) rot6d(rec + RW_OJ + k * 6, s_rl + k * 9);
+  for (int i = threadIdx.x; i < K * 9; i += 64) s_drg[i] = ld_or0(dR_ext, (long long)b * K * 9 + i);
+  for (int i = threadIdx.x; i < K4; i += 64) {
+    const float d = rec[RW_DXG + i] + ld_or0(df_ext, (long long)b * K4 + i);
+    if ((i & 3) == 3) s_dint[i >> 2] = d;
+    else s_dpos[(i >> 2) * 3 + (i & 3)] = d;
+  }
+  for (int i = threadIdx.x; i < K * 3; i += 64) s_doff[i] = 0.f;
+  for (int i = threadIdx.x; i < Z; i += 64) rec[RW_DXG + K4 + i] += ld_or0(dz_ext, (long long)b * Z + i);   // dz
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    for (int j = K - 1; j >= 1; j--) {
+      const int i = order[j], pa = parents[i];
+      const float* Ri = Rg + i * 9;
+      const float* Rp = Rg + pa * 9;
+      const float* Rl = s_rl + i * 9;
+      const float* o = offset + ((long long)b * K + i) * 3;
+      float* dRi = s_drg + i * 9;
+      float* dRp = s_drg + pa * 9;
+      const float dp0 = s_dpos[i * 3], dp1 = s_dpos[i * 3 + 1], dp2 = s_dpos[i * 3 + 2];
+      s_dpos[pa * 3] += dp0; s_dpos[pa * 3 + 1] += dp1; s_dpos[pa * 3 + 2] += dp2;
+#pragma unroll
+      for (int c = 0; c < 3; c++) {
+        s_doff[i * 3 + c] = Ri[c] * dp0 + Ri[3 + c] * dp1 + Ri[6 + c] * dp2;
+        dRi[c] += dp0 * o[c]; dRi[3 + c] += dp1 * o[c]; dRi[6 + c] += dp2 * o[c];
+      }
+      float dl[9];
+#pragma unroll
+      for (int r = 0; r < 3; r++)
+#pragma unroll
+        for (int c = 0; c < 3; c++) {
+          dRp[r * 3 + c] += dRi[r * 3] * Rl[c * 3] + dRi[r * 3 + 1] * Rl[c * 3 + 1] + dRi[r * 3 + 2] * Rl[c * 3 + 2];
+          dl[r * 3 + c] = Rp[r] * dRi[c] + Rp[3 + r] * dRi[3 + c] + Rp[6 + r] * dRi[6 + c];
+        }
+#pragma unroll
+      for (int e = 0; e < 9; e++) dRi[e] = dl[e];      // d Rl_i from here on
+    }
+  }
+  __syncthreads();
+  // the root's global rotation is its local one: s_drg[root] already holds d Rl_root
+  for (int k = threadIdx.x; k < K; k += 64) {
+    float dp[6];
+    rot6d_bwd(rec + RW_OJ + k * 6, s_drg + k * 9, dp);
+#pragma unroll
+    for (int e = 0; e < 6; e++) rec[RW_DOJ + k * 6 + e] = dp[e];
+  }
+  const int root = order[0];
+  for (int c = threadIdx.x; c < 3 + K; c += 64) {
+    const float y = rec[RW_OR + c];
+    const float d = c < 3 ? s_dpos[root * 3 + c] : 0.5f * s_dint[c - 3];
+    rec[RW_DOR + c] = d * (1.f - y * y);
+  }
+  for (int i = threadIdx.x; i < K * 3; i += 64) doffset[(long long)b * K * 3 + i] += s_doff[i];
+}
+
+// z = qm + qs * eps_pick: d of the posterior / prior raw outputs (std = softplus(raw) + 1e-4).  One CTA per element.
+__global__ void __launch_bounds__(Z)
+dist_bwd_kernel(const float* __restrict__ eps, const int* __restrict__ pick, const float* __restrict__ dpost,
+                const float* __restrict__ dprior, int B, int K, float* __restrict__ rows) {
+  const int b = blockIdx.x, i = threadIdx.x;
+  float* rec = rows + (long long)b * RW;
+  const float dz = rec[RW_DXG + 4 * K + i] + rec[RW_DXDR + H + i] + rec[RW_DXDJ + H + i];
+  const float e = eps[((long long)pick[b] * B + b) * Z + i];
+  rec[RW_DOQ + i] = dz + ld_or0(dpost, (long long)b * 2 * Z + i);
+  rec[RW_DOQ + Z + i] = (dz * e + ld_or0(dpost, (long long)b * 2 * Z + Z + i)) * dsoftplus_d(rec[RW_OQ + Z + i]);
+  rec[RW_DOP + i] = ld_or0(dprior, (long long)b * 2 * Z + i);
+  rec[RW_DOP + Z + i] = ld_or0(dprior, (long long)b * 2 * Z + Z + i) * dsoftplus_d(rec[RW_OP + Z + i]);
+}
+
+// dh_t = GRU direct part + W_hh^T dgh + decoders' h parts + posterior / prior h parts + external d h_kypts[:, t]
+__global__ void __launch_bounds__(kThreads)
+dh_sum_kernel(const float* __restrict__ rows, const float* __restrict__ dh_ext, float* __restrict__ dh_out) {
+  const int b = blockIdx.x;
+  const float* rec = rows + (long long)b * RW;
+  for (int j = threadIdx.x; j < H; j += kThreads) {
+    float v = rec[RW_DHD + j] + rec[RW_DH1 + j];
+    v += rec[RW_DXDR + j] + rec[RW_DXDJ + j];
+    v += rec[RW_DXQ + j] + rec[RW_DXP + j];
+    dh_out[(long long)b * H + j] = v + ld_or0(dh_ext, (long long)b * H + j);
+  }
+}
+
+GemmJob gemm_job(const float* x0, int ldx0, int k0, const float* x1, int ldx1, int K, const float* m, int ldm, int N,
+                 float* y, int ldy) {
+  GemmJob j;
+  j.x0 = x0; j.ldx0 = ldx0; j.k0 = k0; j.x1 = x1; j.ldx1 = ldx1; j.K = K;
+  j.m = m; j.ldm = ldm; j.N = N; j.bias = nullptr; j.gate = nullptr; j.ldgate = 0; j.y = y; j.ldy = ldy;
+  j.xlrelu = 0; j.tanh_out = 0;
+  return j;
+}
+
+int launch_gemm(GemmJobs& js, int n, int B, cudaStream_t st) {
+  js.n = n; js.B = B;
+  int tiles = 0, kmax = 0;
+  for (int i = 0; i < n; i++) {
+    tiles += nm_cdiv(js.j[i].N, GC);
+    js.tile_end[i] = tiles;
+    kmax = max(kmax, js.j[i].K);
+  }
+  const size_t smem = ((size_t)GR * kmax + 8 * GR * GC) * sizeof(float);
+  NM_CHECK_CUDA(cudaFuncSetAttribute(rows_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  rows_gemm_kernel<<<dim3(tiles, nm_cdiv(B, GR)), kThreads, smem, st>>>(js);
+  NM_CHECK_LAUNCH("hsvrnn_step_backward(gemm)");
+  return NM_OK;
+}
+
+// ------------------------------------------------------------------ weight gradients over the T*B rows, fixed order
+// dW[o][i] = sum_r dY[r][o] X[r][i] (X == null: a column of ones -> bias / init-state sums); 64 x 64 tiles, each thread a
+// 4 x 4 block, rows streamed through shared memory 16 at a time in ascending order.  No atomics: bit-reproducible.
+constexpr int kMaxWgJobs = 24;
+struct WgJob {
+  const float* dy; const float* x0; const float* x1; float* dw;
+  int lddy, O, ldx0, ldx1, k0, I, xlrelu, R, ldw;
+};
+struct WgJobs {
+  WgJob j[kMaxWgJobs];
+  int tile_end[kMaxWgJobs];
+  int n;
+  const float* offset; const float* doffset; const float* offset_param; float* d_offset_param;
+  int B, K;
+};
+
+__global__ void __launch_bounds__(kThreads)
+hsvrnn_wgrad_kernel(const __grid_constant__ WgJobs js) {
+  __shared__ float s_dy[16][64], s_x[16][64];
+  const int tid = threadIdx.x;
+  const int tile = blockIdx.x;
+  if (tile >= js.tile_end[js.n - 1]) {
+    // offset_param: offset[b, k] = op_k / (|op_k| + 1e-10) * scale[b, k]  (scale = the bone-length median)
+    const int k = tid;
+    if (k >= js.K) return;
+    const float* op = js.offset_param + k * 3;
+    const float lo = sqrtf(op[0] * op[0] + op[1] * op[1] + op[2] * op[2]), n = lo + 1e-10f;
+    const float u0 = op[0] / n, u1 = op[1] / n, u2 = op[2] / n, uu = u0 * u0 + u1 * u1 + u2 * u2;
+    float du0 = 0.f, du1 = 0.f, du2 = 0.f;
+    for (int b = 0; b < js.B; b++) {
+      const float* o = js.offset + ((long long)b * js.K + k) * 3;
+      const float* d = js.doffset + ((long long)b * js.K + k) * 3;
+      const float scale = uu > 0.f ? (o[0] * u0 + o[1] * u1 + o[2] * u2) / uu : 0.f;
+      du0 = fmaf(scale, d[0], du0); du1 = fmaf(scale, d[1], du1); du2 = fmaf(scale, d[2], du2);
+    }
+    const float od = (op[0] * du0 + op[1] * du1 + op[2] * du2) / (lo > 0.f ? lo * n * n : 1.f);
+    js.d_offset_param[k * 3] = du0 / n - op[0] * od;
+    js.d_offset_param[k * 3 + 1] = du1 / n - op[1] * od;
+    js.d_offset_param[k * 3 + 2] = du2 / n - op[2] * od;
+    return;
+  }
+  int ji = 0;
+  while (tile >= js.tile_end[ji]) ji++;
+  const WgJob& J = js.j[ji];
+  const int local = tile - (ji ? js.tile_end[ji - 1] : 0);
+  const int ti = (J.I + 63) / 64;
+  const int o0 = (local / ti) * 64, i0 = (local % ti) * 64;
+  const int tx = tid & 15, ty = tid >> 4;
+  float acc[4][4];
+#pragma unroll
+  for (int e = 0; e < 4; e++) acc[e][0] = acc[e][1] = acc[e][2] = acc[e][3] = 0.f;
+  for (int r0 = 0; r0 < J.R; r0 += 16) {
+    for (int i = tid; i < 16 * 64; i += kThreads) {
+      const int rr = i >> 6, c = i & 63, r = r0 + rr;
+      float dy = 0.f, x = 0.f;
+      if (r < J.R) {
+        if (o0 + c < J.O) dy = J.dy[(long long)r * J.lddy + o0 + c];
+        const int ii = i0 + c;
+        if (ii < J.I) {
+          if (!J.x0) x = 1.f;
+          else {
+            x = ii < J.k0 ? J.x0[(long long)r * J.ldx0 + ii] : J.x1[(long long)r * J.ldx1 + (ii - J.k0)];
+            if (J.xlrelu) x = nm_lrelu(x);
+          }
+        }
+      }
+      s_dy[rr][c] = dy;
+      s_x[rr][c] = x;
+    }
+    __syncthreads();
+#pragma unroll 4
+    for (int rr = 0; rr < 16; rr++) {
+      float a[4], v[4];
+#pragma unroll
+      for (int e = 0; e < 4; e++) { a[e] = s_dy[rr][ty * 4 + e]; v[e] = s_x[rr][tx * 4 + e]; }
+#pragma unroll
+      for (int e = 0; e < 4; e++)
+#pragma unroll
+        for (int f = 0; f < 4; f++) acc[e][f] = fmaf(a[e], v[f], acc[e][f]);
+    }
+    __syncthreads();
+  }
+#pragma unroll
+  for (int e = 0; e < 4; e++) {
+    const int o = o0 + ty * 4 + e;
+    if (o >= J.O) continue;
+#pragma unroll
+    for (int f = 0; f < 4; f++) {
+      const int i = i0 + tx * 4 + f;
+      if (i < J.I) J.dw[(long long)o * J.ldw + i] = acc[e][f];
+    }
+  }
+}
+
+}  // namespace
+
+extern "C" size_t nm_hsvrnn_backward_workspace_bytes(int B, int T) { return (size_t)B * T * RW * sizeof(float); }
+
+extern "C" int nm_hsvrnn_step_backward(const nm_hsvrnn_weights* wt, const nm_hsvrnn_weights* w, const float* h,
+                                       const float* kp, const float* eps, const int* pick, const float* f, const float* z,
+                                       const float* R, const float* offset, const int* order, const int* parents, int B,
+                                       int K, int S, const float* dh_next, const float* dh_ext, const float* df,
+                                       const float* dR, const float* dz, const float* dpost, const float* dprior,
+                                       float* dh_out, float* doffset, float* rows, void* stream) {
+  NM_CHECK_ARG(wt && w && h && kp && eps && pick && f && z && R && offset && order && parents && dh_next && dh_out &&
+                   doffset && rows, "nm_hsvrnn_step_backward: null pointer");
+  NM_CHECK_ARG(K > 0 && K <= KP_MAX && S >= 1 && S <= 16, "nm_hsvrnn_step_backward: K=%d S=%d unsupported", K, S);
+  if (B == 0) return NM_OK;
+  (void)S;
+  cudaStream_t st = (cudaStream_t)stream;
+  const int K4 = 4 * K, R2 = 3 + K, J2 = 6 * K;
+  GemmJobs js;
+  // 1. forward recompute, first layers and both GRU halves (everything that reads h, kp, f, z)
+  js.j[0] = gemm_job(h, H, H, nullptr, 0, H, wt->prior0_wt, HID, HID, rows + RW_AP, RW);
+  js.j[0].bias = wt->prior0_b;
+  js.j[1] = gemm_job(h, H, H, kp, K4, H + K4, wt->post0_wt, HID, HID, rows + RW_AQ, RW);
+  js.j[1].bias = wt->post0_b;
+  js.j[2] = gemm_job(h, H, H, z, Z, H + Z, wt->root0_wt, HID, HID, rows + RW_AR, RW);
+  js.j[2].bias = wt->root0_b;
+  js.j[3] = gemm_job(h, H, H, z, Z, H + Z, wt->joint0_wt, HID, HID, rows + RW_AJ, RW);
+  js.j[3].bias = wt->joint0_b;
+  js.j[4] = gemm_job(h, H, H, nullptr, 0, H, wt->gru_hh_wt, 3 * H, 3 * H, rows + RW_GH, RW);
+  js.j[4].bias = wt->gru_hh_b;
+  js.j[5] = gemm_job(f, K4, K4, z, Z, K4 + Z, wt->gru_ih_wt, 3 * H, 3 * H, rows + RW_GI, RW);
+  js.j[5].bias = wt->gru_ih_b;
+  if (int rc = launch_gemm(js, 6, B, st)) return rc;
+  // 2. forward recompute, second layers (raw outputs; tanh for the root / intensity decoder)
+  js.j[0] = gemm_job(rows + RW_AP, RW, HID, nullptr, 0, HID, wt->prior2_wt, 2 * Z, 2 * Z, rows + RW_OP, RW);
+  js.j[1] = gemm_job(rows + RW_AQ, RW, HID, nullptr, 0, HID, wt->post2_wt, 2 * Z, 2 * Z, rows + RW_OQ, RW);
+  js.j[2] = gemm_job(rows + RW_AR, RW, HID, nullptr, 0, HID, wt->root2_wt, R2, R2, rows + RW_OR, RW);
+  js.j[3] = gemm_job(rows + RW_AJ, RW, HID, nullptr, 0, HID, wt->joint2_wt, J2, J2, rows + RW_OJ, RW);
+  js.j[0].bias = wt->prior2_b; js.j[1].bias = wt->post2_b; js.j[2].bias = wt->root2_b; js.j[3].bias = wt->joint2_b;
+  for (int i = 0; i < 4; i++) js.j[i].xlrelu = 1;
+  js.j[2].tanh_out = 1;
+  if (int rc = launch_gemm(js, 4, B, st)) return rc;
+  // 3. GRU backward
+  gru_bwd_kernel<<<B, kThreads, 0, st>>>(h, dh_next, rows);
+  NM_CHECK_LAUNCH("hsvrnn_step_backward(gru)");
+  js.j[0] = gemm_job(rows + RW_DGI, RW, 3 * H, nullptr, 0, 3 * H, w->gru_ih_wt, K4 + Z, K4 + Z, rows + RW_DXG, RW);
+  js.j[1] = gemm_job(rows + RW_DGH, RW, 3 * H, nullptr, 0, 3 * H, w->gru_hh_wt, H, H, rows + RW_DH1, RW);
+  if (int rc = launch_gemm(js, 2, B, st)) return rc;
+  // 4. forward kinematics, 6-D rotations, tanh
+  pose_bwd_kernel<<<B, 64, 0, st>>>(R, offset, order, parents, df, dR, dz, K, doffset, rows);
+  NM_CHECK_LAUNCH("hsvrnn_step_backward(pose)");
+  // 5. decoders: second layers (times LeakyReLU' of the first), then the first layers' [h | z] parts
+  js.j[0] = gemm_job(rows + RW_DOR, RW, R2, nullptr, 0, R2, w->root2_wt, HID, HID, rows + RW_DAR, RW);
+  js.j[1] = gemm_job(rows + RW_DOJ, RW, J2, nullptr, 0, J2, w->joint2_wt, HID, HID, rows + RW_DAJ, RW);
+  js.j[0].gate = rows + RW_AR; js.j[1].gate = rows + RW_AJ;
+  js.j[0].ldgate = js.j[1].ldgate = RW;
+  if (int rc = launch_gemm(js, 2, B, st)) return rc;
+  js.j[0] = gemm_job(rows + RW_DAR, RW, HID, nullptr, 0, HID, w->root0_wt, H + Z, H + Z, rows + RW_DXDR, RW);
+  js.j[1] = gemm_job(rows + RW_DAJ, RW, HID, nullptr, 0, HID, w->joint0_wt, H + Z, H + Z, rows + RW_DXDJ, RW);
+  if (int rc = launch_gemm(js, 2, B, st)) return rc;
+  // 6. posterior / prior distributions, then their MLPs (the posterior's kp columns are not needed)
+  dist_bwd_kernel<<<B, Z, 0, st>>>(eps, pick, dpost, dprior, B, K, rows);
+  NM_CHECK_LAUNCH("hsvrnn_step_backward(dist)");
+  js.j[0] = gemm_job(rows + RW_DOQ, RW, 2 * Z, nullptr, 0, 2 * Z, w->post2_wt, HID, HID, rows + RW_DAQ, RW);
+  js.j[1] = gemm_job(rows + RW_DOP, RW, 2 * Z, nullptr, 0, 2 * Z, w->prior2_wt, HID, HID, rows + RW_DAP, RW);
+  js.j[0].gate = rows + RW_AQ; js.j[1].gate = rows + RW_AP;
+  js.j[0].ldgate = js.j[1].ldgate = RW;
+  if (int rc = launch_gemm(js, 2, B, st)) return rc;
+  js.j[0] = gemm_job(rows + RW_DAQ, RW, HID, nullptr, 0, HID, w->post0_wt, H + K4, H, rows + RW_DXQ, RW);
+  js.j[1] = gemm_job(rows + RW_DAP, RW, HID, nullptr, 0, HID, w->prior0_wt, H, H, rows + RW_DXP, RW);
+  if (int rc = launch_gemm(js, 2, B, st)) return rc;
+  // 7. dh_t
+  dh_sum_kernel<<<B, kThreads, 0, st>>>(rows, dh_ext, dh_out);
+  NM_CHECK_LAUNCH("hsvrnn_step_backward(dh)");
+  return NM_OK;
+}
+
+extern "C" int nm_hsvrnn_weight_grads(const float* rows, const float* h, const float* kp, const float* f, const float* z,
+                                      const float* dh0, const float* offset, const float* doffset,
+                                      const float* offset_param, int B, int T, int K, const nm_hsvrnn_grads* g,
+                                      void* stream) {
+  NM_CHECK_ARG(rows && h && kp && f && z && dh0 && g, "nm_hsvrnn_weight_grads: null pointer");
+  NM_CHECK_ARG(K > 0 && K <= KP_MAX && T >= 1, "nm_hsvrnn_weight_grads: K=%d T=%d unsupported", K, T);
+  NM_CHECK_ARG(!g->offset_param || (offset && doffset && offset_param), "nm_hsvrnn_weight_grads: offset_param needs offsets");
+  if (B == 0) return NM_OK;
+  const int K4 = 4 * K, R = T * B;
+  WgJobs js;
+  int n = 0;
+  auto add = [&](const float* dy, int O, const float* x0, int ldx0, int k0, const float* x1, int ldx1, int I, int xl,
+                 float* dw, float* db) {
+    WgJob j;
+    j.dy = dy; j.lddy = RW; j.O = O; j.x0 = x0; j.ldx0 = ldx0; j.k0 = k0; j.x1 = x1; j.ldx1 = ldx1; j.I = I;
+    j.xlrelu = xl; j.R = R; j.dw = dw; j.ldw = I;
+    js.j[n++] = j;
+    j.x0 = j.x1 = nullptr; j.I = 1; j.ldw = 1; j.dw = db;
+    js.j[n++] = j;
+  };
+  add(rows + RW_DAQ, HID, h, H, H, kp, K4, H + K4, 0, g->post0_w, g->post0_b);
+  add(rows + RW_DOQ, 2 * Z, rows + RW_AQ, RW, HID, nullptr, 0, HID, 1, g->post2_w, g->post2_b);
+  add(rows + RW_DAP, HID, h, H, H, nullptr, 0, H, 0, g->prior0_w, g->prior0_b);
+  add(rows + RW_DOP, 2 * Z, rows + RW_AP, RW, HID, nullptr, 0, HID, 1, g->prior2_w, g->prior2_b);
+  add(rows + RW_DAR, HID, h, H, H, z, Z, H + Z, 0, g->root0_w, g->root0_b);
+  add(rows + RW_DOR, 3 + K, rows + RW_AR, RW, HID, nullptr, 0, HID, 1, g->root2_w, g->root2_b);
+  add(rows + RW_DAJ, HID, h, H, H, z, Z, H + Z, 0, g->joint0_w, g->joint0_b);
+  add(rows + RW_DOJ, 6 * K, rows + RW_AJ, RW, HID, nullptr, 0, HID, 1, g->joint2_w, g->joint2_b);
+  add(rows + RW_DGI, 3 * H, f, K4, K4, z, Z, K4 + Z, 0, g->gru_ih_w, g->gru_ih_b);
+  add(rows + RW_DGH, 3 * H, h, H, H, nullptr, 0, H, 0, g->gru_hh_w, g->gru_hh_b);
+  {  // d init_kypt_rnn_state = sum over b of dh_0
+    WgJob j;
+    j.dy = dh0; j.lddy = H; j.O = H; j.x0 = j.x1 = nullptr; j.ldx0 = j.ldx1 = j.k0 = 0; j.I = 1; j.xlrelu = 0; j.R = B;
+    j.dw = g->init_state; j.ldw = 1;
+    js.j[n++] = j;
+  }
+  int tiles = 0;
+  for (int i = 0; i < n; i++) {
+    tiles += nm_cdiv(js.j[i].O, 64) * nm_cdiv(js.j[i].I, 64);
+    js.tile_end[i] = tiles;
+  }
+  js.n = n; js.B = B; js.K = K;
+  js.offset = offset; js.doffset = doffset; js.offset_param = offset_param; js.d_offset_param = g->offset_param;
+  hsvrnn_wgrad_kernel<<<tiles + (g->offset_param ? 1 : 0), kThreads, 0, (cudaStream_t)stream>>>(js);
+  NM_CHECK_LAUNCH("hsvrnn_weight_grads");
   return NM_OK;
 }

@@ -3,7 +3,9 @@
 Same class / parameter / attribute names (`extract_post_dist`, `extract_prior_dist`,
 `root_intensity_decoder`, `joint_matrix_decoder`, `kypt_rnn_cell`, `init_kypt_rnn_state`, `offset_param`,
 `A`, `priority`, `parents`) because the reference's demo scripts reach inside the module.  `encode` /
-`generate` run ONE fused CUDA kernel per time step (`nm_hsvrnn_step`) instead of ~4.7k ATen launches.
+`generate` run ONE fused CUDA kernel per time step (`nm_hsvrnn_step`) instead of ~4.7k ATen launches.  In training mode
+with autograd on, `encode` is differentiable (stage 2 of the reference's train.py): `autograd.HSVRNNEncode` runs the same
+steps and backpropagates through time on the `nm_hsvrnn_step_backward` / `nm_hsvrnn_weight_grads` kernels.
 
 Random draws: the reference calls `Normal.rsample`, i.e. standard-normal noise of shape (S, B, Z) per
 conditioned step and (B, Z) per generated step, in time order.  The same draws are made here with
@@ -16,6 +18,7 @@ import torch
 from torch import nn
 
 from .. import ops
+from ..autograd import HSVRNNEncode
 from ..utils.dyna_utils import process_affinity_glob
 
 
@@ -94,8 +97,10 @@ class HSVRNNBVH(nn.Module):
 
     # ------------------------------------------------------------------ rollouts
     def encode(self, keypoints, affinity, SAMPLE_NUM=10, eps=None):
-        """Track a keypoint sequence (reference :67-156).  keypoints (B, T, K, 4); eps optional (T, S, B, Z)."""
-        self._guard()
+        """Track a keypoint sequence (reference :67-156).  keypoints (B, T, K, 4); eps optional (T, S, B, Z).
+        Differentiable in training mode with grad enabled (the parameters only: keypoints must not require grad)."""
+        if self.training and torch.is_grad_enabled():
+            return self._encode_train(keypoints, affinity, SAMPLE_NUM, eps)
         B, T, K, _ = keypoints.shape
         dev = keypoints.device
         self._ensure_skeleton(affinity)
@@ -122,6 +127,29 @@ class HSVRNNBVH(nn.Module):
                 h_kypts=torch.stack(hs, dim=1), kl_kypt=torch.stack(kls, dim=1).mean(),
                 kypt_recon_loss=(inferred - kp).pow(2).sum(dim=(2, 3)).mean(),
                 gae_recon_loss=torch.tensor(0).to(dev), topo_recon_loss=torch.tensor(0).to(dev))
+
+    def _encode_train(self, keypoints, affinity, SAMPLE_NUM, eps):
+        if keypoints.requires_grad:
+            raise NotImplementedError("neural_marionette_b200: HSVRNNBVH.encode has no gradient for the keypoints; pass "
+                                      "keypoints.detach() (as NeuralMarionette.forward and the reference do)")
+        B, T, K, _ = keypoints.shape
+        dev = keypoints.device
+        self._ensure_skeleton(affinity)
+        Z = self.nlatent_kypt
+        kp = keypoints.float().contiguous()
+        if eps is None:     # the same draws, in the same order, as the step loop of the eval path
+            eps = torch.stack([torch.randn(SAMPLE_NUM, B, Z, device=dev) for _ in range(T)])
+        f, R, z, h, post, prior = HSVRNNEncode.apply(kp, eps.float().contiguous(), self, *ops.hsvrnn_params(self))
+        kls = []
+        for t in range(T):       # the eval path's expressions on the same (B, 2Z) slices: bit-identical values
+            qm, qs, pm, ps = post[t][:, :Z], post[t][:, Z:], prior[t][:, :Z], prior[t][:, Z:]
+            ratio = (qs / ps).pow(2)
+            kls.append(0.5 * (ratio + ((qm - pm) / ps).pow(2) - 1 - ratio.log()))
+        return dict(
+            kypt_recon=f[..., :4], R=R, z_kypts=z, h_kypts=h, kl_kypt=torch.stack(kls, dim=1).mean(),
+            kypt_recon_loss=(f - kp).pow(2).sum(dim=(2, 3)).mean(),      # zeros made on the device: no host copy
+            gae_recon_loss=torch.zeros((), dtype=torch.int64, device=dev),
+            topo_recon_loss=torch.zeros((), dtype=torch.int64, device=dev))
 
     def generate(self, keypoints_cond, affinity=None, Ttot=10, Tcond=3, SAMPLE_NUM=10, eps_cond=None, eps_gen=None):
         """Condition on Tcond detected frames, then roll the prior out to Ttot (reference :158-234).

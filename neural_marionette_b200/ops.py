@@ -790,27 +790,39 @@ def decoder_adjust(ff_act, conv: torch.nn.Conv3d, frames_per_clip: int, g: int, 
 
 
 # ------------------------------------------------------------------ dynamics
-def hsvrnn_weight_struct(mod) -> "L.HsvrnnWeights":
-    """Transposed fp32 copies ([in][out]) of the HSVRNN matrices + the ctypes struct pointing at them."""
-    names = [("post0", mod.extract_post_dist[0]), ("post2", mod.extract_post_dist[2]),
-             ("prior0", mod.extract_prior_dist[0]), ("prior2", mod.extract_prior_dist[2]),
-             ("root0", mod.root_intensity_decoder[0]), ("root2", mod.root_intensity_decoder[2]),
-             ("joint0", mod.joint_matrix_decoder[0]), ("joint2", mod.joint_matrix_decoder[2])]
+def _hsvrnn_layers(mod):
+    return [("post0", mod.extract_post_dist[0]), ("post2", mod.extract_post_dist[2]),
+            ("prior0", mod.extract_prior_dist[0]), ("prior2", mod.extract_prior_dist[2]),
+            ("root0", mod.root_intensity_decoder[0]), ("root2", mod.root_intensity_decoder[2]),
+            ("joint0", mod.joint_matrix_decoder[0]), ("joint2", mod.joint_matrix_decoder[2])]
+
+
+def hsvrnn_params(mod):
+    """The parameters `nm_hsvrnn_weight_grads` differentiates, in the order of `L.HsvrnnGrads`."""
     cell = mod.kypt_rnn_cell
-    params = [p for _, lin in names for p in (lin.weight, lin.bias)] + \
-             [cell.weight_ih, cell.weight_hh, cell.bias_ih, cell.bias_hh]
+    return [p for _, lin in _hsvrnn_layers(mod) for p in (lin.weight, lin.bias)] + \
+           [cell.weight_ih, cell.weight_hh, cell.bias_ih, cell.bias_hh, mod.init_kypt_rnn_state, mod.offset_param]
+
+
+def hsvrnn_weight_struct(mod, transposed: bool = True) -> "L.HsvrnnWeights":
+    """The ctypes struct of the HSVRNN matrices: transposed fp32 copies ([in][out], what the step kernels read) or, with
+    transposed=False, the fp32 parameters in their own [out][in] layout (what the backward's W^T dy products read)."""
+    names = _hsvrnn_layers(mod)
+    cell = mod.kypt_rnn_cell
+    params = hsvrnn_params(mod)[:20]
 
     def build():
         keep = []
         st = L.HsvrnnWeights()
+        f = (lambda p: p.detach().float().t().contiguous()) if transposed else (lambda p: p.detach().float().contiguous())
         for tag, lin in names:
-            wt = lin.weight.detach().float().t().contiguous()
+            wt = f(lin.weight)
             b = lin.bias.detach().float().contiguous()
             keep += [wt, b]
             setattr(st, tag + "_wt", wt.data_ptr())
             setattr(st, tag + "_b", b.data_ptr())
         for tag, p in (("gru_ih_wt", cell.weight_ih), ("gru_hh_wt", cell.weight_hh)):
-            wt = p.detach().float().t().contiguous()
+            wt = f(p)
             keep.append(wt)
             setattr(st, tag, wt.data_ptr())
         for tag, p in (("gru_ih_b", cell.bias_ih), ("gru_hh_b", cell.bias_hh)):
@@ -818,7 +830,7 @@ def hsvrnn_weight_struct(mod) -> "L.HsvrnnWeights":
             keep.append(b)
             setattr(st, tag, b.data_ptr())
         return st, keep
-    return _cached(mod, "hsvrnn", params, build)[0]
+    return _cached(mod, "hsvrnn" if transposed else "hsvrnn_oi", params, build)[0]
 
 
 def hsvrnn_step(wstruct, h, kp_flat, eps, offset, order, parents, K: int, posterior: bool,
@@ -837,6 +849,45 @@ def hsvrnn_step(wstruct, h, kp_flat, eps, offset, order, parents, K: int, poster
            L.ptr(parents), B, K, S, int(posterior), L.ptr(h_out), L.ptr(kp_out), L.ptr(z_out), L.ptr(R_out),
            L.ptr(post), L.ptr(prior), L.stream())
     return h_out, kp_out, z_out, R_out, post, prior
+
+
+def hsvrnn_step_record(wstruct, h, kp_flat, eps, offset, order, parents, K: int, h_out, kp_out, z_out, R_out, post_out,
+                       prior_out, pick_out):
+    """A posterior `hsvrnn_step` into caller-provided outputs that also records the picked sample (pick_out (B) int32)."""
+    _need_cuda(h, kp_flat, eps, offset, h_out, pick_out)
+    L.call("nm_hsvrnn_step_record", ctypes.byref(wstruct), L.ptr(h), L.ptr(kp_flat), L.ptr(eps), L.ptr(offset),
+           L.ptr(order), L.ptr(parents), h.shape[0], K, eps.shape[0], 1, L.ptr(h_out), L.ptr(kp_out), L.ptr(z_out),
+           L.ptr(R_out), L.ptr(post_out), L.ptr(prior_out), L.ptr(pick_out), L.stream())
+
+
+def hsvrnn_backward_workspace(B: int, T: int, device) -> torch.Tensor:
+    """(T, B, row) fp32 records of the reverse loop; step t writes slice t."""
+    row = L.query("nm_hsvrnn_backward_workspace_bytes", 1, 1) // 4
+    return torch.empty(T, B, row, dtype=torch.float32, device=device)
+
+
+def hsvrnn_step_backward(wt, w, h, kp_flat, eps, pick, f, z, R, offset, order, parents, K: int, dh_next, dh_ext, df, dR, dz,
+                         dpost, dprior, dh_out, doffset, rows):
+    """Backward of one conditioned step (see include/nm_b200.h): writes dh_out, accumulates doffset, fills rows."""
+    _need_cuda(h, kp_flat, eps, pick, f, z, R, offset, dh_next, dh_ext, df, dR, dz, dpost, dprior, dh_out, doffset, rows)
+    L.call("nm_hsvrnn_step_backward", ctypes.byref(wt), ctypes.byref(w), L.ptr(h), L.ptr(kp_flat), L.ptr(eps), L.ptr(pick),
+           L.ptr(f), L.ptr(z), L.ptr(R), L.ptr(offset), L.ptr(order), L.ptr(parents), h.shape[0], K, eps.shape[0],
+           L.ptr(dh_next), L.ptr(dh_ext), L.ptr(df), L.ptr(dR), L.ptr(dz), L.ptr(dpost), L.ptr(dprior), L.ptr(dh_out),
+           L.ptr(doffset), L.ptr(rows), L.stream())
+
+
+def hsvrnn_weight_grads(rows, h, kp, f, z, dh0, offset, doffset, offset_param, grads):
+    """Every parameter gradient of the reverse loop in one launch.  grads: tensors shaped like `hsvrnn_params` (the last,
+    offset_param's, may be None); all are fully overwritten."""
+    _need_cuda(rows, h, kp, f, z, dh0, offset, doffset, offset_param)
+    T, B = rows.shape[:2]
+    K = kp.shape[-1] // 4
+    g = L.HsvrnnGrads()
+    for (name, _), t in zip(L.HsvrnnGrads._fields_, grads):
+        _need_cuda(t)
+        setattr(g, name, L.ptr(t))
+    L.call("nm_hsvrnn_weight_grads", L.ptr(rows), L.ptr(h), L.ptr(kp), L.ptr(f), L.ptr(z), L.ptr(dh0), L.ptr(offset),
+           L.ptr(doffset), L.ptr(offset_param), B, T, K, ctypes.byref(g), L.stream())
 
 
 def hsvrnn_decode_pose(wstruct, dec_in, offset, order, parents, K: int):
