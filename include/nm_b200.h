@@ -162,7 +162,9 @@ int nm_chamfer_vol_fit(const float* seq, const float* keypoints, const float* li
  * feature: act (n, g^3, C); w1 (K, C); prev (n/frames_per_clip, K, g^3); heat/gaussians (n, K, g^3); keypoints (n,K,4).
  * heat_mean (optional, (n,K)): per-keypoint heat-map mean = input of get_keypoint_sparsity_loss (:92-103).
  * gauss_width = 2*(sigma/g)^2 computed by the caller in double.
- * prop_dev (optional, also in nm_heatmap_head_backward): device pointer to (pw0, pw1, pb) - overrides the by-value copies. */
+ * prop_dev (optional, also in nm_heatmap_head_backward): device pointer to (pw0, pw1, pb) - overrides the by-value copies.
+ * K <= 64 here, in nm_gaussian_render / nm_decoder_adjust and in their backward entry points (K <= 24 runs the tuned
+ * kernels). */
 int nm_heatmap_head(const void* feature, const float* w1, const float* b1, int n, int g, int C, int K, int mode,
                     const float* prev, int frames_per_clip, float pw0, float pw1, float pb, const float* prop_dev,
                     const float* linspace, float gauss_width, float* heat, float* keypoints, float* gaussians, float* heat_mean,
@@ -191,7 +193,8 @@ typedef struct nm_hsvrnn_weights {
 /* One time step (hsvrnn_bvh.py:89-135 posterior / :208-225 prior).  `w` is a HOST pointer to the struct.
  * h_in/h_out (B,512); kp (B,4K) detected keypoints (posterior); eps (S,B,128) standard-normal draws;
  * offset (B,K,3); order/parents (K) int32 = priority.indices / parents; kp_out (B,4K) decoded keypoints fed to
- * the GRU; optional outputs: z_out (B,128), R_out (B,K,9), post_out / prior_out (B,256) = mean | std. */
+ * the GRU; optional outputs: z_out (B,128), R_out (B,K,9), post_out / prior_out (B,256) = mean | std.
+ * 0 < K <= 64 here and in every nm_hsvrnn_* entry point (K <= 24 runs the tuned kernels); S <= 16. */
 int nm_hsvrnn_step(const nm_hsvrnn_weights* w, const float* h_in, const float* kp, const float* eps, const float* offset,
                    const int* order, const int* parents, int B, int K, int S, int posterior, float* h_out,
                    float* kp_out, float* z_out, float* R_out, float* post_out, float* prior_out, void* stream);

@@ -16,7 +16,9 @@
 
 namespace {
 
-constexpr int KMAX = 24;
+// Keypoint capacity of the heat-map / adjust / chamfer backward kernels: K <= kTunedK (the shipped 24) runs the tuned
+// instantiations, 24 < K <= kMaxK a set compiled for kMaxK (template parameter KMAX).
+constexpr int kTunedK = 24, kMaxK = 64;
 
 // ------------------------------------------------------------------ trilinear x2 backward
 // d_in[i] = sum_{j in -1..2} w_j * g[clamp(2i + j)], w = (.25, .75, .75, .25) per axis (the transpose of PyTorch's
@@ -209,7 +211,13 @@ reduce_cols_kernel(const float* __restrict__ partial, long long rows, int ld, in
 //   u  [k][s] = w1 f      thread = (voxel, 6 keypoints): per 4 channels 1 LDS.128 of f + 6 broadcast LDS.128 of w1, 24 FMA
 //   dfeat[s][c] = W1^T du thread = (4 voxels, 8 channels): per keypoint 1 + 2 LDS.128, 32 FMA
 //   dW1[k][c] += du f^T   thread = (channel, 12 or 24 keypoints): per voxel 1 LDS + 3 or 6 broadcast LDS.128, 12 or 24 FMA
-template <int C>
+// At capacity 64 the dW1 tile is split over blockIdx.z: block z owns keypoints [KW z, KW z + KW) of dW1 (KW = 32 at
+// C = 128, 16 at C = 256: 16 accumulators per thread instead of 32 or 64, which spill); every z computes u and du for all
+// keypoints, only z = 0 writes dfeat, dq, db1 and the propagation partials.
+template <int C, int KMAX>
+constexpr int head_bwd_kw() { return KMAX <= kTunedK ? KMAX : (C == 256 ? 16 : 32); }
+
+template <int C, int KMAX>
 __global__ void __launch_bounds__(256)
 head_bwd_kernel(const __half* __restrict__ feature, const float* __restrict__ w1, const float* __restrict__ b1, int K, int g,
                 int mode, const float* __restrict__ prev, int frames_per_clip, float pw0, float pw1, float pb,
@@ -222,7 +230,9 @@ head_bwd_kernel(const __half* __restrict__ feature, const float* __restrict__ w1
   if (prop_dev) { pw0 = __ldg(prop_dev); pw1 = __ldg(prop_dev + 1); pb = __ldg(prop_dev + 2); }   // live parameters
   constexpr int TS = 64;                                   // voxels per tile
   constexpr int FS = C + 4;                                // fp32 feature row stride: 16-byte aligned rows, conflict-free LDS.128
-  constexpr int KPT = KMAX * C / 256;                      // dW1 accumulators per thread (12 or 24)
+  constexpr int KW = head_bwd_kw<C, KMAX>();               // keypoints of dW1 per block
+  constexpr int KPT = KW * C / 256;                        // dW1 accumulators per thread (12 or 24; 16 at 64)
+  const bool lead = KW == KMAX || blockIdx.z == 0;         // writes dfeat, dq, db1 and the propagation partials
   constexpr int NC8 = C / 8, VPT = TS / (256 / NC8);       // dfeat: voxels per thread (4 or 8, in rounds of 4)
   extern __shared__ __align__(16) float smem[];
   float* s_w = smem;                                       // [KMAX][C]
@@ -270,7 +280,7 @@ head_bwd_kernel(const __half* __restrict__ feature, const float* __restrict__ w1
 #pragma unroll
   for (int i = 0; i < KPT; i++) accw[i] = 0.f;
   float accb = 0.f, sp0 = 0.f, sp1 = 0.f, sp2 = 0.f;
-  const int wc = threadIdx.x % C, wk0 = (threadIdx.x / C) * KPT;      // dW1 ownership: channel wc, keypoints wk0..
+  const int wc = threadIdx.x % C, wk0 = (KW == KMAX ? 0 : blockIdx.z * KW) + (threadIdx.x / C) * KPT;   // dW1: channel wc, keypoints wk0..
   const __half* fbase = feature + (long long)n * S * C;
   for (int tile = tile0; tile < tile0 + tiles; tile++) {
     const int s0 = tile * TS;
@@ -317,7 +327,7 @@ head_bwd_kernel(const __half* __restrict__ feature, const float* __restrict__ w1
             float dhm = s_co[k * 4] + s_co[k * 4 + 1] * lx + s_co[k * 4 + 2] * ly + s_co[k * 4 + 3] * lz;
             if (dheat) dhm += dheat[((long long)n * K + k) * S + s];
             const float dq = dhm * (1.f - expf(-hm));
-            dq_out[((long long)n * K + k) * S + s] = dq;
+            if (lead) dq_out[((long long)n * K + k) * S + s] = dq;
             sp0 = fmaf(dq, h, sp0);
             sp1 = fmaf(dq, pv, sp1);
             sp2 += dq;
@@ -338,7 +348,7 @@ head_bwd_kernel(const __half* __restrict__ feature, const float* __restrict__ w1
     }
     __syncthreads();
     // dfeat[s][c] = grad_scale * sum_k du[k][s] w1[k][c]: thread = (4 voxels, channels c8*4 .. +3 and C/2 + c8*4 .. +3)
-    {
+    if (lead) {
       const int c8 = threadIdx.x % NC8, slg = threadIdx.x / NC8;
 #pragma unroll 1
       for (int v0 = 0; v0 < VPT; v0 += 4) {
@@ -384,7 +394,7 @@ head_bwd_kernel(const __half* __restrict__ feature, const float* __restrict__ w1
         accw[q * 4 + 3] = fmaf(d.w, f, accw[q * 4 + 3]);
       }
     }
-    if (threadIdx.x < KMAX) {
+    if (lead && threadIdx.x < KMAX) {
       const float4* dr = reinterpret_cast<const float4*>(s_du + threadIdx.x * TS);
       float t = 0.f;
 #pragma unroll 4
@@ -399,6 +409,7 @@ head_bwd_kernel(const __half* __restrict__ feature, const float* __restrict__ w1
 #pragma unroll
   for (int i = 0; i < KPT; i++)
     if (wk0 + i < K) pw_partial[(part * K + wk0 + i) * C + wc] = accw[i];
+  if (!lead) return;
   if (threadIdx.x < K) pb_partial[part * K + threadIdx.x] = accb;
   if (mode == 1) {
     s_red[threadIdx.x * 3] = sp0; s_red[threadIdx.x * 3 + 1] = sp1; s_red[threadIdx.x * 3 + 2] = sp2;
@@ -459,9 +470,11 @@ __device__ __forceinline__ void adj_load_dz(const __half* dy, const __half* y, l
 }
 
 // render backward accumulation for the keypoints owned by this thread (6 of them, one voxel)
+template <int KMAX>
 struct RenderAcc { float v[KMAX / 4][4]; };
 
 // Gaussians of the tile, voxel-major: s_GT[sl][KMAX]
+template <int KMAX>
 __device__ __forceinline__ void adj_gauss_tile(const float* s_e, const float* s_kp, int K, int g, int s0, float* s_GT) {
   for (int i = threadIdx.x; i < KMAX * kAdjTS; i += 256) {
     const int k = i / kAdjTS, sl = i % kAdjTS, s = s0 + sl;
@@ -476,9 +489,10 @@ __device__ __forceinline__ void adj_gauss_tile(const float* s_e, const float* s_
 
 // dG[k][s] = sum_co W[co][col0 + k] dz[co][s] for this thread's 6 keypoints (per co: one LDS of dz, three broadcast
 // LDS.64 of the weights, 6 FMA), accumulated into the render gradient
+template <int KMAX>
 __device__ __forceinline__ void adj_render_bwd(const float* s_wg /* [128][KMAX] */, const float* s_dz, const float* s_e,
                                                const float* s_kp, const float* lin, int K, int g, int s0, float width,
-                                               RenderAcc& r) {
+                                               RenderAcc<KMAX>& r) {
   constexpr int KG = KMAX / 4;
   const int sl = threadIdx.x % kAdjTS, kg = threadIdx.x / kAdjTS, s = s0 + sl;
   const int x = s / (g * g), yy = (s / g) % g, z = s % g;
@@ -512,15 +526,16 @@ __device__ __forceinline__ void adj_render_bwd(const float* s_wg /* [128][KMAX] 
   }
 }
 
-// dWg[co][k0 .. k0+11] += sum_s dz[co][s] G[k][s] (thread = output channel co, 12 keypoints; per voxel one LDS of dz and
-// three broadcast LDS.128 of the Gaussians); returns sum_s dz[co][s] through `dsum`
-__device__ __forceinline__ void adj_wg_accumulate(const float* s_dzT, const float* s_GT, int co, int k0, float (&acc)[12], float& dsum) {
+// dWg[co][k0 .. k0+KMAX/2-1] += sum_s dz[co][s] G[k][s] (thread = output channel co, half the keypoints; per voxel one LDS of
+// dz and KMAX/8 broadcast LDS.128 of the Gaussians); returns sum_s dz[co][s] through `dsum`
+template <int KMAX>
+__device__ __forceinline__ void adj_wg_accumulate(const float* s_dzT, const float* s_GT, int co, int k0, float (&acc)[KMAX / 2], float& dsum) {
 #pragma unroll 2
   for (int sl = 0; sl < kAdjTS; sl++) {
     const float d = s_dzT[sl * kAdjDT + co];
     const float4* gr = reinterpret_cast<const float4*>(s_GT + sl * KMAX + k0);
 #pragma unroll
-    for (int q = 0; q < 3; q++) {
+    for (int q = 0; q < KMAX / 8; q++) {
       const float4 gv = gr[q];
       acc[q * 4] = fmaf(d, gv.x, acc[q * 4]);
       acc[q * 4 + 1] = fmaf(d, gv.y, acc[q * 4 + 1]);
@@ -532,26 +547,36 @@ __device__ __forceinline__ void adj_wg_accumulate(const float* s_dzT, const floa
 }
 
 // fold the per-thread render accumulators over the 64 voxel lanes of each keypoint group (fixed order)
-__device__ __forceinline__ void adj_render_store(const RenderAcc& r, float* s_tmp /* [256][24] */, int K, float* out /* [K][4] */) {
+template <int KMAX>
+__device__ __forceinline__ void adj_render_store(const RenderAcc<KMAX>& r, float* s_tmp /* [256][KMAX] */, int K, float* out /* [K][4] */) {
 #pragma unroll
   for (int kk = 0; kk < KMAX / 4; kk++)
 #pragma unroll
-    for (int q = 0; q < 4; q++) s_tmp[threadIdx.x * 24 + kk * 4 + q] = r.v[kk][q];
+    for (int q = 0; q < 4; q++) s_tmp[threadIdx.x * KMAX + kk * 4 + q] = r.v[kk][q];
   __syncthreads();
   if (threadIdx.x < KMAX * 4) {
     const int k = threadIdx.x / 4, q = threadIdx.x % 4, kg = k / (KMAX / 4), kk = k % (KMAX / 4);
     float t = 0.f;
-    for (int sl = 0; sl < kAdjTS; sl++) t += s_tmp[(kg * kAdjTS + sl) * 24 + kk * 4 + q];
+    for (int sl = 0; sl < kAdjTS; sl++) t += s_tmp[(kg * kAdjTS + sl) * KMAX + kk * 4 + q];
     if (k < K) out[k * 4 + q] = t;
   }
   __syncthreads();
 }
 
-// shared-memory floats: frame kernel / extra of the clip kernel (s_tmp of adj_render_store aliases s_dz .. s_dzT)
-constexpr int kAdjFrameFloats = kAdjC * KMAX + kAdjC * kAdjDS + kAdjTS * kAdjDT + kAdjTS * KMAX + KMAX * 96 + KMAX * 4;
-constexpr int kAdjClipFloats = kAdjFrameFloats + kAdjC * kAdjC + kAdjTS * kAdjC + kAdjTS * 4;
-static_assert(256 * 24 <= kAdjC * kAdjDS + kAdjTS * kAdjDT, "s_tmp must fit in the dz buffers");
+// shared-memory floats: frame kernel / extra of the clip kernel (s_tmp of adj_render_store aliases s_dz .. s_dzT).  At
+// capacity 64 the clip kernel would need 237 KB with the first-feature weights staged; it reads them from L2 instead.
+template <int KMAX>
+constexpr int adj_frame_floats() { return kAdjC * KMAX + kAdjC * kAdjDS + kAdjTS * kAdjDT + kAdjTS * KMAX + KMAX * 96 + KMAX * 4; }
+template <int KMAX>
+constexpr bool adj_wff_shared() { return KMAX <= kTunedK; }
+template <int KMAX>
+constexpr int adj_clip_floats() {
+  return adj_frame_floats<KMAX>() + (adj_wff_shared<KMAX>() ? kAdjC * kAdjC : 0) + kAdjTS * kAdjC + kAdjTS * 4;
+}
+static_assert(256 * kMaxK <= kAdjC * kAdjDS + kAdjTS * kAdjDT, "s_tmp must fit in the dz buffers");
+static_assert(adj_clip_floats<kMaxK>() * 4 <= 227 * 1024, "adjust_bwd_clip_kernel<64> must fit in shared memory");
 
+template <int KMAX>
 __global__ void __launch_bounds__(256)
 adjust_bwd_frame_kernel(const __half* __restrict__ dy, const __half* __restrict__ y, const float* __restrict__ kp,
                         const float* __restrict__ W, int ld, int K, int g, const float* __restrict__ lin, float width,
@@ -564,7 +589,7 @@ adjust_bwd_frame_kernel(const __half* __restrict__ dy, const __half* __restrict_
   float* s_GT = s_dzT + kAdjTS * kAdjDT;                  // [TS][KMAX]
   float* s_e = s_GT + kAdjTS * KMAX;                      // [KMAX][3][32]
   float* s_kp = s_e + KMAX * 96;                          // [KMAX][4]
-  float* s_tmp = s_dz;                                    // [256][24], after the tile loop
+  float* s_tmp = s_dz;                                    // [256][KMAX], after the tile loop
   const int n = blockIdx.x, S = g * g * g;
   for (int i = threadIdx.x; i < kAdjC * KMAX; i += 256) {
     const int co = i / KMAX, k = i % KMAX;
@@ -572,31 +597,33 @@ adjust_bwd_frame_kernel(const __half* __restrict__ dy, const __half* __restrict_
   }
   adj_stage_exps(kp + (long long)n * K * 4, K, g, lin, width, s_e, s_kp);
   __syncthreads();
-  RenderAcc r;
+  RenderAcc<KMAX> r;
 #pragma unroll
   for (int kk = 0; kk < KMAX / 4; kk++)
 #pragma unroll
     for (int q = 0; q < 4; q++) r.v[kk][q] = 0.f;
-  float accw[12], accb = 0.f;
+  constexpr int KH = KMAX / 2;                            // keypoints of dW per thread
+  float accw[KH], accb = 0.f;
 #pragma unroll
-  for (int i = 0; i < 12; i++) accw[i] = 0.f;
-  const int wco = threadIdx.x % kAdjC, wk0 = (threadIdx.x / kAdjC) * 12;
+  for (int i = 0; i < KH; i++) accw[i] = 0.f;
+  const int wco = threadIdx.x % kAdjC, wk0 = (threadIdx.x / kAdjC) * KH;
   for (int s0 = 0; s0 < S; s0 += kAdjTS) {
     adj_load_dz(dy, y, n, 1, S, s0, inv_scale, s_dz, s_dzT);
-    adj_gauss_tile(s_e, s_kp, K, g, s0, s_GT);
+    adj_gauss_tile<KMAX>(s_e, s_kp, K, g, s0, s_GT);
     __syncthreads();
-    adj_render_bwd(s_wg, s_dz, s_e, s_kp, lin, K, g, s0, width, r);
+    adj_render_bwd<KMAX>(s_wg, s_dz, s_e, s_kp, lin, K, g, s0, width, r);
     // dW[co][k] += sum_s dz[co][s] G[k][s];  db[co] += sum_s dz[co][s]
-    adj_wg_accumulate(s_dzT, s_GT, wco, wk0, accw, accb);
+    adj_wg_accumulate<KMAX>(s_dzT, s_GT, wco, wk0, accw, accb);
     __syncthreads();
   }
-  adj_render_store(r, s_tmp, K, dkp + (long long)n * K * 4);
+  adj_render_store<KMAX>(r, s_tmp, K, dkp + (long long)n * K * 4);
 #pragma unroll
-  for (int i = 0; i < 12; i++) pwg[((long long)n * kAdjC + wco) * KMAX + wk0 + i] = accw[i];
+  for (int i = 0; i < KH; i++) pwg[((long long)n * kAdjC + wco) * KMAX + wk0 + i] = accw[i];
   if (threadIdx.x < kAdjC) pbias[(long long)n * kAdjC + threadIdx.x] = accb;
 }
 
 // per clip, split over `splits` voxel ranges: works on dzs = sum over the clip's frames of dz
+template <int KMAX>
 __global__ void __launch_bounds__(256)
 adjust_bwd_clip_kernel(const __half* __restrict__ dy, const __half* __restrict__ y, const __half* __restrict__ ff,
                        const float* __restrict__ kp, const float* __restrict__ W, int ld, int K, int g, int frames_per_clip,
@@ -610,37 +637,40 @@ adjust_bwd_clip_kernel(const __half* __restrict__ dy, const __half* __restrict__
   float* s_GT = s_dzT + kAdjTS * kAdjDT;                  // [TS][KMAX]
   float* s_e = s_GT + kAdjTS * KMAX;                      // [KMAX][3][32]
   float* s_kp = s_e + KMAX * 96;                          // [KMAX][4]
-  float* s_wff = s_kp + KMAX * 4;                         // [128 co][128 c]
-  float* s_ff = s_wff + kAdjC * kAdjC;                    // [TS][128]
+  constexpr bool kWff = adj_wff_shared<KMAX>();
+  float* s_wff = s_kp + KMAX * 4;                         // [128 co][128 c] (capacity 24 only)
+  float* s_ff = s_wff + (kWff ? kAdjC * kAdjC : 0);       // [TS][128]
   float* s_xyz = s_ff + kAdjTS * kAdjC;                   // [TS][4]: lin[x], lin[y], lin[z] of the tile's voxels
-  float* s_tmp = s_dz;                                    // [256][24], after the tile loop
+  float* s_tmp = s_dz;                                    // [256][KMAX], after the tile loop
   const int clip = blockIdx.x, split = blockIdx.y, splits = gridDim.y, S = g * g * g;
   const int per = S / splits;                             // multiple of TS (checked by the host)
-  for (int i = threadIdx.x; i < kAdjC * kAdjC; i += 256) s_wff[i] = W[(long long)(i / kAdjC) * ld + K + i % kAdjC];
+  if (kWff)
+    for (int i = threadIdx.x; i < kAdjC * kAdjC; i += 256) s_wff[i] = W[(long long)(i / kAdjC) * ld + K + i % kAdjC];
   for (int i = threadIdx.x; i < kAdjC * KMAX; i += 256) {
     const int co = i / KMAX, k = i % KMAX;
     s_wg[i] = k < K ? W[(long long)co * ld + K + kAdjC + k] : 0.f;
   }
   adj_stage_exps(kp + (long long)clip * frames_per_clip * K * 4, K, g, lin, width, s_e, s_kp);
   __syncthreads();
-  RenderAcc r;
+  RenderAcc<KMAX> r;
 #pragma unroll
   for (int kk = 0; kk < KMAX / 4; kk++)
 #pragma unroll
     for (int q = 0; q < 4; q++) r.v[kk][q] = 0.f;
   // dW[:, K:K+128]: thread = (4 feature channels fc4*4.., 16 output channels cog*16..)
-  float accf[16][4], accg[12], accx[3] = {0.f, 0.f, 0.f}, dsum = 0.f;
+  constexpr int KH = KMAX / 2;
+  float accf[16][4], accg[KH], accx[3] = {0.f, 0.f, 0.f}, dsum = 0.f;
 #pragma unroll
   for (int i = 0; i < 16; i++)
 #pragma unroll
     for (int e = 0; e < 4; e++) accf[i][e] = 0.f;
 #pragma unroll
-  for (int i = 0; i < 12; i++) accg[i] = 0.f;
+  for (int i = 0; i < KH; i++) accg[i] = 0.f;
   const int wc = threadIdx.x % kAdjC, half_id = threadIdx.x / kAdjC;   // half_id: 0 / 1
   const int fc4 = threadIdx.x % 32, cog = threadIdx.x / 32;            // cog doubles as the voxel group of d first_feature
   for (int s0 = split * per; s0 < (split + 1) * per; s0 += kAdjTS) {
     adj_load_dz(dy, y, (long long)clip * frames_per_clip, frames_per_clip, S, s0, inv_scale, s_dz, s_dzT);
-    adj_gauss_tile(s_e, s_kp, K, g, s0, s_GT);
+    adj_gauss_tile<KMAX>(s_e, s_kp, K, g, s0, s_GT);
     for (int i = threadIdx.x; i < kAdjTS * (kAdjC / 4); i += 256) {
       const int sl = i / (kAdjC / 4), c4 = i % (kAdjC / 4);
       const uint2 raw = *reinterpret_cast<const uint2*>(ff + ((long long)clip * S + s0 + sl) * kAdjC + c4 * 4);
@@ -653,7 +683,7 @@ adjust_bwd_clip_kernel(const __half* __restrict__ dy, const __half* __restrict__
       *reinterpret_cast<float4*>(s_xyz + threadIdx.x * 4) = make_float4(lin[s / (g * g)], lin[(s / g) % g], lin[s % g], 0.f);
     }
     __syncthreads();
-    adj_render_bwd(s_wg, s_dz, s_e, s_kp, lin, K, g, s0, width, r);
+    adj_render_bwd<KMAX>(s_wg, s_dz, s_e, s_kp, lin, K, g, s0, width, r);
     // d first_feature[s][c] = grad_scale * sum_co W[co][K + c] dzs[co][s]: thread = (channels fc4*4.., voxels cog*8..);
     // per co one LDS.128 of the weights and two broadcast LDS.128 of dzs for 32 FMA
     {
@@ -664,7 +694,13 @@ adjust_bwd_clip_kernel(const __half* __restrict__ dy, const __half* __restrict__
         for (int e = 0; e < 4; e++) o[v][e] = 0.f;
 #pragma unroll 2
       for (int co = 0; co < kAdjC; co++) {
-        const float4 w = *reinterpret_cast<const float4*>(s_wff + co * kAdjC + fc4 * 4);
+        float4 w;
+        if (kWff) {
+          w = *reinterpret_cast<const float4*>(s_wff + co * kAdjC + fc4 * 4);
+        } else {
+          const float* wr = W + (long long)co * ld + K + fc4 * 4;
+          w = make_float4(__ldg(wr), __ldg(wr + 1), __ldg(wr + 2), __ldg(wr + 3));
+        }
         const float4 d0 = *reinterpret_cast<const float4*>(s_dz + co * kAdjDS + cog * 8);
         const float4 d1 = *reinterpret_cast<const float4*>(s_dz + co * kAdjDS + cog * 8 + 4);
         const float dv[8] = {d0.x, d0.y, d0.z, d0.w, d1.x, d1.y, d1.z, d1.w};
@@ -702,8 +738,8 @@ adjust_bwd_clip_kernel(const __half* __restrict__ dy, const __half* __restrict__
         }
       }
     }
-    // dW[co][K + 128 + k] += sum_s dzs[co][s] G0[k][s]  (co = wc, 12 keypoints);  coords: thread co = wc of half 0
-    adj_wg_accumulate(s_dzT, s_GT, wc, half_id * 12, accg, dsum);
+    // dW[co][K + 128 + k] += sum_s dzs[co][s] G0[k][s]  (co = wc, KMAX / 2 keypoints);  coords: thread co = wc of half 0
+    adj_wg_accumulate<KMAX>(s_dzT, s_GT, wc, half_id * KH, accg, dsum);
     if (half_id == 0) {
 #pragma unroll 4
       for (int sl = 0; sl < kAdjTS; sl++) {
@@ -717,7 +753,7 @@ adjust_bwd_clip_kernel(const __half* __restrict__ dy, const __half* __restrict__
     __syncthreads();
   }
   const long long part = (long long)clip * splits + split;
-  adj_render_store(r, s_tmp, K, dkp0 + part * K * 4);
+  adj_render_store<KMAX>(r, s_tmp, K, dkp0 + part * K * 4);
   constexpr int LDP = kAdjC + KMAX + 3;
   float* o = pw + part * kAdjC * LDP;
 #pragma unroll
@@ -725,12 +761,13 @@ adjust_bwd_clip_kernel(const __half* __restrict__ dy, const __half* __restrict__
 #pragma unroll
     for (int e = 0; e < 4; e++) o[(long long)(cog * 16 + i) * LDP + fc4 * 4 + e] = accf[i][e];
 #pragma unroll
-  for (int i = 0; i < 12; i++) o[(long long)wc * LDP + kAdjC + half_id * 12 + i] = accg[i];
+  for (int i = 0; i < KH; i++) o[(long long)wc * LDP + kAdjC + half_id * KH + i] = accg[i];
   if (half_id == 0)
     for (int a = 0; a < 3; a++) o[(long long)wc * LDP + kAdjC + KMAX + a] = accx[a];
 }
 
 // dW (128, 2K + 131) and db (128) from the per-frame / per-clip partials; dkp[clip's frame 0] += sum over splits of dkp0
+template <int KMAX>
 __global__ void adjust_bwd_finalize_kernel(const float* __restrict__ pwg, const float* __restrict__ pbias, const float* __restrict__ pw,
                                            const float* __restrict__ dkp0, int n, int parts, int clips, int splits,
                                            int frames_per_clip, int K, float* __restrict__ dW, float* __restrict__ db,
@@ -764,6 +801,7 @@ __global__ void adjust_bwd_finalize_kernel(const float* __restrict__ pwg, const 
 // ------------------------------------------------------------------ chamfer volume-fitting loss backward
 // loss_n = sum_v o_v min_k |c_v - kp_k|^2 / sum_v o_v  ->  d kp_k = g_n / sum o * sum_{v: argmin = k} o_v 2 (kp_k - c_v)
 constexpr int kChbBlocks = 32;
+template <int KMAX>
 __global__ void __launch_bounds__(256)
 chamfer_bwd_kernel(const float* __restrict__ seq, const float* __restrict__ kp, int K, int G, const float* __restrict__ lin,
                    float* __restrict__ partial /* [n][blocks][K*3 + 1] */) {
@@ -1223,6 +1261,21 @@ static int head_bwd_splits(int n) {
   return splits;
 }
 
+template <int C, int KMAX>
+static int launch_head_bwd(int n, int splits, cudaStream_t st, const __half* feature, const float* w1, const float* b1, int K, int g,
+                           int mode, const float* prev, int frames_per_clip, float pw0, float pw1, float pb, const float* prop_dev,
+                           const float* lin, const float* heat, const float* kp, const float* heat_mean, const float* dkp,
+                           const float* dmean_up, const float* dheat, const float* dq_in, float grad_scale, __half* dfeat,
+                           float* dq_out, float* pwp, float* pbp, float* ppp) {
+  const size_t smem = (size_t)(KMAX * C + 64 * (C + 4) + 2 * KMAX * 64 + KMAX * 4 + 256 * 3) * sizeof(float);
+  const dim3 grid(n, splits, KMAX / head_bwd_kw<C, KMAX>());
+  NM_CHECK_CUDA(cudaFuncSetAttribute(head_bwd_kernel<C, KMAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  head_bwd_kernel<C, KMAX><<<grid, 256, smem, st>>>(feature, w1, b1, K, g, mode, prev, frames_per_clip, pw0, pw1, pb, prop_dev, lin,
+                                                    heat, kp, heat_mean, dkp, dmean_up, dheat, dq_in, grad_scale, dfeat, dq_out,
+                                                    pwp, pbp, ppp);
+  return NM_OK;
+}
+
 extern "C" size_t nm_heatmap_head_backward_workspace_bytes(int n, int C, int K) {
   const size_t rows = (size_t)n * head_bwd_splits(n);
   return (rows * K * C + rows * K + rows * 3) * sizeof(float);
@@ -1236,7 +1289,7 @@ extern "C" int nm_heatmap_head_backward(const void* feature, const float* w1, co
                                         const float* grad_heat, const float* dq_in, float grad_scale, void* grad_feature,
                                         float* dq_out, float* dw1, float* db1, float* dprop, void* workspace, void* stream) {
   NM_CHECK_ARG(feature && w1 && b1 && linspace && grad_feature && dw1 && db1 && workspace, "nm_heatmap_head_backward: null pointer");
-  NM_CHECK_ARG(K <= KMAX && (g == 8 || g == 16 || g == 32), "nm_heatmap_head_backward: K=%d g=%d unsupported", K, g);
+  NM_CHECK_ARG(K <= kMaxK && (g == 8 || g == 16 || g == 32), "nm_heatmap_head_backward: K=%d g=%d unsupported", K, g);
   NM_CHECK_ARG(mode == 0 || (prev && heat && keypoints && heat_mean && dq_out && dprop),
                "nm_heatmap_head_backward: mode 1 needs prev, heat, keypoints, heat_mean, dq_out and dprop");
   NM_CHECK_ARG(C == 128 || C == 256, "nm_heatmap_head_backward: C=%d unsupported", C);
@@ -1247,23 +1300,20 @@ extern "C" int nm_heatmap_head_backward(const void* feature, const float* w1, co
   float* pwp = reinterpret_cast<float*>(workspace);
   float* pbp = pwp + (size_t)rows * K * C;
   float* ppp = pbp + (size_t)rows * K;
-  const size_t smem = (size_t)(KMAX * C + 64 * (C + 4) + 2 * KMAX * 64 + KMAX * 4 + 256 * 3) * sizeof(float);
-  const dim3 grid(n, splits);
-  if (C == 128) {
-    NM_CHECK_CUDA(cudaFuncSetAttribute(head_bwd_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    head_bwd_kernel<128><<<grid, 256, smem, st>>>(reinterpret_cast<const __half*>(feature), w1, b1, K, g, mode, prev, frames_per_clip,
-                                                  pw0, pw1, pb, prop_dev, linspace, heat, keypoints, heat_mean, grad_keypoints, grad_heat_mean,
-                                                  grad_heat, dq_in, grad_scale, reinterpret_cast<__half*>(grad_feature), dq_out, pwp, pbp, ppp);
-  } else {
-    NM_CHECK_CUDA(cudaFuncSetAttribute(head_bwd_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    head_bwd_kernel<256><<<grid, 256, smem, st>>>(reinterpret_cast<const __half*>(feature), w1, b1, K, g, mode, prev, frames_per_clip,
-                                                  pw0, pw1, pb, prop_dev, linspace, heat, keypoints, heat_mean, grad_keypoints, grad_heat_mean,
-                                                  grad_heat, dq_in, grad_scale, reinterpret_cast<__half*>(grad_feature), dq_out, pwp, pbp, ppp);
-  }
+  const __half* f = reinterpret_cast<const __half*>(feature);
+  __half* gf = reinterpret_cast<__half*>(grad_feature);
+  int rc;
+  if (K <= kTunedK)
+    rc = C == 128 ? launch_head_bwd<128, kTunedK>(n, splits, st, f, w1, b1, K, g, mode, prev, frames_per_clip, pw0, pw1, pb, prop_dev, linspace, heat, keypoints, heat_mean, grad_keypoints, grad_heat_mean, grad_heat, dq_in, grad_scale, gf, dq_out, pwp, pbp, ppp)
+                  : launch_head_bwd<256, kTunedK>(n, splits, st, f, w1, b1, K, g, mode, prev, frames_per_clip, pw0, pw1, pb, prop_dev, linspace, heat, keypoints, heat_mean, grad_keypoints, grad_heat_mean, grad_heat, dq_in, grad_scale, gf, dq_out, pwp, pbp, ppp);
+  else
+    rc = C == 128 ? launch_head_bwd<128, kMaxK>(n, splits, st, f, w1, b1, K, g, mode, prev, frames_per_clip, pw0, pw1, pb, prop_dev, linspace, heat, keypoints, heat_mean, grad_keypoints, grad_heat_mean, grad_heat, dq_in, grad_scale, gf, dq_out, pwp, pbp, ppp)
+                  : launch_head_bwd<256, kMaxK>(n, splits, st, f, w1, b1, K, g, mode, prev, frames_per_clip, pw0, pw1, pb, prop_dev, linspace, heat, keypoints, heat_mean, grad_keypoints, grad_heat_mean, grad_heat, dq_in, grad_scale, gf, dq_out, pwp, pbp, ppp);
+  if (rc) return rc;
   NM_CHECK_LAUNCH("head_bwd_kernel");
   reduce_cols_kernel<<<nm_cdiv(K * C, 32), dim3(32, 8), 0, st>>>(pwp, rows, K * C, K * C, 1.0f, dw1);
   NM_CHECK_LAUNCH("head_bwd(reduce dw1)");
-  reduce_cols_kernel<<<1, dim3(32, 8), 0, st>>>(pbp, rows, K, K, 1.0f, db1);
+  reduce_cols_kernel<<<nm_cdiv(K, 32), dim3(32, 8), 0, st>>>(pbp, rows, K, K, 1.0f, db1);
   NM_CHECK_LAUNCH("head_bwd(reduce db1)");
   if (mode == 1) {
     reduce_cols_kernel<<<1, dim3(32, 8), 0, st>>>(ppp, rows, 3, 3, 1.0f, dprop);
@@ -1273,10 +1323,46 @@ extern "C" int nm_heatmap_head_backward(const void* feature, const float* w1, co
 }
 
 constexpr int kAdjSplits = 8;
+
+template <int KMAX>
+size_t adjust_bwd_ws_bytes(size_t n, size_t n_clips) {
+  return (n * kAdjC * KMAX + n * kAdjC + n_clips * kAdjSplits * kAdjC * (kAdjC + KMAX + 3) + n_clips * kAdjSplits * KMAX * 4) *
+         sizeof(float);
+}
+
+template <int KMAX>
+static int launch_adjust_bwd(const __half* dy, const __half* y, const __half* ff, const float* keypoints, const float* weight,
+                             int n_clips, int frames_per_clip, int g, int K, const float* linspace, float gauss_width,
+                             float grad_scale, __half* dff, float* grad_keypoints, float* dweight, float* dbias, float* ws,
+                             cudaStream_t st) {
+  const int n = n_clips * frames_per_clip, ld = 2 * K + kAdjC + 3;
+  float* pwg = ws;
+  float* pbias = pwg + (size_t)n * kAdjC * KMAX;
+  float* pw = pbias + (size_t)n * kAdjC;
+  float* dkp0 = pw + (size_t)n_clips * kAdjSplits * kAdjC * (kAdjC + KMAX + 3);
+  const float inv_scale = 1.0f / grad_scale;
+  const size_t smem_f = (size_t)adj_frame_floats<KMAX>() * sizeof(float);
+  NM_CHECK_CUDA(cudaFuncSetAttribute(adjust_bwd_frame_kernel<KMAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_f));
+  adjust_bwd_frame_kernel<KMAX><<<n, 256, smem_f, st>>>(dy, y, keypoints, weight, ld, K, g, linspace, gauss_width, inv_scale,
+                                                        grad_keypoints, pwg, pbias);
+  NM_CHECK_LAUNCH("adjust_bwd_frame_kernel");
+  const size_t smem_c = (size_t)adj_clip_floats<KMAX>() * sizeof(float);
+  NM_CHECK_CUDA(cudaFuncSetAttribute(adjust_bwd_clip_kernel<KMAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_c));
+  adjust_bwd_clip_kernel<KMAX><<<dim3(n_clips, kAdjSplits), 256, smem_c, st>>>(dy, y, ff, keypoints, weight, ld, K, g,
+                                                                               frames_per_clip, linspace, gauss_width, inv_scale,
+                                                                               grad_scale, dff, dkp0, pw);
+  NM_CHECK_LAUNCH("adjust_bwd_clip_kernel");
+  const int total = kAdjC * ld + kAdjC + n_clips * K * 4;
+  adjust_bwd_finalize_kernel<KMAX><<<nm_cdiv(total, 128), 128, 0, st>>>(pwg, pbias, pw, dkp0, n, n_clips * kAdjSplits, n_clips,
+                                                                        kAdjSplits, frames_per_clip, K, dweight, dbias,
+                                                                        grad_keypoints);
+  NM_CHECK_LAUNCH("adjust_bwd_finalize_kernel");
+  return NM_OK;
+}
+
+// sized for the kMaxK layout (the larger one) whatever K is, since the size does not take K
 extern "C" size_t nm_decoder_adjust_backward_workspace_bytes(int n_clips, int frames_per_clip) {
-  const size_t n = (size_t)n_clips * frames_per_clip;
-  return (n * kAdjC * KMAX + n * kAdjC + (size_t)n_clips * kAdjSplits * kAdjC * (kAdjC + KMAX + 3) +
-          (size_t)n_clips * kAdjSplits * KMAX * 4) * sizeof(float);
+  return adjust_bwd_ws_bytes<kMaxK>((size_t)n_clips * frames_per_clip, (size_t)n_clips);
 }
 
 extern "C" int nm_decoder_adjust_backward(const void* grad_out, const void* out, const void* first_feature, const float* keypoints,
@@ -1285,32 +1371,18 @@ extern "C" int nm_decoder_adjust_backward(const void* grad_out, const void* out,
                                           float* grad_keypoints, float* dweight, float* dbias, void* workspace, void* stream) {
   NM_CHECK_ARG(grad_out && out && first_feature && keypoints && weight && linspace && grad_first_feature && grad_keypoints &&
                dweight && dbias && workspace, "nm_decoder_adjust_backward: null pointer");
-  NM_CHECK_ARG(K <= KMAX && (g == 8 || g == 16 || g == 32), "nm_decoder_adjust_backward: K=%d g=%d unsupported", K, g);
+  NM_CHECK_ARG(K <= kMaxK && (g == 8 || g == 16 || g == 32), "nm_decoder_adjust_backward: K=%d g=%d unsupported", K, g);
   if (n_clips == 0) return NM_OK;
-  cudaStream_t st = (cudaStream_t)stream;
-  const int n = n_clips * frames_per_clip, S = g * g * g, ld = 2 * K + kAdjC + 3;
-  float* pwg = reinterpret_cast<float*>(workspace);
-  float* pbias = pwg + (size_t)n * kAdjC * KMAX;
-  float* pw = pbias + (size_t)n * kAdjC;
-  float* dkp0 = pw + (size_t)n_clips * kAdjSplits * kAdjC * (kAdjC + KMAX + 3);
-  const float inv_scale = 1.0f / grad_scale;
-  const size_t smem_f = (size_t)kAdjFrameFloats * sizeof(float);
-  NM_CHECK_CUDA(cudaFuncSetAttribute(adjust_bwd_frame_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_f));
-  adjust_bwd_frame_kernel<<<n, 256, smem_f, st>>>(reinterpret_cast<const __half*>(grad_out), reinterpret_cast<const __half*>(out),
-                                                  keypoints, weight, ld, K, g, linspace, gauss_width, inv_scale, grad_keypoints, pwg, pbias);
-  NM_CHECK_LAUNCH("adjust_bwd_frame_kernel");
-  const size_t smem_c = (size_t)kAdjClipFloats * sizeof(float);
-  NM_CHECK_CUDA(cudaFuncSetAttribute(adjust_bwd_clip_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_c));
-  adjust_bwd_clip_kernel<<<dim3(n_clips, kAdjSplits), 256, smem_c, st>>>(
-      reinterpret_cast<const __half*>(grad_out), reinterpret_cast<const __half*>(out), reinterpret_cast<const __half*>(first_feature),
-      keypoints, weight, ld, K, g, frames_per_clip, linspace, gauss_width, inv_scale, grad_scale,
-      reinterpret_cast<__half*>(grad_first_feature), dkp0, pw);
-  NM_CHECK_LAUNCH("adjust_bwd_clip_kernel");
-  const int total = kAdjC * ld + kAdjC + n_clips * K * 4;
-  adjust_bwd_finalize_kernel<<<nm_cdiv(total, 128), 128, 0, st>>>(pwg, pbias, pw, dkp0, n, n_clips * kAdjSplits, n_clips, kAdjSplits,
-                                                                 frames_per_clip, K, dweight, dbias, grad_keypoints);
-  NM_CHECK_LAUNCH("adjust_bwd_finalize_kernel");
-  return NM_OK;
+  const __half* dy = reinterpret_cast<const __half*>(grad_out);
+  const __half* y = reinterpret_cast<const __half*>(out);
+  const __half* ff = reinterpret_cast<const __half*>(first_feature);
+  __half* dff = reinterpret_cast<__half*>(grad_first_feature);
+  float* ws = reinterpret_cast<float*>(workspace);
+  if (K <= kTunedK)
+    return launch_adjust_bwd<kTunedK>(dy, y, ff, keypoints, weight, n_clips, frames_per_clip, g, K, linspace, gauss_width,
+                                      grad_scale, dff, grad_keypoints, dweight, dbias, ws, (cudaStream_t)stream);
+  return launch_adjust_bwd<kMaxK>(dy, y, ff, keypoints, weight, n_clips, frames_per_clip, g, K, linspace, gauss_width,
+                                  grad_scale, dff, grad_keypoints, dweight, dbias, ws, (cudaStream_t)stream);
 }
 
 extern "C" size_t nm_chamfer_vol_fit_backward_workspace_bytes(int n, int K) { return (size_t)n * kChbBlocks * (K * 3 + 1) * sizeof(float); }
@@ -1318,12 +1390,20 @@ extern "C" size_t nm_chamfer_vol_fit_backward_workspace_bytes(int n, int K) { re
 extern "C" int nm_chamfer_vol_fit_backward(const float* seq, const float* keypoints, const float* linspace, const float* grad_out,
                                            int n, int K, int G, float* grad_keypoints, void* workspace, void* stream) {
   NM_CHECK_ARG(seq && keypoints && linspace && grad_out && grad_keypoints && workspace, "nm_chamfer_vol_fit_backward: null pointer");
-  NM_CHECK_ARG(K <= KMAX, "nm_chamfer_vol_fit_backward: K=%d unsupported", K);
+  NM_CHECK_ARG(K <= kMaxK, "nm_chamfer_vol_fit_backward: K=%d unsupported", K);
   if (n == 0) return NM_OK;
   cudaStream_t st = (cudaStream_t)stream;
-  const size_t smem = (size_t)(KMAX * 3 + KMAX * 3 * 256) * sizeof(float);
-  NM_CHECK_CUDA(cudaFuncSetAttribute(chamfer_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  chamfer_bwd_kernel<<<dim3(kChbBlocks, n), 256, smem, st>>>(seq, keypoints, K, G, linspace, reinterpret_cast<float*>(workspace));
+  float* ws = reinterpret_cast<float*>(workspace);
+  if (K <= kTunedK) {
+    const size_t smem = (size_t)(kTunedK * 3 + kTunedK * 3 * 256) * sizeof(float);
+    NM_CHECK_CUDA(cudaFuncSetAttribute(chamfer_bwd_kernel<kTunedK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    chamfer_bwd_kernel<kTunedK><<<dim3(kChbBlocks, n), 256, smem, st>>>(seq, keypoints, K, G, linspace, ws);
+  } else {
+    // 196 KB: one CTA per SM
+    const size_t smem = (size_t)(kMaxK * 3 + kMaxK * 3 * 256) * sizeof(float);
+    NM_CHECK_CUDA(cudaFuncSetAttribute(chamfer_bwd_kernel<kMaxK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    chamfer_bwd_kernel<kMaxK><<<dim3(kChbBlocks, n), 256, smem, st>>>(seq, keypoints, K, G, linspace, ws);
+  }
   NM_CHECK_LAUNCH("chamfer_bwd_kernel");
   chamfer_bwd_finalize_kernel<<<nm_cdiv((long long)n * K * 4, 128), 128, 0, st>>>(reinterpret_cast<const float*>(workspace), grad_out, n, K,
                                                                                  kChbBlocks, grad_keypoints);

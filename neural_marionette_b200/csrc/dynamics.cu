@@ -18,7 +18,16 @@ namespace {
 
 constexpr int kThreads = 256;
 constexpr int H = 512, Z = 128, HID = 128;
-constexpr int KP_MAX = 24;
+// Keypoint capacity of a kernel instantiation: K <= kTunedK (the shipped 24) runs the tuned kernels, 24 < K <= kMaxK a
+// set compiled for kMaxK.  Shared-memory rows sized by the capacity KC:
+template <int KC>
+struct KpDims {
+  static constexpr int K4 = 4 * KC;                  // flat pose (x, y, z, intensity) per keypoint
+  static constexpr int XW = 4 * KC + 128;            // GRU input: pose | z
+  static constexpr int JO = (3 + KC + 7) / 8 * 8;    // decoder row: root / intensity (3 + K) at 0, joint 6-D (6K) at JO
+  static constexpr int DW = JO + 6 * KC;
+};
+constexpr int kTunedK = 24, kMaxK = 64;
 constexpr int VC = 8;  // vectors per register chunk
 
 __device__ __forceinline__ float softplus_d(float x) { return x > 20.f ? x : log1pf(expf(x)); }
@@ -114,9 +123,10 @@ struct StepArgs {
   int B, K, S, posterior;
 };
 
-template <int NB>
+template <int NB, int KC>
 __global__ void __launch_bounds__(kThreads)
 hsvrnn_step_kernel(const StepArgs a) {
+  using D = KpDims<KC>;
   extern __shared__ float sm[];
   const int K = a.K, S = a.S, K4 = 4 * a.K;
   const int b0 = blockIdx.x * NB;
@@ -125,24 +135,24 @@ hsvrnn_step_kernel(const StepArgs a) {
   const int NVS = ((NB * S + VC - 1) / VC) * VC;  // padded
   constexpr int NBP = ((NB + VC - 1) / VC) * VC;
   // ---- shared-memory carve-up (floats)
-  float* s_in = sm;                         // [NBP][H + 96]  h | kp   (posterior MLP input)
+  float* s_in = sm;                         // [NBP][H + D::K4]  h | kp   (posterior MLP input)
   const int IN = H + K4;
-  float* s_hid = s_in + NBP * (H + 96);     // [NBP][HID]
+  float* s_hid = s_in + NBP * (H + D::K4);     // [NBP][HID]
   float* s_dist = s_hid + NBP * HID;        // [NBP][2Z]  mean | std (posterior, or prior in prior mode)
   float* s_z = s_dist + NBP * 2 * Z;        // [NVS][Z]
   float* s_ah = s_z + NVS * Z;              // [NBP][2 HID]  W0[:, :H] h + b0 for (root | joint) decoders
   float* s_h2 = s_ah + NBP * 2 * HID;       // [NVS][2 HID]
-  float* s_dec = s_h2 + NVS * 2 * HID;      // [NVS][176]  root(3+K) at 0, joint(6K) at 32
-  float* s_flat = s_dec + NVS * 176;        // [NVS][96]
-  float* s_rg = s_flat + NVS * 96;          // [NVS][K*9]
-  float* s_x = s_rg + NVS * KP_MAX * 9;     // [NBP][224]  GRU input
-  float* s_off = s_x + NBP * 224;           // [NB][K*3]
-  int* s_tree = reinterpret_cast<int*>(s_off + NB * KP_MAX * 3);  // order[K] | parents[K] | best[NB]
-  int* s_best = s_tree + 2 * KP_MAX;
+  float* s_dec = s_h2 + NVS * 2 * HID;      // [NVS][D::DW]  root(3+K) at 0, joint(6K) at JO
+  float* s_flat = s_dec + NVS * D::DW;      // [NVS][D::K4]
+  float* s_rg = s_flat + NVS * D::K4;          // [NVS][K*9]
+  float* s_x = s_rg + NVS * KC * 9;     // [NBP][D::XW]  GRU input
+  float* s_off = s_x + NBP * D::XW;           // [NB][K*3]
+  int* s_tree = reinterpret_cast<int*>(s_off + NB * KC * 3);  // order[K] | parents[K] | best[NB]
+  int* s_best = s_tree + 2 * KC;
 
   // ---- stage 0: load, zero the padding rows
-  for (int i = threadIdx.x; i < NBP * (H + 96); i += kThreads) {
-    const int v = i / (H + 96), j = i % (H + 96);
+  for (int i = threadIdx.x; i < NBP * (H + D::K4); i += kThreads) {
+    const int v = i / (H + D::K4), j = i % (H + D::K4);
     float val = 0.f;
     if (v < nb) {
       if (j < H) val = a.h_in[(long long)(b0 + v) * H + j];
@@ -152,17 +162,17 @@ hsvrnn_step_kernel(const StepArgs a) {
   }
   for (int i = threadIdx.x; i < NVS * Z; i += kThreads) s_z[i] = 0.f;
   for (int i = threadIdx.x; i < NBP * HID; i += kThreads) s_hid[i] = 0.f;
-  for (int i = threadIdx.x; i < NBP * 224; i += kThreads) s_x[i] = 0.f;
-  for (int i = threadIdx.x; i < nb * K * 3; i += kThreads) s_off[(i / (K * 3)) * KP_MAX * 3 + i % (K * 3)] = a.offset[(long long)b0 * K * 3 + i];
+  for (int i = threadIdx.x; i < NBP * D::XW; i += kThreads) s_x[i] = 0.f;
+  for (int i = threadIdx.x; i < nb * K * 3; i += kThreads) s_off[(i / (K * 3)) * KC * 3 + i % (K * 3)] = a.offset[(long long)b0 * K * 3 + i];
   for (int i = threadIdx.x; i < K; i += kThreads) {
     s_tree[i] = a.order[i];
-    s_tree[KP_MAX + i] = a.parents[i];
+    s_tree[KC + i] = a.parents[i];
   }
   __syncthreads();
 
   // ---- prior MLP (hsvrnn_bvh.py:92-96 / 210-214): 512 -> 128 -> 256
   if (a.prior_out || !a.posterior) {
-    cols_matvec(a.w.prior0_wt, HID, 0, HID, H, s_in, H + 96, nb, a.w.prior0_b, nullptr, 0, 1, 1, s_hid, HID);
+    cols_matvec(a.w.prior0_wt, HID, 0, HID, H, s_in, H + D::K4, nb, a.w.prior0_b, nullptr, 0, 1, 1, s_hid, HID);
     __syncthreads();
     cols_matvec(a.w.prior2_wt, 2 * Z, 0, 2 * Z, HID, s_hid, HID, nb, a.w.prior2_b, nullptr, 0, 1, 0, s_dist, 2 * Z);
     __syncthreads();
@@ -178,7 +188,7 @@ hsvrnn_step_kernel(const StepArgs a) {
   }
   // ---- posterior MLP (hsvrnn_bvh.py:99-104): (512 + 4K) -> 128 -> 256
   if (a.posterior) {
-    cols_matvec(a.w.post0_wt, HID, 0, HID, IN, s_in, H + 96, nb, a.w.post0_b, nullptr, 0, 1, 1, s_hid, HID);
+    cols_matvec(a.w.post0_wt, HID, 0, HID, IN, s_in, H + D::K4, nb, a.w.post0_b, nullptr, 0, 1, 1, s_hid, HID);
     __syncthreads();
     cols_matvec(a.w.post2_wt, 2 * Z, 0, 2 * Z, HID, s_hid, HID, nb, a.w.post2_b, nullptr, 0, 1, 0, s_dist, 2 * Z);
     __syncthreads();
@@ -197,22 +207,22 @@ hsvrnn_step_kernel(const StepArgs a) {
     s_z[vs * Z + j] = s_dist[v * 2 * Z + j] + s_dist[v * 2 * Z + Z + j] * e;
   }
   // ---- decoders, first layer split: W0 [h; z] = W0[:, :H] h (shared by the S samples) + W0[:, H:] z
-  cols_matvec(a.w.root0_wt, HID, 0, HID, H, s_in, H + 96, nb, a.w.root0_b, nullptr, 0, 1, 0, s_ah, 2 * HID);
-  cols_matvec(a.w.joint0_wt, HID, 0, HID, H, s_in, H + 96, nb, a.w.joint0_b, nullptr, 0, 1, 0, s_ah + HID, 2 * HID);
+  cols_matvec(a.w.root0_wt, HID, 0, HID, H, s_in, H + D::K4, nb, a.w.root0_b, nullptr, 0, 1, 0, s_ah, 2 * HID);
+  cols_matvec(a.w.joint0_wt, HID, 0, HID, H, s_in, H + D::K4, nb, a.w.joint0_b, nullptr, 0, 1, 0, s_ah + HID, 2 * HID);
   __syncthreads();
   cols_matvec(a.w.root0_wt + (long long)H * HID, HID, 0, HID, Z, s_z, Z, nvs, nullptr, s_ah, 2 * HID, S, 1, s_h2, 2 * HID);
   cols_matvec(a.w.joint0_wt + (long long)H * HID, HID, 0, HID, Z, s_z, Z, nvs, nullptr, s_ah + HID, 2 * HID, S, 1,
               s_h2 + HID, 2 * HID);
   __syncthreads();
   // second layers: root/intensity (3+K, tanh), joint (6K)
-  cols_matvec(a.w.root2_wt, 3 + K, 0, 3 + K, HID, s_h2, 2 * HID, nvs, a.w.root2_b, nullptr, 0, 1, 2, s_dec, 176);
-  cols_matvec(a.w.joint2_wt, 6 * K, 0, 6 * K, HID, s_h2 + HID, 2 * HID, nvs, a.w.joint2_b, nullptr, 0, 1, 0, s_dec + 32, 176);
+  cols_matvec(a.w.root2_wt, 3 + K, 0, 3 + K, HID, s_h2, 2 * HID, nvs, a.w.root2_b, nullptr, 0, 1, 2, s_dec, D::DW);
+  cols_matvec(a.w.joint2_wt, 6 * K, 0, 6 * K, HID, s_h2 + HID, 2 * HID, nvs, a.w.joint2_b, nullptr, 0, 1, 0, s_dec + D::JO, D::DW);
   __syncthreads();
   // ---- rotations + forward kinematics, one thread per (element, sample)
   if ((int)threadIdx.x < nvs) {
     const int vs = threadIdx.x, v = vs / S;
-    fk_pose(s_dec + vs * 176, s_dec + vs * 176 + 32, s_off + v * KP_MAX * 3, s_tree, s_tree + KP_MAX, K,
-            s_rg + vs * KP_MAX * 9, s_flat + vs * 96);
+    fk_pose(s_dec + vs * D::DW, s_dec + vs * D::DW + D::JO, s_off + v * KC * 3, s_tree, s_tree + KC, K,
+            s_rg + vs * KC * 9, s_flat + vs * D::K4);
   }
   __syncthreads();
   // ---- nearest sample to the detected keypoints (:116-123); prior mode: the single sample
@@ -224,7 +234,7 @@ hsvrnn_step_kernel(const StepArgs a) {
       for (int s = 0; s < S; s++) {
         float d = 0.f;
         for (int j = 0; j < K4; j++) {
-          const float t = s_in[v * (H + 96) + H + j] - s_flat[(v * S + s) * 96 + j];
+          const float t = s_in[v * (H + D::K4) + H + j] - s_flat[(v * S + s) * D::K4 + j];
           d += t * t;
         }
         if (d < bd) { bd = d; best = s; }
@@ -237,15 +247,15 @@ hsvrnn_step_kernel(const StepArgs a) {
   for (int i = threadIdx.x; i < nb * (K4 + Z); i += kThreads) {
     const int v = i / (K4 + Z), j = i % (K4 + Z);
     const int vs = v * S + s_best[v];
-    const float val = j < K4 ? s_flat[vs * 96 + j] : s_z[vs * Z + (j - K4)];
-    s_x[v * 224 + j] = val;
+    const float val = j < K4 ? s_flat[vs * D::K4 + j] : s_z[vs * Z + (j - K4)];
+    s_x[v * D::XW + j] = val;
     if (j < K4) a.kp_out[(long long)(b0 + v) * K4 + j] = val;
     else if (a.z_out) a.z_out[(long long)(b0 + v) * Z + (j - K4)] = val;
   }
   if (a.R_out)
     for (int i = threadIdx.x; i < nb * K * 9; i += kThreads) {
       const int v = i / (K * 9), j = i % (K * 9);
-      a.R_out[(long long)(b0 + v) * K * 9 + j] = s_rg[(v * S + s_best[v]) * KP_MAX * 9 + j];
+      a.R_out[(long long)(b0 + v) * K * 9 + j] = s_rg[(v * S + s_best[v]) * KC * 9 + j];
     }
   __syncthreads();
   // ---- GRU cell (gate order r, z, n); thread per hidden unit
@@ -262,7 +272,7 @@ hsvrnn_step_kernel(const StepArgs a) {
       const float w2 = __ldg(a.w.gru_ih_wt + (long long)i * 3 * H + 2 * H + j);
 #pragma unroll
       for (int v = 0; v < NB; v++) {
-        const float xv = s_x[v * 224 + i];
+        const float xv = s_x[v * D::XW + i];
         gi[0][v] = fmaf(w0, xv, gi[0][v]);
         gi[1][v] = fmaf(w1, xv, gi[1][v]);
         gi[2][v] = fmaf(w2, xv, gi[2][v]);
@@ -274,7 +284,7 @@ hsvrnn_step_kernel(const StepArgs a) {
       const float w2 = __ldg(a.w.gru_hh_wt + (long long)i * 3 * H + 2 * H + j);
 #pragma unroll
       for (int v = 0; v < NB; v++) {
-        const float hv = s_in[v * (H + 96) + i];
+        const float hv = s_in[v * (H + D::K4) + i];
         gh[0][v] = fmaf(w0, hv, gh[0][v]);
         gh[1][v] = fmaf(w1, hv, gh[1][v]);
         gh[2][v] = fmaf(w2, hv, gh[2][v]);
@@ -286,19 +296,20 @@ hsvrnn_step_kernel(const StepArgs a) {
         const float r = sigmoid_d(gi[0][v] + a.w.gru_ih_b[j] + gh[0][v] + a.w.gru_hh_b[j]);
         const float zg = sigmoid_d(gi[1][v] + a.w.gru_ih_b[H + j] + gh[1][v] + a.w.gru_hh_b[H + j]);
         const float ng = tanhf(gi[2][v] + a.w.gru_ih_b[2 * H + j] + r * (gh[2][v] + a.w.gru_hh_b[2 * H + j]));
-        a.h_out[(long long)(b0 + v) * H + j] = (1.0f - zg) * ng + zg * s_in[v * (H + 96) + j];
+        a.h_out[(long long)(b0 + v) * H + j] = (1.0f - zg) * ng + zg * s_in[v * (H + D::K4) + j];
       }
     }
   }
 }
 
-template <int NB>
+template <int NB, int KC>
 size_t step_smem_bytes(int S) {
+  using D = KpDims<KC>;
   const int NVS = ((NB * S + VC - 1) / VC) * VC;
   const int NBP = ((NB + VC - 1) / VC) * VC;
-  size_t f = (size_t)NBP * (H + 96) + NBP * HID + NBP * 2 * Z + (size_t)NVS * Z + NBP * 2 * HID + (size_t)NVS * 2 * HID +
-             (size_t)NVS * 176 + (size_t)NVS * 96 + (size_t)NVS * KP_MAX * 9 + NBP * 224 + NB * KP_MAX * 3;
-  return f * sizeof(float) + (2 * KP_MAX + NB + 8) * sizeof(int);
+  size_t f = (size_t)NBP * (H + D::K4) + NBP * HID + NBP * 2 * Z + (size_t)NVS * Z + NBP * 2 * HID + (size_t)NVS * 2 * HID +
+             (size_t)NVS * D::DW + (size_t)NVS * D::K4 + (size_t)NVS * KC * 9 + NBP * D::XW + NB * KC * 3;
+  return f * sizeof(float) + (2 * KC + NB + 8) * sizeof(int);
 }
 
 // ------------------------------------------------------------------ small batches: one thread-block cluster per element
@@ -373,13 +384,17 @@ __device__ __forceinline__ void quad_dot(const float* __restrict__ WT, int ldw, 
   }
 }
 
+// The cluster kernel serves K <= kTunedK only: its layout keeps both decoders' second layers resident, which at
+// kMaxK (231 KB for them alone) exceeds the 227 KB a CTA can have.  Larger K runs the per-element kernel.
+constexpr int kClK = kTunedK;
+using ClD = KpDims<kClK>;
 struct ClSmem {   // offsets in floats
   int in, hid, ah, gh, dist, part, z, h2, dec, flat, rl, rg, x, off, w2, tree, total;
 };
 __host__ __device__ inline ClSmem cl_layout(int SV) {
   ClSmem m;
   int o = 0;
-  m.in = o;   o += H + 96;
+  m.in = o;   o += H + ClD::K4;
   m.hid = o;  o += 2 * HID;                 // prior0 | post0 outputs
   m.ah = o;   o += 2 * HID;                 // root0 | joint0 applied to h (+ bias)
   m.gh = o;   o += 3 * kGruSlice;           // this rank's W_hh h (3 gates x 64 units)
@@ -387,14 +402,14 @@ __host__ __device__ inline ClSmem cl_layout(int SV) {
   m.part = o; o += 4 * SV * 256 > 1024 ? 4 * SV * 256 : 1024;
   m.z = o;    o += SV * Z;
   m.h2 = o;   o += SV * 2 * HID;
-  m.dec = o;  o += SV * 176;
-  m.flat = o; o += SV * 96;
-  m.rl = o;   o += SV * KP_MAX * 9;
-  m.rg = o;   o += SV * KP_MAX * 9;
-  m.x = o;    o += 224;
-  m.off = o;  o += KP_MAX * 3;
-  m.w2 = o;   o += HID * (3 + KP_MAX) + HID * 6 * KP_MAX;
-  m.tree = o; o += 2 * KP_MAX + 8;
+  m.dec = o;  o += SV * ClD::DW;
+  m.flat = o; o += SV * ClD::K4;
+  m.rl = o;   o += SV * kClK * 9;
+  m.rg = o;   o += SV * kClK * 9;
+  m.x = o;    o += ClD::XW;
+  m.off = o;  o += kClK * 3;
+  m.w2 = o;   o += HID * (3 + kClK) + HID * 6 * kClK;
+  m.tree = o; o += 2 * kClK + 8;
   m.total = o;
   return m;
 }
@@ -444,7 +459,7 @@ hsvrnn_step_cluster_kernel(const StepArgs a) {
     }
     asm volatile("cp.async.commit_group;" ::: "memory");
   }
-  for (int j = tid; j < H + 96; j += kThreads) {
+  for (int j = tid; j < H + ClD::K4; j += kThreads) {
     float val = 0.f;
     if (j < H) val = a.h_in[(long long)b * H + j];
     else if (a.posterior && j - H < K4) val = a.kp[(long long)b * K4 + (j - H)];
@@ -453,7 +468,7 @@ hsvrnn_step_cluster_kernel(const StepArgs a) {
   for (int i = tid; i < K * 3; i += kThreads) s_off[i] = a.offset[(long long)b * K * 3 + i];
   for (int i = tid; i < K; i += kThreads) {
     s_tree[i] = a.order[i];
-    s_tree[KP_MAX + i] = a.parents[i];
+    s_tree[kClK + i] = a.parents[i];
   }
   __syncthreads();
 
@@ -550,7 +565,7 @@ hsvrnn_step_cluster_kernel(const StepArgs a) {
   }
   asm volatile("cp.async.wait_all;" ::: "memory");
   __syncthreads();
-  // second layers from shared memory: root / intensity (3 + K, tanh) at s_dec[0..], joint 6-D rotations at s_dec[32..]
+  // second layers from shared memory: root / intensity (3 + K, tanh) at s_dec[0..], joint 6-D rotations at s_dec[JO..]
   for (int i = tid; i < S * (R2 + J2); i += kThreads) {
     const int v = i / (R2 + J2), c = i % (R2 + J2);
     float t;
@@ -558,30 +573,30 @@ hsvrnn_step_cluster_kernel(const StepArgs a) {
       t = a.w.root2_b[c];
       const float* hv = s_h2 + v * 2 * HID;
       for (int k = 0; k < HID; k++) t = fmaf(s_w2r[k * R2 + c], hv[k], t);
-      s_dec[v * 176 + c] = tanhf(t);
+      s_dec[v * ClD::DW + c] = tanhf(t);
     } else {
       const int cj = c - R2;
       t = a.w.joint2_b[cj];
       const float* hv = s_h2 + v * 2 * HID + HID;
       for (int k = 0; k < HID; k++) t = fmaf(s_w2j[k * J2 + cj], hv[k], t);
-      s_dec[v * 176 + 32 + cj] = t;
+      s_dec[v * ClD::DW + ClD::JO + cj] = t;
     }
   }
   __syncthreads();
   // rotations in parallel over (sample, joint), then the kinematic chain per sample
-  for (int i = tid; i < S * K; i += kThreads) rot6d(s_dec + (i / K) * 176 + 32 + (i % K) * 6, s_rl + (i / K) * KP_MAX * 9 + (i % K) * 9);
+  for (int i = tid; i < S * K; i += kThreads) rot6d(s_dec + (i / K) * ClD::DW + ClD::JO + (i % K) * 6, s_rl + (i / K) * kClK * 9 + (i % K) * 9);
   __syncthreads();
   if (tid < S) {
     const int v = tid;
-    const float* raw = s_dec + v * 176;
-    float* Rg = s_rg + v * KP_MAX * 9;
-    float* flat = s_flat + v * 96;
-    const float* Rl0 = s_rl + v * KP_MAX * 9;
+    const float* raw = s_dec + v * ClD::DW;
+    float* Rg = s_rg + v * kClK * 9;
+    float* flat = s_flat + v * ClD::K4;
+    const float* Rl0 = s_rl + v * kClK * 9;
     const int root = s_tree[0];
     for (int e = 0; e < 9; e++) Rg[root * 9 + e] = Rl0[root * 9 + e];
     flat[root * 4] = raw[0]; flat[root * 4 + 1] = raw[1]; flat[root * 4 + 2] = raw[2];
     for (int j = 1; j < K; j++) {
-      const int i = s_tree[j], pa = s_tree[KP_MAX + i];
+      const int i = s_tree[j], pa = s_tree[kClK + i];
       const float* Rl = Rl0 + i * 9;
       const float* Rp = Rg + pa * 9;
       float* Ri = Rg + i * 9;
@@ -603,20 +618,20 @@ hsvrnn_step_cluster_kernel(const StepArgs a) {
       for (int sidx = 0; sidx < S; sidx++) {
         float d = 0.f;
         for (int j = 0; j < K4; j++) {
-          const float t = s_in[H + j] - s_flat[sidx * 96 + j];
+          const float t = s_in[H + j] - s_flat[sidx * ClD::K4 + j];
           d += t * t;
         }
         if (d < bd) { bd = d; best = sidx; }
       }
     }
-    s_tree[2 * KP_MAX] = best;
+    s_tree[2 * kClK] = best;
     if (rank == 0 && a.pick_out) a.pick_out[b] = best;
   }
   __syncthreads();
-  const int best = s_tree[2 * KP_MAX];
-  for (int j = tid; j < 224; j += kThreads) {
+  const int best = s_tree[2 * kClK];
+  for (int j = tid; j < ClD::XW; j += kThreads) {
     float val = 0.f;
-    if (j < K4) val = s_flat[best * 96 + j];
+    if (j < K4) val = s_flat[best * ClD::K4 + j];
     else if (j < K4 + Z) val = s_z[best * Z + (j - K4)];
     s_x[j] = val;
     if (rank == 0) {
@@ -625,7 +640,7 @@ hsvrnn_step_cluster_kernel(const StepArgs a) {
     }
   }
   if (rank == 0 && a.R_out)
-    for (int j = tid; j < K * 9; j += kThreads) a.R_out[(long long)b * K * 9 + j] = s_rg[best * KP_MAX * 9 + j];
+    for (int j = tid; j < K * 9; j += kThreads) a.R_out[(long long)b * K * 9 + j] = s_rg[best * kClK * 9 + j];
   __syncthreads();
   // ---- GRU: this rank's 64 hidden units; input half W_ih x: 192 columns = 48 quads x 4 input slices
   {
@@ -658,28 +673,29 @@ hsvrnn_step_cluster_kernel(const StepArgs a) {
 
 // Pose decoding on its own (extract_kypt_from_latent_and_state, hsvrnn_bvh.py:255-286) for callers that
 // drive the sub-modules by hand (vis_generation.py:108-113).
+template <int KC>
 __global__ void __launch_bounds__(kThreads)
 decode_pose_kernel(nm_hsvrnn_weights w, const float* __restrict__ dec_in /* (B, H+Z) */,
                    const float* __restrict__ offset, const int* __restrict__ order, const int* __restrict__ parents,
                    int B, int K, float* __restrict__ flat_out, float* __restrict__ R_out) {
   __shared__ float s_in[VC * (H + Z)];
   __shared__ float s_hid[VC * 2 * HID];
-  __shared__ float s_dec[176];
-  __shared__ float s_rg[KP_MAX * 9];
-  __shared__ float s_flat[96];
-  __shared__ int s_tree[2 * KP_MAX];
+  __shared__ float s_dec[KpDims<KC>::DW];
+  __shared__ float s_rg[KC * 9];
+  __shared__ float s_flat[KpDims<KC>::K4];
+  __shared__ int s_tree[2 * KC];
   const int b = blockIdx.x;
   for (int i = threadIdx.x; i < VC * (H + Z); i += kThreads) s_in[i] = i < H + Z ? dec_in[(long long)b * (H + Z) + i] : 0.f;
-  for (int i = threadIdx.x; i < K; i += kThreads) { s_tree[i] = order[i]; s_tree[KP_MAX + i] = parents[i]; }
+  for (int i = threadIdx.x; i < K; i += kThreads) { s_tree[i] = order[i]; s_tree[KC + i] = parents[i]; }
   __syncthreads();
   cols_matvec(w.root0_wt, HID, 0, HID, H + Z, s_in, H + Z, 1, w.root0_b, nullptr, 0, 1, 1, s_hid, 2 * HID);
   cols_matvec(w.joint0_wt, HID, 0, HID, H + Z, s_in, H + Z, 1, w.joint0_b, nullptr, 0, 1, 1, s_hid + HID, 2 * HID);
   __syncthreads();
-  cols_matvec(w.root2_wt, 3 + K, 0, 3 + K, HID, s_hid, 2 * HID, 1, w.root2_b, nullptr, 0, 1, 2, s_dec, 176);
-  cols_matvec(w.joint2_wt, 6 * K, 0, 6 * K, HID, s_hid + HID, 2 * HID, 1, w.joint2_b, nullptr, 0, 1, 0, s_dec + 32, 176);
+  cols_matvec(w.root2_wt, 3 + K, 0, 3 + K, HID, s_hid, 2 * HID, 1, w.root2_b, nullptr, 0, 1, 2, s_dec, KpDims<KC>::DW);
+  cols_matvec(w.joint2_wt, 6 * K, 0, 6 * K, HID, s_hid + HID, 2 * HID, 1, w.joint2_b, nullptr, 0, 1, 0, s_dec + KpDims<KC>::JO, KpDims<KC>::DW);
   __syncthreads();
   if (threadIdx.x == 0)
-    fk_pose(s_dec, s_dec + 32, offset + (long long)b * K * 3, s_tree, s_tree + KP_MAX, K, s_rg, s_flat);
+    fk_pose(s_dec, s_dec + KpDims<KC>::JO, offset + (long long)b * K * 3, s_tree, s_tree + KC, K, s_rg, s_flat);
   __syncthreads();
   for (int i = threadIdx.x; i < 4 * K; i += kThreads) flat_out[(long long)b * 4 * K + i] = s_flat[i];
   if (R_out)
@@ -716,13 +732,30 @@ __global__ void bone_offset_kernel(const float* __restrict__ kp /* (B,T,K,4) */,
 
 }  // namespace
 
+// one CTA per NB elements; NB = 4 only for batches that fill the GPU four times over and when its layout fits
+// (at kMaxK it does for S = 1, not for S = 10: 22 KB + 4 S x 6.8 KB)
+template <int KC>
+static int launch_step(const StepArgs& a, cudaStream_t st) {
+  if (a.B >= 4 * nm_num_sms() && step_smem_bytes<4, KC>(a.S) <= 227 * 1024) {
+    const size_t smem = step_smem_bytes<4, KC>(a.S);
+    NM_CHECK_CUDA(cudaFuncSetAttribute(hsvrnn_step_kernel<4, KC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    hsvrnn_step_kernel<4, KC><<<nm_cdiv(a.B, 4), kThreads, smem, st>>>(a);
+  } else {
+    const size_t smem = step_smem_bytes<1, KC>(a.S);
+    NM_CHECK_CUDA(cudaFuncSetAttribute(hsvrnn_step_kernel<1, KC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    hsvrnn_step_kernel<1, KC><<<a.B, kThreads, smem, st>>>(a);
+  }
+  NM_CHECK_LAUNCH("hsvrnn_step");
+  return NM_OK;
+}
+
 static int hsvrnn_step_impl(const nm_hsvrnn_weights* w, const float* h_in, const float* kp, const float* eps,
                             const float* offset, const int* order, const int* parents, int B, int K, int S, int posterior,
                             float* h_out, float* kp_out, float* z_out, float* R_out, float* post_out, float* prior_out,
                             int* pick_out, void* stream) {
   NM_CHECK_ARG(w && h_in && eps && offset && order && parents && h_out && kp_out, "nm_hsvrnn_step: null pointer");
   NM_CHECK_ARG(!posterior || kp, "nm_hsvrnn_step: posterior step needs detected keypoints");
-  NM_CHECK_ARG(K > 0 && K <= KP_MAX && S >= 1 && S <= 16, "nm_hsvrnn_step: K=%d S=%d unsupported", K, S);
+  NM_CHECK_ARG(K > 0 && K <= kMaxK && S >= 1 && S <= 16, "nm_hsvrnn_step: K=%d S=%d unsupported", K, S);
   NM_CHECK_ARG(posterior || S == 1, "nm_hsvrnn_step: prior step draws one sample");
   if (B == 0) return NM_OK;
   StepArgs a;
@@ -733,7 +766,7 @@ static int hsvrnn_step_impl(const nm_hsvrnn_weights* w, const float* h_in, const
   cudaStream_t st = (cudaStream_t)stream;
   // small and medium batches: a cluster of 8 CTAs per element (weights split over the ranks, DSMEM broadcasts)
   // measured, cluster vs one-CTA-per-element kernel (us per step): B = 1: 30 vs 216, B = 16: 59 vs 228, B = 64: 144 vs 235, B = 256: 510 vs 240
-  if (S <= 10 && B <= 96) {
+  if (K <= kClK && S <= 10 && B <= 96) {
     const int SV = S == 1 ? 1 : 10;
     const size_t smem = (size_t)cl_layout(SV).total * sizeof(float);
     if (SV == 1) {
@@ -746,17 +779,8 @@ static int hsvrnn_step_impl(const nm_hsvrnn_weights* w, const float* h_in, const
     NM_CHECK_LAUNCH("hsvrnn_step(cluster)");
     return NM_OK;
   }
-  if (B >= 4 * nm_num_sms() && step_smem_bytes<4>(S) <= 227 * 1024) {
-    const size_t smem = step_smem_bytes<4>(S);
-    NM_CHECK_CUDA(cudaFuncSetAttribute(hsvrnn_step_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    hsvrnn_step_kernel<4><<<nm_cdiv(B, 4), kThreads, smem, st>>>(a);
-  } else {
-    const size_t smem = step_smem_bytes<1>(S);
-    NM_CHECK_CUDA(cudaFuncSetAttribute(hsvrnn_step_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    hsvrnn_step_kernel<1><<<B, kThreads, smem, st>>>(a);
-  }
-  NM_CHECK_LAUNCH("hsvrnn_step");
-  return NM_OK;
+  if (K <= kTunedK) return launch_step<kTunedK>(a, st);
+  return launch_step<kMaxK>(a, st);
 }
 
 extern "C" int nm_hsvrnn_step(const nm_hsvrnn_weights* w, const float* h_in, const float* kp, const float* eps,
@@ -779,9 +803,12 @@ extern "C" int nm_hsvrnn_decode_pose(const nm_hsvrnn_weights* w, const float* de
                                      const int* order, const int* parents, int B, int K, float* flat_out,
                                      float* R_out, void* stream) {
   NM_CHECK_ARG(w && dec_in && offset && order && parents && flat_out, "nm_hsvrnn_decode_pose: null pointer");
-  NM_CHECK_ARG(K > 0 && K <= KP_MAX, "nm_hsvrnn_decode_pose: K=%d unsupported", K);
+  NM_CHECK_ARG(K > 0 && K <= kMaxK, "nm_hsvrnn_decode_pose: K=%d unsupported", K);
   if (B == 0) return NM_OK;
-  decode_pose_kernel<<<B, kThreads, 0, (cudaStream_t)stream>>>(*w, dec_in, offset, order, parents, B, K, flat_out, R_out);
+  if (K <= kTunedK)
+    decode_pose_kernel<kTunedK><<<B, kThreads, 0, (cudaStream_t)stream>>>(*w, dec_in, offset, order, parents, B, K, flat_out, R_out);
+  else
+    decode_pose_kernel<kMaxK><<<B, kThreads, 0, (cudaStream_t)stream>>>(*w, dec_in, offset, order, parents, B, K, flat_out, R_out);
   NM_CHECK_LAUNCH("hsvrnn_decode_pose");
   return NM_OK;
 }
@@ -807,16 +834,18 @@ extern "C" int nm_hsvrnn_bone_offsets(const float* keypoints, const int* parents
 // [out][in] layout: both are coalesced along the output columns.  Every reduction runs in a fixed order.
 namespace {
 
-// Per-(t, b) row record (floats): forward recomputes, then every d pre-activation the weight gradients need.
+// Per-(t, b) row record (floats): forward recomputes, then every d pre-activation the weight gradients need.  One layout
+// at capacity kMaxK serves every K: nm_hsvrnn_backward_workspace_bytes does not take K.
+using RD = KpDims<kMaxK>;
 enum : int {
   RW_AP = 0, RW_AQ = RW_AP + HID, RW_AR = RW_AQ + HID, RW_AJ = RW_AR + HID,       // first-layer pre-activations
   RW_GI = RW_AJ + HID, RW_GH = RW_GI + 3 * H,                                      // W_ih x + b_ih, W_hh h + b_hh
   RW_OP = RW_GH + 3 * H, RW_OQ = RW_OP + 2 * Z,                                    // prior / posterior raw outputs
-  RW_OR = RW_OQ + 2 * Z, RW_OJ = RW_OR + 32,                                       // tanh(root) (3+K), joint 6-D (6K)
-  RW_DGI = RW_OJ + 6 * KP_MAX, RW_DGH = RW_DGI + 3 * H,                            // d gates (input / hidden side)
-  RW_DXG = RW_DGH + 3 * H, RW_DH1 = RW_DXG + 4 * KP_MAX + Z,                       // W_ih^T dgi (then df | dz), W_hh^T dgh
-  RW_DOR = RW_DH1 + H, RW_DOJ = RW_DOR + 32,                                       // d pre-tanh root, d joint 6-D
-  RW_DAR = RW_DOJ + 6 * KP_MAX, RW_DAJ = RW_DAR + HID,                             // d first-layer pre-activations
+  RW_OR = RW_OQ + 2 * Z, RW_OJ = RW_OR + RD::JO,                                   // tanh(root) (3+K), joint 6-D (6K)
+  RW_DGI = RW_OJ + 6 * kMaxK, RW_DGH = RW_DGI + 3 * H,                             // d gates (input / hidden side)
+  RW_DXG = RW_DGH + 3 * H, RW_DH1 = RW_DXG + RD::XW,                               // W_ih^T dgi (then df | dz), W_hh^T dgh
+  RW_DOR = RW_DH1 + H, RW_DOJ = RW_DOR + RD::JO,                                   // d pre-tanh root, d joint 6-D
+  RW_DAR = RW_DOJ + 6 * kMaxK, RW_DAJ = RW_DAR + HID,                              // d first-layer pre-activations
   RW_DXDR = RW_DAJ + HID, RW_DXDJ = RW_DXDR + H + Z,                               // W0^T da of the decoders ([h | z])
   RW_DOP = RW_DXDJ + H + Z, RW_DOQ = RW_DOP + 2 * Z,                               // d prior / posterior raw outputs
   RW_DAP = RW_DOQ + 2 * Z, RW_DAQ = RW_DAP + HID,
@@ -965,11 +994,12 @@ __device__ void rot6d_bwd(const float* p, const float* dR, float* dp) {
 
 // Pose backward of the picked decode: forward kinematics down `order` in reverse, then the 6-D rotations and the tanh.
 // df = W_ih^T dgi [:4K] + external d kypt_recon; dR external d R; accumulates d offset.  One CTA of 64 threads per element.
+template <int KC>
 __global__ void __launch_bounds__(64)
 pose_bwd_kernel(const float* __restrict__ Rg_all /* (B, K, 9) */, const float* __restrict__ offset, const int* __restrict__ order,
                 const int* __restrict__ parents, const float* __restrict__ df_ext, const float* __restrict__ dR_ext,
                 const float* __restrict__ dz_ext, int K, float* __restrict__ doffset, float* __restrict__ rows) {
-  __shared__ float s_rl[KP_MAX * 9], s_drg[KP_MAX * 9], s_dpos[KP_MAX * 3], s_doff[KP_MAX * 3], s_dint[KP_MAX];
+  __shared__ float s_rl[KC * 9], s_drg[KC * 9], s_dpos[KC * 3], s_doff[KC * 3], s_dint[KC];
   const int b = blockIdx.x, K4 = 4 * K;
   float* rec = rows + (long long)b * RW;
   const float* Rg = Rg_all + (long long)b * K * 9;
@@ -1185,7 +1215,7 @@ extern "C" int nm_hsvrnn_step_backward(const nm_hsvrnn_weights* wt, const nm_hsv
                                        float* dh_out, float* doffset, float* rows, void* stream) {
   NM_CHECK_ARG(wt && w && h && kp && eps && pick && f && z && R && offset && order && parents && dh_next && dh_out &&
                    doffset && rows, "nm_hsvrnn_step_backward: null pointer");
-  NM_CHECK_ARG(K > 0 && K <= KP_MAX && S >= 1 && S <= 16, "nm_hsvrnn_step_backward: K=%d S=%d unsupported", K, S);
+  NM_CHECK_ARG(K > 0 && K <= kMaxK && S >= 1 && S <= 16, "nm_hsvrnn_step_backward: K=%d S=%d unsupported", K, S);
   if (B == 0) return NM_OK;
   (void)S;
   cudaStream_t st = (cudaStream_t)stream;
@@ -1221,7 +1251,8 @@ extern "C" int nm_hsvrnn_step_backward(const nm_hsvrnn_weights* wt, const nm_hsv
   js.j[1] = gemm_job(rows + RW_DGH, RW, 3 * H, nullptr, 0, 3 * H, w->gru_hh_wt, H, H, rows + RW_DH1, RW);
   if (int rc = launch_gemm(js, 2, B, st)) return rc;
   // 4. forward kinematics, 6-D rotations, tanh
-  pose_bwd_kernel<<<B, 64, 0, st>>>(R, offset, order, parents, df, dR, dz, K, doffset, rows);
+  if (K <= kTunedK) pose_bwd_kernel<kTunedK><<<B, 64, 0, st>>>(R, offset, order, parents, df, dR, dz, K, doffset, rows);
+  else pose_bwd_kernel<kMaxK><<<B, 64, 0, st>>>(R, offset, order, parents, df, dR, dz, K, doffset, rows);
   NM_CHECK_LAUNCH("hsvrnn_step_backward(pose)");
   // 5. decoders: second layers (times LeakyReLU' of the first), then the first layers' [h | z] parts
   js.j[0] = gemm_job(rows + RW_DOR, RW, R2, nullptr, 0, R2, w->root2_wt, HID, HID, rows + RW_DAR, RW);
@@ -1254,7 +1285,7 @@ extern "C" int nm_hsvrnn_weight_grads(const float* rows, const float* h, const f
                                       const float* offset_param, int B, int T, int K, const nm_hsvrnn_grads* g,
                                       void* stream) {
   NM_CHECK_ARG(rows && h && kp && f && z && dh0 && g, "nm_hsvrnn_weight_grads: null pointer");
-  NM_CHECK_ARG(K > 0 && K <= KP_MAX && T >= 1, "nm_hsvrnn_weight_grads: K=%d T=%d unsupported", K, T);
+  NM_CHECK_ARG(K > 0 && K <= kMaxK && T >= 1, "nm_hsvrnn_weight_grads: K=%d T=%d unsupported", K, T);
   NM_CHECK_ARG(!g->offset_param || (offset && doffset && offset_param), "nm_hsvrnn_weight_grads: offset_param needs offsets");
   if (B == 0) return NM_OK;
   const int K4 = 4 * K, R = T * B;

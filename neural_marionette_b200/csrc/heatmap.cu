@@ -15,7 +15,9 @@
 
 namespace {
 
-constexpr int KMAX = 24;   // keypoints (compile-time upper bound for register arrays)
+// Keypoint capacity of a kernel instantiation (compile-time bound of register and shared arrays).  K <= 24 (the shipped
+// configuration) runs the kTunedK instantiations; 24 < K <= kMaxK runs a second set compiled for kMaxK.
+constexpr int kTunedK = 24, kMaxK = 64;
 
 __device__ __forceinline__ float softplus1(float x) {
   // nn.Softplus(beta=1, threshold=20)
@@ -23,8 +25,8 @@ __device__ __forceinline__ float softplus1(float x) {
 }
 
 // Phase 1 (parallel over voxels): heat-map values on mma.sync (m16n8k16, fp16 operands, fp32 accumulate).
-// grid = (g^3 / 512, n); a warp owns M-tiles of 16 consecutive voxels, K = C feature channels, N = 24 keypoints (3
-// n-blocks).  The K order is permuted so that the 8 consecutive channels a lane loads with one 16-byte load are the
+// grid = (g^3 / 512, n); a warp owns M-tiles of 16 consecutive voxels, K = C feature channels, N = the keypoint capacity
+// (NB n-blocks).  The K order is permuted so that the 8 consecutive channels a lane loads with one 16-byte load are the
 // K slots it owns in two k-steps (as in conv_pw.cu); the 1x1 conv weights are packed into B fragments once per block.
 //   mode 0: heat = lrelu(w1 f + b1);  mode 1: heat = softplus(pw0 * lrelu(w1 f + b1) + pw1 * prev[clip] + pb)
 __device__ __forceinline__ void head_mma(float (&c)[4], const uint32_t a0, const uint32_t a1, const uint32_t a2,
@@ -34,17 +36,26 @@ __device__ __forceinline__ void head_mma(float (&c)[4], const uint32_t a0, const
                : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b.x), "r"(b.y));
 }
 
-template <int C>
+// NB: n-blocks of 8 keypoints (3 for K <= 24, 8 for K <= 64).  The 3-block fragments fit in static shared memory; the
+// 8-block ones (64 KB at C = 256) are dynamic (smem bytes = head_frag_bytes<C, 8>()).
+template <int C, int NB>
+constexpr int head_frag_bytes() { return 2 * (C / 16) * NB * 32 * (int)sizeof(uint2); }
+
+template <int C, int NB>
 __global__ void __launch_bounds__(256)
 head_heat_kernel(const act_t* __restrict__ feature, const float* __restrict__ w1, const float* __restrict__ b1,
                  int K, int S, int mode, const float* __restrict__ prev, int frames_per_clip, float pw0, float pw1,
                  float pb, const float* __restrict__ prop_dev, float* __restrict__ heat) {
   if (prop_dev) { pw0 = __ldg(prop_dev); pw1 = __ldg(prop_dev + 1); pb = __ldg(prop_dev + 2); }   // live parameters
-  constexpr int KS = C / 16, NB = KMAX / 8;
+  constexpr int KS = C / 16, KC = NB * 8;
+  constexpr bool kStatic = KC <= kTunedK;
   // the fp32 weights are split into fp16 hi + lo parts (two MMAs per k-step): the heat-maps keep fp32-weight accuracy
-  __shared__ __align__(16) uint2 s_frag[KS * NB * 32];
-  __shared__ __align__(16) uint2 s_frag_lo[KS * NB * 32];
-  __shared__ float s_b[KMAX];
+  __shared__ __align__(16) uint2 s_frag_st[kStatic ? KS * NB * 32 : 1];
+  __shared__ __align__(16) uint2 s_frag_lo_st[kStatic ? KS * NB * 32 : 1];
+  extern __shared__ __align__(16) uint2 s_frag_dyn[];
+  uint2* s_frag = kStatic ? s_frag_st : s_frag_dyn;
+  uint2* s_frag_lo = kStatic ? s_frag_lo_st : s_frag_dyn + KS * NB * 32;
+  __shared__ float s_b[KC];
   const int n = blockIdx.y;
   // k-step ks = 2m + s of the 32-channel group m: slot (2t + j + 8 hi) <-> channel m*32 + t*8 + s*4 + hi*2 + j
   for (int i = threadIdx.x; i < KS * NB * 32; i += 256) {
@@ -62,7 +73,7 @@ head_heat_kernel(const act_t* __restrict__ feature, const float* __restrict__ w1
     __half2 l0 = __floats2half2_rn(v[0] - f0.x, v[1] - f0.y), l1 = __floats2half2_rn(v[2] - f1.x, v[3] - f1.y);
     s_frag_lo[i] = make_uint2(*reinterpret_cast<uint32_t*>(&l0), *reinterpret_cast<uint32_t*>(&l1));
   }
-  for (int i = threadIdx.x; i < KMAX; i += 256) s_b[i] = i < K ? b1[i] : 0.f;
+  for (int i = threadIdx.x; i < KC; i += 256) s_b[i] = i < K ? b1[i] : 0.f;
   __syncthreads();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
   const float* pv = prev ? prev + (long long)(n / frames_per_clip) * K * S : nullptr;
@@ -109,6 +120,7 @@ head_heat_kernel(const act_t* __restrict__ feature, const float* __restrict__ w1
 // heat: (n, K, g^3) fp32 written by head_heat_kernel, g in {8, 16, 32}.  Per keypoint a thread reads z rows of g
 // floats (16-byte loads): the row sum feeds the x and y marginals, the row itself is accumulated into per-thread z
 // partials that are folded through shared memory in a fixed order.  No float atomics: bit-reproducible run to run.
+template <int KMAX>
 __global__ void __launch_bounds__(256)
 head_reduce_kernel(int K, int g, const float* __restrict__ lin, float gauss_width, const float* __restrict__ heat,
                    float* __restrict__ keypoints, float* __restrict__ gaussians, float* __restrict__ heat_mean) {
@@ -221,6 +233,7 @@ head_reduce_kernel(int K, int g, const float* __restrict__ lin, float gauss_widt
 }
 
 // Standalone render for decode_from_dyna (model/kypt_detector.py:213-231): keypoints (n,K,4) -> (n,K,g^3)
+template <int KMAX>
 __global__ void __launch_bounds__(256)
 gaussian_render_kernel(const float* __restrict__ keypoints, int K, int g, const float* __restrict__ lin,
                        float gauss_width, float* __restrict__ gaussians) {
@@ -263,16 +276,20 @@ gaussian_render_kernel(const float* __restrict__ keypoints, int K, int g, const 
 // (16-byte base loads / stores, 8-byte fp16 stores).  The Gaussian operand is evaluated straight into the A fragment
 // from the separable exp tables.  coords and bias stay fp32 (CUDA cores).
 constexpr int kAdjCO = 128, kAdjFD = 128, kAdjNB = kAdjCO / 8;
-constexpr int kAdjFragG = 2 * kAdjNB * 32;                 // uint2 per Gaussian weight block (K <= 32: 2 k-steps)
+// uint2 per Gaussian weight block: one k-step per 16 keypoints of the capacity (2 for kTunedK, 4 for kMaxK)
+template <int KMAX>
+constexpr int adj_frag_g() { return (KMAX + 15) / 16 * kAdjNB * 32; }
 constexpr int kAdjFragFF = (kAdjFD / 16) * kAdjNB * 32;    // first-feature block (8 k-steps)
 
 // output channel of fragment column c (0..7) of n-block nb
 __host__ __device__ inline int adj_channel(int nb, int c) { return (nb >> 1) * 16 + (c >> 1) * 4 + (nb & 1) * 2 + (c & 1); }
 
-// frags: [gauss_t (2 k-steps)][gauss_0 (2)][first_feature (8)] x [16 n-blocks][32 lanes]; xyzb[co] = (Wx, Wy, Wz, bias)
+// frags: [gauss_t (GS k-steps)][gauss_0 (GS)][first_feature (8)] x [16 n-blocks][32 lanes]; xyzb[co] = (Wx, Wy, Wz, bias)
+template <int KMAX>
 __global__ void adjust_pack_kernel(const float* __restrict__ w, const float* __restrict__ bias, int K, int ld,
                                    uint2* __restrict__ frags, float4* __restrict__ xyzb) {
-  const int total = 2 * kAdjFragG + kAdjFragFF;
+  constexpr int GS = (KMAX + 15) / 16;
+  const int total = 2 * adj_frag_g<KMAX>() + kAdjFragFF;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
     const int lane = i & 31, g = lane >> 2, t = lane & 3;
     int rest = i >> 5;
@@ -284,12 +301,12 @@ __global__ void adjust_pack_kernel(const float* __restrict__ w, const float* __r
       const int j = e & 1, hi = e >> 1;
       int col;
       bool ok = true;
-      if (rest < 4) {                                      // Gaussian blocks: k = s*16 + 2t + j + 8*hi
-        const int k = (rest & 1) * 16 + 2 * t + j + 8 * hi;
+      if (rest < 2 * GS) {                                 // Gaussian blocks: k = s*16 + 2t + j + 8*hi
+        const int k = (rest & (GS - 1)) * 16 + 2 * t + j + 8 * hi;
         ok = k < K;
-        col = (rest < 2 ? 0 : K + kAdjFD) + k;
+        col = (rest < GS ? 0 : K + kAdjFD) + k;
       } else {                                             // first feature: ci = m*32 + t*8 + s*4 + hi*2 + j
-        const int ks = rest - 4, m = ks >> 1, sst = ks & 1;
+        const int ks = rest - 2 * GS, m = ks >> 1, sst = ks & 1;
         col = K + m * 32 + t * 8 + sst * 4 + hi * 2 + j;
       }
       v[e] = ok ? w[(long long)co * ld + col] : 0.f;
@@ -310,18 +327,19 @@ __device__ __forceinline__ void adj_mma(float (&c)[4], const uint32_t a0, const 
                : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b.x), "r"(b.y));
 }
 
-// Gaussian A fragments (2 k-steps) of one M-tile: rows r0 / r1 are voxels s0 / s1 of frame `gn`
+// Gaussian A fragments (GS k-steps) of one M-tile: rows r0 / r1 are voxels s0 / s1 of frame `gn`
 struct GaussSrc {
   const float* s_e;     // [K][3][32] separable exps (keypoint mode)
   const float* s_i;     // [K] intensities
   const float* gs;      // gaussians tensor of this frame (K, S) or null
   int K, g, S;
 };
-__device__ __forceinline__ void gauss_frags(const GaussSrc& q, int s0, int s1, int t, uint32_t (&a)[2][4]) {
+template <int GS>
+__device__ __forceinline__ void gauss_frags(const GaussSrc& q, int s0, int s1, int t, uint32_t (&a)[GS][4]) {
   const int z0 = s0 % q.g, y0 = (s0 / q.g) % q.g, x0 = s0 / (q.g * q.g);
   const int z1 = s1 % q.g, y1 = (s1 / q.g) % q.g, x1 = s1 / (q.g * q.g);
 #pragma unroll
-  for (int st = 0; st < 2; st++)
+  for (int st = 0; st < GS; st++)
 #pragma unroll
     for (int hi = 0; hi < 2; hi++) {
       float v[2][2];
@@ -358,6 +376,7 @@ __device__ __forceinline__ void stage_exps(const float* kp /* (K,4) of one frame
 }
 
 // base[clip][s][co] (fp32): one block = 128 voxels of one clip, one M-tile per warp
+template <int KMAX>
 __global__ void __launch_bounds__(256)
 adjust_base_kernel(const act_t* __restrict__ ff /* (clips, S, 128) */, const float* __restrict__ kp /* (n,K,4) */,
                    const float* __restrict__ gs /* optional (n,K,S) */, int frames_per_clip,
@@ -368,7 +387,7 @@ adjust_base_kernel(const act_t* __restrict__ ff /* (clips, S, 128) */, const flo
   __shared__ float s_i[KMAX];
   const int clip = blockIdx.y;
   const int S = g * g * g;
-  for (int i = threadIdx.x; i < kAdjFragG + kAdjFragFF; i += 256) s_frag[i] = __ldg(frags + kAdjFragG + i);
+  for (int i = threadIdx.x; i < adj_frag_g<KMAX>() + kAdjFragFF; i += 256) s_frag[i] = __ldg(frags + adj_frag_g<KMAX>() + i);
   // gauss_0 = the gaussians of the clip's first frame (kypt_detector.py:406: gaussians[:, 0])
   if (!gs) stage_exps(kp + (long long)clip * frames_per_clip * K * 4, K, g, lin, gauss_width, s_e, s_i);
   __syncthreads();
@@ -390,10 +409,11 @@ adjust_base_kernel(const act_t* __restrict__ ff /* (clips, S, 128) */, const flo
       }
   }
   GaussSrc q{s_e, s_i, gs ? gs + (long long)clip * frames_per_clip * K * S : nullptr, K, g, S};
-  uint32_t a[2][4];
-  gauss_frags(q, s0, s1, t, a);
+  constexpr int GS = (KMAX + 15) / 16;
+  uint32_t a[GS][4];
+  gauss_frags<GS>(q, s0, s1, t, a);
 #pragma unroll
-  for (int st = 0; st < 2; st++)
+  for (int st = 0; st < GS; st++)
 #pragma unroll
     for (int nb = 0; nb < kAdjNB; nb++) adj_mma(c[nb], a[st][0], a[st][1], a[st][2], a[st][3], s_frag[(st * kAdjNB + nb) * 32 + lane]);
   const uint4* f0 = reinterpret_cast<const uint4*>(ff + ((long long)clip * S + s0) * kAdjFD + t * 8);
@@ -401,7 +421,7 @@ adjust_base_kernel(const act_t* __restrict__ ff /* (clips, S, 128) */, const flo
 #pragma unroll
   for (int m = 0; m < kAdjFD / 32; m++) {
     const uint4 r0 = __ldg(f0 + m * 4), r1 = __ldg(f1 + m * 4);
-    const uint2* fr = s_frag + kAdjFragG + (2 * m) * kAdjNB * 32 + lane;
+    const uint2* fr = s_frag + adj_frag_g<KMAX>() + (2 * m) * kAdjNB * 32 + lane;
 #pragma unroll
     for (int nb = 0; nb < kAdjNB; nb++) {
       adj_mma(c[nb], r0.x, r1.x, r0.y, r1.y, fr[nb * 32]);
@@ -417,17 +437,18 @@ adjust_base_kernel(const act_t* __restrict__ ff /* (clips, S, 128) */, const flo
 }
 
 // out[frame][s][co] = lrelu(base[clip][s][co] + W[:, :K] gauss_t[frame][s]); one block = TILES*128 voxels of a frame
+template <int KMAX>
 __global__ void __launch_bounds__(256)
 adjust_frame_kernel(const float* __restrict__ base, const float* __restrict__ kp /* (n,K,4) */,
                     const float* __restrict__ gs /* optional (n,K,S) */, const uint2* __restrict__ frags, int K, int g,
                     int frames_per_clip, int tiles_per_warp, const float* __restrict__ lin, float gauss_width,
                     act_t* __restrict__ out) {
-  __shared__ __align__(16) uint2 s_frag[kAdjFragG];
+  __shared__ __align__(16) uint2 s_frag[adj_frag_g<KMAX>()];
   __shared__ float s_e[KMAX * 3 * 32];
   __shared__ float s_i[KMAX];
   const int n = blockIdx.y, clip = n / frames_per_clip;
   const int S = g * g * g;
-  for (int i = threadIdx.x; i < kAdjFragG; i += 256) s_frag[i] = __ldg(frags + i);
+  for (int i = threadIdx.x; i < adj_frag_g<KMAX>(); i += 256) s_frag[i] = __ldg(frags + i);
   if (!gs) stage_exps(kp + (long long)n * K * 4, K, g, lin, gauss_width, s_e, s_i);
   __syncthreads();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, gr = lane >> 2, t = lane & 3;
@@ -445,10 +466,11 @@ adjust_frame_kernel(const float* __restrict__ base, const float* __restrict__ kp
       c[2 * m][0] = v0.x; c[2 * m][1] = v0.y; c[2 * m + 1][0] = v0.z; c[2 * m + 1][1] = v0.w;
       c[2 * m][2] = v1.x; c[2 * m][3] = v1.y; c[2 * m + 1][2] = v1.z; c[2 * m + 1][3] = v1.w;
     }
-    uint32_t a[2][4];
-    gauss_frags(q, s0, s1, t, a);
+    constexpr int GS = (KMAX + 15) / 16;
+    uint32_t a[GS][4];
+    gauss_frags<GS>(q, s0, s1, t, a);
 #pragma unroll
-    for (int st = 0; st < 2; st++)
+    for (int st = 0; st < GS; st++)
 #pragma unroll
       for (int nb = 0; nb < kAdjNB; nb++)
         adj_mma(c[nb], a[st][0], a[st][1], a[st][2], a[st][3], s_frag[(st * kAdjNB + nb) * 32 + lane]);
@@ -466,6 +488,60 @@ adjust_frame_kernel(const float* __restrict__ base, const float* __restrict__ kp
   }
 }
 
+// ------------------------------------------------------------------ launchers, one per keypoint capacity
+template <int C, int NB>
+int launch_head_heat(dim3 grid, cudaStream_t st, const act_t* feature, const float* w1, const float* b1, int K, int S,
+                      int mode, const float* prev, int frames_per_clip, float pw0, float pw1, float pb,
+                      const float* prop_dev, float* heat) {
+  size_t smem = 0;
+  if (NB * 8 > kTunedK) {
+    smem = head_frag_bytes<C, NB>();
+    NM_PER_DEVICE_ONCE({
+      NM_CHECK_CUDA(cudaFuncSetAttribute(head_heat_kernel<C, NB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    });
+  }
+  head_heat_kernel<C, NB><<<grid, 256, smem, st>>>(feature, w1, b1, K, S, mode, prev, frames_per_clip, pw0, pw1, pb,
+                                                   prop_dev, heat);
+  return NM_OK;
+}
+
+template <int KMAX>
+void launch_head_reduce(int n, cudaStream_t st, int K, int g, const float* lin, float gauss_width, const float* heat,
+                        float* keypoints, float* gaussians, float* heat_mean) {
+  const size_t smem2 = (size_t)(3 * KMAX * 32 + KMAX * 4 + KMAX * 3 * 32 + 32 * 32 + 256 + 256 * 33) * sizeof(float);
+  NM_PER_DEVICE_ONCE({
+    cudaFuncSetAttribute(head_reduce_kernel<KMAX>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                         KMAX <= kTunedK ? 64 * 1024 : (int)smem2);
+  });
+  head_reduce_kernel<KMAX><<<n, 256, smem2, st>>>(K, g, lin, gauss_width, heat, keypoints, gaussians, heat_mean);
+}
+
+template <int KMAX>
+int launch_adjust(const act_t* ff, const float* kp, const float* gaussians, const float* weight, const float* bias,
+                  int n_clips, int frames_per_clip, int g, int K, const float* lin, float width, float* base_ws, act_t* out,
+                  cudaStream_t st) {
+  const int S = g * g * g;
+  // workspace: [base fp32 (n_clips, S, 128)][packed weight fragments][(Wx, Wy, Wz, bias) per channel]
+  uint2* frags = reinterpret_cast<uint2*>(base_ws + (size_t)n_clips * S * kAdjCO);
+  float4* xyzb = reinterpret_cast<float4*>(frags + 2 * adj_frag_g<KMAX>() + kAdjFragFF);
+  adjust_pack_kernel<KMAX><<<8, 256, 0, st>>>(weight, bias, K, 2 * K + kAdjFD + 3, frags, xyzb);
+  NM_CHECK_LAUNCH("decoder_adjust(pack)");
+  const size_t smem = (size_t)(adj_frag_g<KMAX>() + kAdjFragFF) * sizeof(uint2);
+  NM_PER_DEVICE_ONCE({
+    NM_CHECK_CUDA(cudaFuncSetAttribute(adjust_base_kernel<KMAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
+  });
+  const int n = n_clips * frames_per_clip;
+  adjust_base_kernel<KMAX><<<dim3(S / 128, n_clips), 256, smem, st>>>(ff, kp, gaussians, frames_per_clip, frags, xyzb, K,
+                                                                       g, lin, width, base_ws);
+  NM_CHECK_LAUNCH("decoder_adjust(base)");
+  const int tiles_per_warp = S >= 4096 ? 4 : 1;
+  adjust_frame_kernel<KMAX><<<dim3(S / (128 * tiles_per_warp), n), 256, 0, st>>>(base_ws, kp, gaussians, frags, K, g,
+                                                                                  frames_per_clip, tiles_per_warp, lin,
+                                                                                  width, out);
+  NM_CHECK_LAUNCH("decoder_adjust(frame)");
+  return NM_OK;
+}
+
 }  // namespace
 
 extern "C" int nm_heatmap_head(const void* feature, const float* w1, const float* b1, int n, int g, int C, int K,
@@ -473,28 +549,27 @@ extern "C" int nm_heatmap_head(const void* feature, const float* w1, const float
                                const float* linspace, float gauss_width, float* heat, float* keypoints,
                                float* gaussians, float* heat_mean, void* stream) {
   NM_CHECK_ARG(feature && w1 && b1 && heat && linspace, "nm_heatmap_head: null pointer");
-  NM_CHECK_ARG(K <= KMAX && (g == 8 || g == 16 || g == 32), "nm_heatmap_head: K=%d g=%d unsupported", K, g);
+  NM_CHECK_ARG(K <= kMaxK && (g == 8 || g == 16 || g == 32), "nm_heatmap_head: K=%d g=%d unsupported", K, g);
   NM_CHECK_ARG(mode == 0 || (prev && keypoints), "nm_heatmap_head: mode 1 needs prev and keypoints");
   if (n == 0) return NM_OK;
+  NM_CHECK_ARG(C == 128 || C == 256, "nm_heatmap_head: C=%d unsupported", C);
   cudaStream_t st = (cudaStream_t)stream;
   const int S = g * g * g;
   dim3 grid1(nm_cdiv(S, 512), n);
-  if (C == 128) {
-    head_heat_kernel<128><<<grid1, 256, 0, st>>>((const act_t*)feature, w1, b1, K, S, mode, prev, frames_per_clip,
-                                                     pw0, pw1, pb, prop_dev, heat);
-  } else if (C == 256) {
-    head_heat_kernel<256><<<grid1, 256, 0, st>>>((const act_t*)feature, w1, b1, K, S, mode, prev, frames_per_clip,
-                                                     pw0, pw1, pb, prop_dev, heat);
+  const act_t* f = (const act_t*)feature;
+  int rc;
+  if (K <= kTunedK) {
+    if (C == 128) rc = launch_head_heat<128, kTunedK / 8>(grid1, st, f, w1, b1, K, S, mode, prev, frames_per_clip, pw0, pw1, pb, prop_dev, heat);
+    else rc = launch_head_heat<256, kTunedK / 8>(grid1, st, f, w1, b1, K, S, mode, prev, frames_per_clip, pw0, pw1, pb, prop_dev, heat);
   } else {
-    NM_CHECK_ARG(false, "nm_heatmap_head: C=%d unsupported", C);
+    if (C == 128) rc = launch_head_heat<128, kMaxK / 8>(grid1, st, f, w1, b1, K, S, mode, prev, frames_per_clip, pw0, pw1, pb, prop_dev, heat);
+    else rc = launch_head_heat<256, kMaxK / 8>(grid1, st, f, w1, b1, K, S, mode, prev, frames_per_clip, pw0, pw1, pb, prop_dev, heat);
   }
+  if (rc) return rc;
   NM_CHECK_LAUNCH("heatmap_head(heat)");
   if (mode == 0) return NM_OK;
-  const size_t smem2 = (size_t)(3 * KMAX * 32 + KMAX * 4 + KMAX * 3 * 32 + 32 * 32 + 256 + 256 * 33) * sizeof(float);
-  NM_PER_DEVICE_ONCE({
-    cudaFuncSetAttribute(head_reduce_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
-  });
-  head_reduce_kernel<<<n, 256, smem2, st>>>(K, g, linspace, gauss_width, heat, keypoints, gaussians, heat_mean);
+  if (K <= kTunedK) launch_head_reduce<kTunedK>(n, st, K, g, linspace, gauss_width, heat, keypoints, gaussians, heat_mean);
+  else launch_head_reduce<kMaxK>(n, st, K, g, linspace, gauss_width, heat, keypoints, gaussians, heat_mean);
   NM_CHECK_LAUNCH("heatmap_head(reduce)");
   return NM_OK;
 }
@@ -502,16 +577,20 @@ extern "C" int nm_heatmap_head(const void* feature, const float* w1, const float
 extern "C" int nm_gaussian_render(const float* keypoints, int n, int K, int g, const float* linspace,
                                   float gauss_width, float* gaussians, void* stream) {
   NM_CHECK_ARG(keypoints && linspace && gaussians, "nm_gaussian_render: null pointer");
-  NM_CHECK_ARG(K <= KMAX && g <= 32 && g % 4 == 0, "nm_gaussian_render: K=%d g=%d unsupported", K, g);
+  NM_CHECK_ARG(K <= kMaxK && g <= 32 && g % 4 == 0, "nm_gaussian_render: K=%d g=%d unsupported", K, g);
   if (n == 0) return NM_OK;
   const float width = gauss_width;
-  gaussian_render_kernel<<<n, 256, 0, (cudaStream_t)stream>>>(keypoints, K, g, linspace, width, gaussians);
+  if (K <= kTunedK)
+    gaussian_render_kernel<kTunedK><<<n, 256, 0, (cudaStream_t)stream>>>(keypoints, K, g, linspace, width, gaussians);
+  else
+    gaussian_render_kernel<kMaxK><<<n, 256, 0, (cudaStream_t)stream>>>(keypoints, K, g, linspace, width, gaussians);
   NM_CHECK_LAUNCH("gaussian_render");
   return NM_OK;
 }
 
+// sized for the kMaxK layout (the larger one) whatever K is, since the size does not take K
 extern "C" size_t nm_decoder_adjust_workspace_bytes(int n_clips, int g) {
-  return (size_t)n_clips * g * g * g * kAdjCO * sizeof(float) + (size_t)(2 * kAdjFragG + kAdjFragFF) * sizeof(uint2) +
+  return (size_t)n_clips * g * g * g * kAdjCO * sizeof(float) + (size_t)(2 * adj_frag_g<kMaxK>() + kAdjFragFF) * sizeof(uint2) +
          (size_t)kAdjCO * sizeof(float4);
 }
 
@@ -521,30 +600,13 @@ extern "C" int nm_decoder_adjust(const void* first_feature, const float* keypoin
                                  void* stream) {
   NM_CHECK_ARG(first_feature && weight && bias && base_ws && out && linspace, "nm_decoder_adjust: null pointer");
   NM_CHECK_ARG(keypoints || gaussians, "nm_decoder_adjust: need keypoints or gaussians");
-  NM_CHECK_ARG(K <= KMAX && (g == 8 || g == 16 || g == 32), "nm_decoder_adjust: K=%d g=%d unsupported", K, g);
+  NM_CHECK_ARG(K <= kMaxK && (g == 8 || g == 16 || g == 32), "nm_decoder_adjust: K=%d g=%d unsupported", K, g);
   if (n_clips == 0) return NM_OK;
-  const int S = g * g * g;
-  const float width = gauss_width;
-  cudaStream_t st = (cudaStream_t)stream;
-  // workspace: [base fp32 (n_clips, S, 128)][packed weight fragments][(Wx, Wy, Wz, bias) per channel]
-  uint2* frags = reinterpret_cast<uint2*>(base_ws + (size_t)n_clips * S * kAdjCO);
-  float4* xyzb = reinterpret_cast<float4*>(frags + 2 * kAdjFragG + kAdjFragFF);
-  adjust_pack_kernel<<<8, 256, 0, st>>>(weight, bias, K, 2 * K + kAdjFD + 3, frags, xyzb);
-  NM_CHECK_LAUNCH("decoder_adjust(pack)");
-  const size_t smem = (size_t)(kAdjFragG + kAdjFragFF) * sizeof(uint2);
-  NM_PER_DEVICE_ONCE({
-    NM_CHECK_CUDA(cudaFuncSetAttribute(adjust_base_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
-  });
-  const int n = n_clips * frames_per_clip;
   const float* kp = gaussians ? nullptr : keypoints;
-  adjust_base_kernel<<<dim3(S / 128, n_clips), 256, smem, st>>>((const act_t*)first_feature, kp, gaussians,
-                                                                 frames_per_clip, frags, xyzb, K, g, linspace, width,
-                                                                 base_ws);
-  NM_CHECK_LAUNCH("decoder_adjust(base)");
-  const int tiles_per_warp = S >= 4096 ? 4 : 1;
-  adjust_frame_kernel<<<dim3(S / (128 * tiles_per_warp), n), 256, 0, st>>>(base_ws, kp, gaussians, frags, K, g,
-                                                                            frames_per_clip, tiles_per_warp, linspace,
-                                                                            width, (act_t*)out);
-  NM_CHECK_LAUNCH("decoder_adjust(frame)");
-  return NM_OK;
+  const act_t* ff = (const act_t*)first_feature;
+  if (K <= kTunedK)
+    return launch_adjust<kTunedK>(ff, kp, gaussians, weight, bias, n_clips, frames_per_clip, g, K, linspace, gauss_width,
+                                  base_ws, (act_t*)out, (cudaStream_t)stream);
+  return launch_adjust<kMaxK>(ff, kp, gaussians, weight, bias, n_clips, frames_per_clip, g, K, linspace, gauss_width,
+                              base_ws, (act_t*)out, (cudaStream_t)stream);
 }

@@ -43,6 +43,9 @@ class HSVRNNBVH(nn.Module):
         if self.transition_type != "dl" or self.input_dim != 3 or self.nhidden_kypt != 512 or self.nlatent_kypt != 128:
             raise NotImplementedError("only transition_type='dl', input_dim=3, nhidden_kypt=512, nlatent_kypt=128 "
                                       "(the shipped configuration) is implemented")
+        if not 2 <= self.nkeypoints <= 64:
+            raise NotImplementedError(f"nkeypoints={self.nkeypoints}: only 2 <= nkeypoints <= 64 is implemented "
+                                      "(the CUDA kernels are compiled for at most 64 keypoints)")
         state_dim = self.nkeypoints * (self.input_dim + 1)
         H, Z = self.nhidden_kypt, self.nlatent_kypt
         self.extract_post_dist = _mlp(H + state_dim, 2 * Z)

@@ -313,6 +313,9 @@ class KyptDetector(nn.Module):
         self.input_dim = options.input_dim
         self.grid_size = options.grid_size
         self.nkeypoints = options.nkeypoints
+        if not 2 <= self.nkeypoints <= 64:
+            raise NotImplementedError(f"nkeypoints={self.nkeypoints}: only 2 <= nkeypoints <= 64 is implemented "
+                                      "(the CUDA kernels are compiled for at most 64 keypoints)")
         self.sigmas = [self.gaussian_sigma] * self.nkeypoints
         self.vox_to_kypt = VoxToKyptNet(grid_size=options.grid_size, nkeypoints=options.nkeypoints,
                                         input_dim=options.input_dim, sigmas=self.sigmas,
