@@ -17,6 +17,8 @@
 #include "../../include/nm_b200.h"   // the definitions below must match the public declarations
 #include <cuda.h>
 #include <string.h>
+#include <mutex>
+#include <vector>
 
 namespace {
 
@@ -157,6 +159,57 @@ __device__ __forceinline__ void tmem_ld8(uint32_t addr, uint32_t* r) {
                : "r"(addr));
 }
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
+__device__ __forceinline__ void tmem_st8(uint32_t addr, const uint32_t* r) {
+  asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};"
+               ::"r"(addr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7])
+               : "memory");
+}
+__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
+
+// ---- CTA pairs (cluster of 2, cta_group::2): one MMA of M = 256 reads A rows 128r.. and B rows r*N/2.. from the
+// shared memory of CTA r at the same offsets, and writes CTA r's own TMEM lanes (tools/probe/umma2_probe.cu).
+__device__ __forceinline__ uint32_t cluster_ctarank() {
+  uint32_t r;
+  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
+  return r;
+}
+__device__ __forceinline__ void cluster_sync() {
+  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
+  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
+}
+// Arrive on the barrier at the same shared-memory offset in CTA `rank` of the cluster.  Default (CTA-scope release)
+// semantics, as CUTLASS's 2-SM pipelines use: what the arrival publishes is consumed by the leader's tcgen05 ops, which
+// are ordered by the tcgen05 / async-proxy fences around it.  A .release.cluster arrive (a cluster-scope fence per
+// slice in every epilogue and producer warp) made the pair kernels 1.8x slower [measured, B200, 32->32 @ 64^3].
+__device__ __forceinline__ void mbar_arrive_remote(uint64_t* bar, uint32_t rank) {
+  asm volatile(
+      "{\n\t.reg .b32 ra;\n\t"
+      "mapa.shared::cluster.u32 ra, %0, %1;\n\t"
+      "mbarrier.arrive.shared::cluster.b64 _, [ra];\n\t}"
+      ::"r"(smem_u32(bar)), "r"(rank)
+      : "memory");
+}
+__device__ __forceinline__ void umma2_f16(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
+      ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+__device__ __forceinline__ void umma2_f16_acc(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, 1, 0;\n\t"
+      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
+      ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc)
+      : "memory");
+}
+// arrives on the barrier at this offset in both CTAs of the pair once the leader's MMAs issued so far retire
+__device__ __forceinline__ void umma2_commit(uint64_t* bar) {
+  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
+               ::"r"(smem_u32(bar)), "h"((uint16_t)3) : "memory");
+}
 
 // Column sums over the 32 lanes of a warp for 32 per-lane values: recursive halving (31 shuffles instead of
 // 160 for a butterfly all-reduce).  On exit lane l holds the total of column l in v[0].
@@ -423,7 +476,8 @@ constexpr int kHaloW = 10, kHaloH = 18;
 constexpr int kPGroups = 5;    // 5 x 96 TMEM columns = 480 <= 512
 
 // BK: channels per k-chunk (64 -> 128B swizzle, 32 -> 64B); PN: output channels per CTA "part" (32, or 16 when
-// Cin = 128 so that the 27 x kchunks resident weight tiles still fit); MMA N = 3 * PN.
+// Cin = 128 so that the 27 x kchunks resident weight tiles still fit, or 64 on a CTA pair, which holds half of them);
+// MMA N = 3 * PN.
 constexpr int kSlab3EpiWarps = 8;
 constexpr int kSlab3Threads = 64 + 32 * kSlab3EpiWarps;
 constexpr int kSlab3Ring = 8;        // max halo-slice ring depth (Cin = 32 has room for 8 slots, Cin = 64 for 4)
@@ -444,16 +498,27 @@ constexpr int kLoBytes = kLoRows * 128;      // 7680
 constexpr int kUpWarps = 4;                  // up-sampling producer warps launched (3 working)
 
 // ACC: split-K second launch - the epilogue adds the partial sum already in `out`.
-template <int BK, int PN, bool UP = false, bool ACC = false>
+// PAIR: a cluster of two CTAs that own two adjacent 8-wide w tiles of the same (n, h-tile) column and walk d in
+// lockstep.  The leader (rank 0) issues cta_group::2 MMAs of M = 256 x N = 3 * PN; each CTA holds its own halo slices
+// and half of the stacked weight rows (CTA r: rows r * 3PN/2 ..), so per CTA the B-operand read of an MMA and the
+// resident weights are halved.  The peer's slices, transforms and drained TMEM groups are reported to the leader's
+// barriers by remote arrives; the leader's commits arrive on the barriers of both CTAs (multicast).
+template <int BK, int PN, bool UP = false, bool ACC = false, bool PAIR = false>
 __global__ void __launch_bounds__(kSlab3Threads + 32 * kSlab3XformWarps, 1)
 conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
   static_assert(!UP || PN == 32, "the up-sampling epilogue serves 32-channel parts");
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-  constexpr int w_tile_bytes = PN * BK * 2;                            // one (tap, k-chunk)
-  const int w_bytes = 27 * p.kchunks * w_tile_bytes;
+  constexpr int CG = PAIR ? 2 : 1;                                     // CTAs per MMA
+  // TMEM groups P(s) of 3 * PN columns in flight: 5 x 96, or 2 x 192 with PN = 64 (the epilogue then carries the
+  // running sums in the remaining 2 x 64 columns)
+  constexpr int PG = PN == 64 ? 2 : kPGroups;
+  static_assert(PN != 64 || (PAIR && !UP && !ACC), "64-channel parts run on CTA pairs, without up-sampling / split-K");
+  constexpr int box_rows = PN / CG;                                    // rows of one weight TMA box
+  constexpr int w_tile_bytes = 3 * box_rows * BK * 2;                  // one (kh, kw, k-chunk): this CTA's stacked rows
+  const int w_bytes = 9 * p.kchunks * w_tile_bytes;
   const int ring = p.ring;
-  uint8_t* s_w = smem;                                                 // [kh*3+kw][kc][kd][PN rows][BK]
+  uint8_t* s_w = smem;                                                 // [kh*3+kw][kc][3 * PN / CG rows][BK]
   uint8_t* s_ring = smem + w_bytes;
   constexpr int stage_bytes = kTileM * PN * 2;                         // one output tile (128 rows x PN fp16)
   uint8_t* s_lo = s_ring + (size_t)ring * p.slot_bytes;                // UP: [kLoRing][kLoBytes] low-res planes
@@ -478,28 +543,45 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
   constexpr uint32_t tmem_cols = 512;
   // Cout > PN: the output channels are split into parts of PN; CTA b serves part b % parts with its own
   // resident weights (A is re-read once per part, each pass runs at the N = 3*PN rate)
+  // (with PAIR the "unit" is a CTA pair: cluster c = CTAs 2c, 2c+1, column pair (2j, 2j+1))
   const int parts = p.n_tile / PN;
-  const int part = blockIdx.x % parts;
-  const int col0 = blockIdx.x / parts, col_step = gridDim.x / parts;
+  const int rank = PAIR ? (int)cluster_ctarank() : 0;
+  const int unit = blockIdx.x / CG, n_units = gridDim.x / CG;
+  const int part = unit % parts;
+  const int col0 = (unit / parts) * CG + rank, col_step = (n_units / parts) * CG;
+  // barriers of the leader that the peer CTA also arrives on count its arrivals too
+  const uint32_t peers = PAIR && rank == 0 ? 2u : 1u;
+  // arrival on a barrier the MMA issuer waits on: the leader's copy
+  auto arrive_issuer = [&](uint64_t* bar) {
+    if constexpr (PAIR) mbar_arrive_remote(bar, 0);
+    else mbar_arrive(bar);
+  };
 
   if (warp == 0 && lane == 0) {
     asm volatile("prefetch.tensormap [%0];" ::"l"(&p.tmap_a) : "memory");
     asm volatile("prefetch.tensormap [%0];" ::"l"(&p.tmap_b) : "memory");
     asm volatile("prefetch.tensormap [%0];" ::"l"(&p.tmap_o) : "memory");
-    for (int s = 0; s < kSlab3Ring; s++) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
-    for (int s = 0; s < kPGroups; s++) { mbar_init(&pfull[s], 1); mbar_init(&pempty[s], kSlab3EpiWarps); }
-    for (int s = 0; s < kSlab3Ring; s++) mbar_init(&ready[s], nxw);
+    for (int s = 0; s < kSlab3Ring; s++) { mbar_init(&full[s], xform ? 1 : peers); mbar_init(&empty[s], 1); }
+    for (int s = 0; s < kPGroups; s++) { mbar_init(&pfull[s], 1); mbar_init(&pempty[s], kSlab3EpiWarps * peers); }
+    for (int s = 0; s < kSlab3Ring; s++) mbar_init(&ready[s], nxw * peers);
     for (int s = 0; s < kLoRing; s++) { mbar_init(&full_lo[s], 1); mbar_init(&empty_lo[s], nxw); }
-    mbar_init(wfull, 1);
+    mbar_init(wfull, peers);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(tmem_cols)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    if constexpr (PAIR) {   // one warp in each CTA of the pair
+      asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(tmem_cols)
+                   : "memory");
+      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+    } else {
+      asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(tmem_cols)
+                   : "memory");
+      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    }
   }
   tc_fence_before();
   __syncthreads();
+  if constexpr (PAIR) cluster_sync();   // the peer's barriers are initialised before anything arrives on them
   tc_fence_after();
   if (*tmem_slot != 0u) {       // single allocation per SM: base 0 keeps all TMEM addresses warp-uniform
     printf("nm_conv3d_tc(slab3): unexpected TMEM base %u\n", *tmem_slot);
@@ -641,7 +723,7 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
         fence_async_smem();                              // generic-proxy writes -> visible to the UMMA reads
         __syncwarp();
         if (lane == 0) {
-          mbar_arrive(&ready[slot]);
+          arrive_issuer(&ready[slot]);
           mbar_arrive(&empty_lo[g % kLoRing]);
         }
       }
@@ -721,7 +803,7 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
         }
         fence_async_smem();                              // generic-proxy writes -> visible to the UMMA reads
         __syncwarp();
-        if (lane == 0) mbar_arrive(&ready[slot]);
+        if (lane == 0) arrive_issuer(&ready[slot]);
       }
     }
   } else
@@ -730,12 +812,15 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
     // ===================== TMA producer =====================
     if (lane == 0) {
       mbar_expect_tx(wfull, (uint32_t)w_bytes);
-      for (int tap = 0; tap < 27; tap++) {
-        const int kd = tap / 9, khw = tap % 9;
+      // stacked tile of a (kh, kw, k-chunk): W(kd = 0) | W(kd = 1) | W(kd = 2), PN rows each, in boxes of box_rows;
+      // this CTA holds boxes 3 * rank .. 3 * rank + 2
+      for (int khw = 0; khw < 9; khw++)
         for (int kc = 0; kc < p.kchunks; kc++)
-          tma_load_3d(s_w + (size_t)((khw * p.kchunks + kc) * 3 + kd) * w_tile_bytes, &p.tmap_b, wfull,
-                      p.cin_off + kc * BK, part * PN, tap);
-      }
+          for (int b = 0; b < 3; b++) {
+            const int jb = 3 * rank + b, kd = jb / CG;
+            tma_load_3d(s_w + (size_t)(khw * p.kchunks + kc) * w_tile_bytes + (size_t)b * box_rows * BK * 2, &p.tmap_b,
+                        wfull, p.cin_off + kc * BK, part * PN + (jb % CG) * box_rows, kd * 9 + khw);
+          }
       uint32_t fill = 0;
       const uint32_t slice_tx = (uint32_t)(kHaloW * kHaloH * BK * 2 * p.kchunks);
       for (int col = col0; col < n_cols; col += col_step) {
@@ -761,16 +846,46 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
                         p.cin_off + kc * BK, iw * 8 - 1, ih * 16 - 1, dz, n);
         }
       }
+      // a pair's CTA does not exit while the leader's last commits may still arrive on its slot barriers
+      if constexpr (PAIR)
+        for (int i = 0; i < ring; i++, fill++) mbar_wait(&empty[fill % ring], ((fill / ring) & 1) ^ 1);
     }
+  } else if (PAIR && warp == 1 && rank != 0) {
+    // ===================== pair peer: forwards its landed weights / slices to the leader's barriers =====================
+    if (elect_one()) {
+      mbar_wait(wfull, 0);
+      mbar_arrive_remote(wfull, 0);
+      if (!xform) {                                      // (with a transform the producer warps report `ready`)
+        uint32_t q = 0;
+        for (int col = col0; col < n_cols; col += col_step)
+          for (int sl = 0; sl < p.D; sl++, q++) {
+            mbar_wait(&full[q % ring], (q / ring) & 1);
+            mbar_arrive_remote(&full[q % ring], 0);
+          }
+      }
+    }
+    __syncwarp();
   } else if (warp == 1) {
     // ===================== MMA issuer =====================
-    constexpr uint32_t idesc = (1u << 4) | ((uint32_t)((3 * PN) >> 3) << 17) | ((uint32_t)(kTileM >> 4) << 24);
+    constexpr uint32_t idesc = (1u << 4) | ((uint32_t)((3 * PN) >> 3) << 17) | ((uint32_t)(CG * kTileM >> 4) << 24);
     constexpr uint32_t row_bytes = BK * 2;
     constexpr uint32_t layout = row_bytes == 128 ? 2u : 4u;
     const uint32_t hi_a = desc_hi(kHaloW * row_bytes, layout), hi_b = desc_hi(8 * row_bytes, layout);
     const uint32_t ring_lo = desc_lo(smem_u32(s_ring)), w_lo = desc_lo(smem_u32(s_w));
     const uint32_t slot_step = (uint32_t)p.slot_bytes >> 4, chunk_step = (uint32_t)p.chunk_bytes >> 4;
-    constexpr uint32_t w_step = (uint32_t)(3 * w_tile_bytes) >> 4;       // one (khw, kc) B tile = 3 kd tiles
+    constexpr uint32_t w_step = (uint32_t)w_tile_bytes >> 4;             // one (khw, kc) B tile = 3 kd tiles
+    auto mma = [&](uint32_t tmem_d, uint32_t alo, uint32_t blo, uint32_t accumulate) {
+      if constexpr (PAIR) umma2_f16(tmem_d, desc64(hi_a, alo), desc64(hi_b, blo), idesc, accumulate);
+      else umma_f16(tmem_d, desc64(hi_a, alo), desc64(hi_b, blo), idesc, accumulate);
+    };
+    auto mma_acc = [&](uint32_t tmem_d, uint32_t alo, uint32_t blo) {
+      if constexpr (PAIR) umma2_f16_acc(tmem_d, desc64(hi_a, alo), desc64(hi_b, blo), idesc);
+      else umma_f16_acc(tmem_d, desc64(hi_a, alo), desc64(hi_b, blo), idesc);
+    };
+    auto commit = [&](uint64_t* bar) {
+      if constexpr (PAIR) umma2_commit(bar);
+      else umma_commit(bar);
+    };
     if (xform) {
       // With an in-kernel operand producer (fused GroupNorm / up-sampling) the plain loop is faster [measured: dec.8
       // with fused up-sampling 9.0 vs 9.4 ms, dec.11 with fused GroupNorm 5.4 vs 6.0 ms]: the burstier stream of the
@@ -780,11 +895,11 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
       for (int col = col0; col < n_cols; col += col_step) {
         for (int sl = 0; sl < n_sl; sl++, q++) {
           mbar_wait(&ready[q % ring], (q / ring) & 1);
-          mbar_wait(&pempty[q % kPGroups], ((q / kPGroups) & 1) ^ 1);
+          mbar_wait(&pempty[q % PG], ((q / PG) & 1) ^ 1);
           tc_fence_after();
           __syncwarp();
           if (elect_one()) {
-            const uint32_t tmem_d = (q % kPGroups) * (3 * PN);
+            const uint32_t tmem_d = (q % PG) * (3 * PN);
             const uint32_t slot_lo = ring_lo + (q % ring) * slot_step;
             uint32_t blo = w_lo;
 #pragma unroll
@@ -793,16 +908,15 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
 #pragma unroll 1
               for (int kc = 0; kc < p.kchunks; kc++) {
                 const uint32_t alo = tap_lo + kc * chunk_step;
-                if (t9 == 0 && kc == 0) umma_f16(tmem_d, desc64(hi_a, alo), desc64(hi_b, blo), idesc, 0u);
-                else umma_f16_acc(tmem_d, desc64(hi_a, alo), desc64(hi_b, blo), idesc);
+                if (t9 == 0 && kc == 0) mma(tmem_d, alo, blo, 0u);
+                else mma_acc(tmem_d, alo, blo);
 #pragma unroll
-                for (int k = 1; k < BK / 16; k++)
-                  umma_f16_acc(tmem_d, desc64(hi_a, alo + 2 * k), desc64(hi_b, blo + 2 * k), idesc);
+                for (int k = 1; k < BK / 16; k++) mma_acc(tmem_d, alo + 2 * k, blo + 2 * k);
                 blo += w_step;
               }
             }
-            umma_commit(&empty[q % ring]);
-            umma_commit(&pfull[q % kPGroups]);
+            commit(&empty[q % ring]);
+            commit(&pfull[q % PG]);
           }
           __syncwarp();
         }
@@ -816,7 +930,7 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
       uint32_t q = 0;                                    // global slice counter (ring + P-group position)
       auto wait_slice = [&](uint32_t qq) {
         mbar_wait(&full[qq % ring], (qq / ring) & 1);
-        mbar_wait(&pempty[qq % kPGroups], ((qq / kPGroups) & 1) ^ 1);
+        mbar_wait(&pempty[qq % PG], ((qq / PG) & 1) ^ 1);
         tc_fence_after();
       };
       auto issue_tap = [&](int t9, uint32_t tmem_d, uint32_t slot_lo, uint32_t& blo) {
@@ -824,18 +938,17 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
 #pragma unroll 1
         for (int kc = 0; kc < p.kchunks; kc++) {
           const uint32_t alo = tap_lo + kc * chunk_step;
-          if (t9 == 0 && kc == 0) umma_f16(tmem_d, desc64(hi_a, alo), desc64(hi_b, blo), idesc, 0u);
-          else umma_f16_acc(tmem_d, desc64(hi_a, alo), desc64(hi_b, blo), idesc);
+          if (t9 == 0 && kc == 0) mma(tmem_d, alo, blo, 0u);
+          else mma_acc(tmem_d, alo, blo);
 #pragma unroll
-          for (int k = 1; k < BK / 16; k++)
-            umma_f16_acc(tmem_d, desc64(hi_a, alo + 2 * k), desc64(hi_b, blo + 2 * k), idesc);
+          for (int k = 1; k < BK / 16; k++) mma_acc(tmem_d, alo + 2 * k, blo + 2 * k);
           blo += w_step;
         }
       };
       // non-blocking variant: true when both barriers of slice qq have already completed
       auto try_slice = [&](uint32_t qq) -> bool {
         if (!mbar_try_wait(&full[qq % ring], (qq / ring) & 1)) return false;
-        if (!mbar_try_wait(&pempty[qq % kPGroups], ((qq / kPGroups) & 1) ^ 1)) return false;
+        if (!mbar_try_wait(&pempty[qq % PG], ((qq / PG) & 1) ^ 1)) return false;
         tc_fence_after();
         return true;
       };
@@ -843,7 +956,7 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
       for (int col = col0; col < n_cols; col += col_step) {
         for (int sl = 0; sl < p.D; sl++, q++) {
           if (!ready_now) wait_slice(q);
-          const uint32_t tmem_d = (q % kPGroups) * (3 * PN);
+          const uint32_t tmem_d = (q % PG) * (3 * PN);
           const uint32_t slot_lo = ring_lo + (q % ring) * slot_step;
           uint32_t blo = w_lo;
           const bool has_next = sl + 1 < p.D || col + col_step < n_cols;
@@ -851,8 +964,8 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
           for (int t9 = 0; t9 < 8; t9++) issue_tap(t9, tmem_d, slot_lo, blo);
           ready_now = has_next && try_slice(q + 1);      // if it is not there yet, block after this slice's commits
           issue_tap(8, tmem_d, slot_lo, blo);
-          umma_commit(&empty[q % ring]);
-          umma_commit(&pfull[q % kPGroups]);
+          commit(&empty[q % ring]);
+          commit(&pfull[q % PG]);
         }
       }
     }
@@ -870,7 +983,7 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
     // UP: the bias is read from shared memory (broadcast), which keeps that epilogue within 128 registers; it sits
     // behind the scale / shift (Cin = 64, well inside the 2 x 256 floats reserved for them)
     float* s_bias = s_ab + 2 * p.cin;
-    if constexpr (UP) {
+    if constexpr (UP || PN == 64) {
       const int e = threadIdx.x - 64;
       if (e < PN) s_bias[e] = (p.bias && part * PN + e < p.cout) ? __ldg(p.bias + part * PN + e) : 0.f;
       named_bar_sync(1, 32 * kSlab3EpiWarps);
@@ -885,12 +998,12 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
     uint32_t n_out = 0;                                  // output tiles staged so far (staging buffer parity)
     const bool is_issuer = warp == 2 && lane == 0;       // the thread that owns the TMA-store bulk groups
     // this thread's 16-byte chunks in the staging tile (swizzled like the store tensor map): constant per thread
-    constexpr int row_b = PN * 2;                        // 64 B (SWIZZLE_64B) or 32 B (SWIZZLE_32B)
+    constexpr int row_b = PN * 2;                        // 128 B (SWIZZLE_128B), 64 B (SWIZZLE_64B) or 32 B (SWIZZLE_32B)
     uint32_t st_off[CW / 8];
 #pragma unroll
     for (int c8 = 0; c8 < CW / 8; c8++) {
       const uint32_t off = (uint32_t)row * row_b + (uint32_t)(chalf * CW + c8 * 8) * 2;
-      st_off[c8] = off ^ (((off >> 7) & (row_b == 64 ? 3u : 1u)) << 4);
+      st_off[c8] = off ^ (((off >> 7) & (row_b == 128 ? 7u : (row_b == 64 ? 3u : 1u))) << 4);
     }
     const uint32_t s_out_u32 = smem_u32(s_out);
     for (int col = col0; col < n_cols; col += col_step, q0 += n_sl) {
@@ -1016,13 +1129,94 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
           tc_fence_before();
           __syncwarp();
           if (lane == 0) {
-            if (!first) mbar_arrive(&pempty[(q + kPGroups - 1) % kPGroups]);
-            if (last) mbar_arrive(&pempty[q % kPGroups]);
+            if (!first) arrive_issuer(&pempty[(q + kPGroups - 1) % kPGroups]);
+            if (last) arrive_issuer(&pempty[q % kPGroups]);
           }
           if (last) {
             if (ACC) { load_prev(pvq, 2 * s); load_prev(pvq1, 2 * s + 1); }
             emit(part0, 2 * s, pvq);
             emit(part1, 2 * s + 1, pvq1);
+          }
+        }
+      } else if constexpr (PN == 64) {
+        // N = 192: TMEM holds two groups (columns 0 and 192) and two carries: C0 (columns 384..447) = P(s)[0] raw,
+        // C1 (448..511) = the partial sum of out(s).  Event s reads all of P(s) and releases it at once:
+        //   out(s-1) = C1 + P(s)[2]          (emitted)
+        //   C1      <- (P(s)[1] + C0) + bias (C0 = P(s-1)[0]; 0 at s = 0)
+        //   C0      <- P(s)[0]
+        // the same additions in the same order as the 32-channel epilogue, 8 columns at a time (register budget).
+        const uint32_t c0a = lane_addr + 6 * PN, c1a = lane_addr + 7 * PN;
+        auto stage = [&](const float (&f)[8], int c8) {
+#pragma unroll
+          for (int k = 0; k < 8; k++) { ssum[c8 * 8 + k] += f[k]; ssq[c8 * 8 + k] = fmaf(f[k], f[k], ssq[c8 * 8 + k]); }
+          const half8 hv = nm_pack8(f);
+          sts128(s_out_u32 + (n_out & 1) * stage_bytes + st_off[c8], *reinterpret_cast<const uint4*>(&hv));
+        };
+        auto store_tile = [&](int od) {
+          fence_async_smem();
+          named_bar_sync(1, 32 * kSlab3EpiWarps);
+          if (is_issuer) {
+            tma_store_5d(&p.tmap_o, s_out + (n_out & 1) * stage_bytes, part * PN, iw * 8, ih * 16, od, n);
+            bulk_commit();
+          }
+          n_out++;
+        };
+        auto claim_staging = [&]() {
+          if (is_issuer) bulk_wait_read<1>();              // the store that last read this buffer has drained
+          named_bar_sync(1, 32 * kSlab3EpiWarps);
+        };
+        for (int sl = 0; sl < p.D; sl++) {
+          const uint32_t q = q0 + sl;
+          if (xform) mbar_wait_backoff(&pfull[q % PG], (q / PG) & 1, 100u);
+          else mbar_wait(&pfull[q % PG], (q / PG) & 1);
+          tc_fence_after();
+          const uint32_t g = lane_addr + (q % PG) * (3 * PN);
+          if (sl >= 1) claim_staging();
+#pragma unroll
+          for (int c8 = 0; c8 < CW / 8; c8++) {
+            uint32_t ra[8], rb[8];
+            if (sl >= 1) {
+              tmem_ld8(g + 2 * PN + c8 * 8, ra);
+              tmem_ld8(c1a + c8 * 8, rb);
+              tmem_ld_wait();
+              float f[8];
+#pragma unroll
+              for (int k = 0; k < 8; k++) f[k] = __uint_as_float(rb[k]) + __uint_as_float(ra[k]);
+              stage(f, c8);
+            }
+            tmem_ld8(g + PN + c8 * 8, ra);
+            if (sl >= 1) tmem_ld8(c0a + c8 * 8, rb);
+            tmem_ld_wait();
+            if (sl == 0) {
+#pragma unroll
+              for (int k = 0; k < 8; k++) rb[k] = 0u;
+            }
+#pragma unroll
+            for (int k = 0; k < 8; k++)
+              ra[k] = __float_as_uint((__uint_as_float(ra[k]) + __uint_as_float(rb[k])) + s_bias[chalf * CW + c8 * 8 + k]);
+            tmem_st8(c1a + c8 * 8, ra);
+            tmem_ld8(g + c8 * 8, rb);
+            tmem_ld_wait();
+            tmem_st8(c0a + c8 * 8, rb);
+          }
+          tmem_st_wait();
+          tc_fence_before();
+          __syncwarp();
+          if (lane == 0) arrive_issuer(&pempty[q % PG]);
+          if (sl >= 1) store_tile(sl - 1);
+          if (sl == p.D - 1) {                             // out(D-1) = C1
+            claim_staging();
+#pragma unroll
+            for (int c8 = 0; c8 < CW / 8; c8++) {
+              uint32_t ra[8];
+              tmem_ld8(c1a + c8 * 8, ra);
+              tmem_ld_wait();
+              float f[8];
+#pragma unroll
+              for (int k = 0; k < 8; k++) f[k] = __uint_as_float(ra[k]);
+              stage(f, c8);
+            }
+            store_tile(sl);
           }
         }
       } else {
@@ -1050,8 +1244,8 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
           tc_fence_before();
           __syncwarp();
           if (lane == 0) {
-            if (sl >= 1) mbar_arrive(&pempty[(q + kPGroups - 1) % kPGroups]);
-            if (sl == p.D - 1) mbar_arrive(&pempty[q % kPGroups]);
+            if (sl >= 1) arrive_issuer(&pempty[(q + kPGroups - 1) % kPGroups]);
+            if (sl == p.D - 1) arrive_issuer(&pempty[q % kPGroups]);
           }
           // out(sl-1) is complete now; out(D-1) completes together with the last event
           if (sl >= 1) {
@@ -1092,9 +1286,13 @@ conv3d_slab3_kernel(const __grid_constant__ ConvSlabParams p) {
   }
   tc_fence_before();
   __syncthreads();
+  if constexpr (PAIR) cluster_sync();   // no CTA of the pair leaves while the other may still arrive on its barriers
   if (warp == 1) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(0u), "r"(tmem_cols) : "memory");
+    if constexpr (PAIR)
+      asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(0u), "r"(tmem_cols) : "memory");
+    else
+      asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(0u), "r"(tmem_cols) : "memory");
   }
 }
 
@@ -1143,8 +1341,9 @@ extern "C" int nm_pack_conv_weights(const float* weight, void* packed, int Cout,
 namespace {
 // Which kernel serves this conv (slab3: conv3d_slab3_kernel, else conv3d_tc_kernel), and how many GroupNorm partial
 // chunks per sample it can emit (0 = none).
-struct ConvPlan { bool slab3; int bk, kch, ntile, pn, ring, chunk_bytes; size_t need, w_bytes, extra; int stats_chunks; };
-ConvPlan plan_conv(int n, int D, int H, int W, int Cin, int Cout, int k, int stride) {
+struct ConvPlan { bool slab3, pair; int bk, kch, ntile, pn, ring, chunk_bytes; size_t need, w_bytes, extra; int stats_chunks; };
+// wide64: a pair may serve 64 output channels per part (not for the up-sampling and split-K launches)
+ConvPlan plan_conv(int n, int D, int H, int W, int Cin, int Cout, int k, int stride, bool wide64 = true) {
   ConvPlan pl;
   memset(&pl, 0, sizeof(pl));
   pl.bk = Cin >= 64 ? 64 : 32;
@@ -1166,6 +1365,20 @@ ConvPlan plan_conv(int n, int D, int H, int W, int Cin, int Cout, int k, int str
              Cin % pl.bk == 0 && W % 8 == 0 && H % 16 == 0 && pl.need <= 227 * 1024;
   if (pl.slab3) {
     pl.stats_chunks = (H / 16) * (W / 8) * 4;
+    // CTA pairs own two adjacent 8-wide w tiles; each CTA holds half of the weights, the freed room deepens the ring.
+    // (Cin = 128 parts, PN = 16, stay on single CTAs: no pair instantiation.)
+    pl.pair = pl.pn == 32 && W % 16 == 0;
+    if (pl.pair) {
+      // Cout % 64 == 0: one 64-channel part per pair, N = 192 (the full MMA rate; each slice is fetched, transformed and
+      // read as A once per 64 channels instead of once per 32).  Each CTA then holds 96 of the 192 stacked weight rows.
+      if (wide64 && Cout % 64 == 0) pl.pn = 64;
+      pl.w_bytes = (size_t)27 * pl.kch * pl.pn * pl.bk;
+      pl.extra = 1024 + 48 * 8 + 16 + 2 * 256 * 4 + (size_t)2 * kTileM * pl.pn * 2;
+      pl.ring = kSlab3Ring;
+      while (pl.ring > 2 && pl.w_bytes + (size_t)pl.ring * pl.kch * pl.chunk_bytes + pl.extra > 227 * 1024) pl.ring--;
+      pl.need = pl.w_bytes + (size_t)pl.ring * pl.kch * pl.chunk_bytes + pl.extra;
+      if (pl.need > 227 * 1024) pl.pair = false;   // (cannot happen for kch == 1; kept as the fit condition)
+    }
   } else {
     const int OD = D / stride, OH = H / stride, OW = W / stride;
     const int tw = OW < 8 ? OW : 8, th = OH < 4 ? OH : 4, td = OD < 4 ? OD : 4;
@@ -1211,7 +1424,7 @@ int conv3d_tc_impl(const void* x, const void* packed_w, const float* bias, void*
 bool up2x_ok(int n, int D, int H, int W, int Cin, int Cout) {
   if ((D | H | W) & 1) return false;
   if (Cin == 128) Cin = 64;   // split-K: two launches over 64-channel slices of the low-resolution tensor
-  const ConvPlan pl = plan_conv(n, D, H, W, Cin, Cout, 3, 1);
+  const ConvPlan pl = plan_conv(n, D, H, W, Cin, Cout, 3, 1, false);
   return pl.slab3 && pl.bk == 64 && pl.kch == 1 && pl.pn == 32 &&
          pl.w_bytes + (size_t)3 * pl.chunk_bytes + kLoRing * kLoBytes + pl.extra <= 227 * 1024;
 }
@@ -1252,6 +1465,32 @@ extern "C" int nm_conv3d_tc_up2x(const void* x_lo, const void* packed_w, const f
 }
 
 namespace {
+// Clusters of two CTAs of `kern` that can be resident at once with this block size and shared memory.  It depends on
+// how the SMs group into TPCs and GPCs, so it is asked of the runtime rather than taken as #SMs / 2; cached per
+// (device, kernel, block size, shared memory).
+cudaError_t max_resident_pairs(const void* kern, const cudaLaunchConfig_t& cfg, int* out) {
+  struct Entry { int dev; const void* kern; unsigned threads; size_t smem; int pairs; };
+  static std::mutex mu;
+  static std::vector<Entry> cache;
+  int dev = 0;
+  cudaError_t e = cudaGetDevice(&dev);
+  if (e != cudaSuccess) return e;
+  std::lock_guard<std::mutex> lock(mu);
+  for (const Entry& c : cache)
+    if (c.dev == dev && c.kern == kern && c.threads == cfg.blockDim.x && c.smem == cfg.dynamicSmemBytes) {
+      *out = c.pairs;
+      return cudaSuccess;
+    }
+  cudaLaunchConfig_t probe = cfg;
+  probe.gridDim = dim3(2 * nm_num_sms());
+  int pairs = 0;
+  e = cudaOccupancyMaxActiveClusters(&pairs, kern, &probe);
+  if (e != cudaSuccess) return e;
+  cache.push_back({dev, kern, cfg.blockDim.x, cfg.dynamicSmemBytes, pairs});
+  *out = pairs;
+  return cudaSuccess;
+}
+
 int conv3d_tc_impl(const void* x, const void* packed_w, const float* bias, void* out, int n, int D, int H, int W,
                    int Cin, int Cout, int k, int stride, const float* in_scale, const float* in_shift, int in_act,
                    float* stats_partial, void* stream, bool up, int cin_total, int cin_off, int accum) {
@@ -1262,7 +1501,7 @@ int conv3d_tc_impl(const void* x, const void* packed_w, const float* bias, void*
   // chunk at a time allows 32-channel parts (N = 96, 92 cycles for 48).  The second launch adds the fp16 partial sum
   // the first one left in `out`; GroupNorm statistics come from the second.
   if (!up && !in_scale && cin_total == Cin && Cin == 128 && Cout % 32 == 0 && Cout <= 64 && k == 3 && stride == 1 && n > 0) {
-    const ConvPlan half = plan_conv(n, D, H, W, 64, Cout, k, stride);
+    const ConvPlan half = plan_conv(n, D, H, W, 64, Cout, k, stride, false);
     if (half.slab3 && half.pn == 32) {
       const int rc = conv3d_tc_impl(x, packed_w, bias, out, n, D, H, W, 64, Cout, k, stride, nullptr, nullptr, 0, nullptr,
                                     stream, false, 128, 0, 0);
@@ -1283,7 +1522,7 @@ int conv3d_tc_impl(const void* x, const void* packed_w, const float* bias, void*
     return NM_ERR_DRIVER;
   }
   // ---- slab-walking kernel: k3, weights resident in smem
-  ConvPlan pl = plan_conv(n, D, H, W, Cin, Cout, k, stride);
+  ConvPlan pl = plan_conv(n, D, H, W, Cin, Cout, k, stride, !up && cin_total == Cin);
   if (up) {
     pl.ring = 3;
     pl.need = pl.w_bytes + (size_t)3 * pl.chunk_bytes + kLoRing * kLoBytes + pl.extra;
@@ -1321,7 +1560,7 @@ int conv3d_tc_impl(const void* x, const void* packed_w, const float* bias, void*
     if (r != CUDA_SUCCESS) { nm_set_error("nm_conv3d_tc(slab3): cuTensorMapEncodeTiled(A) failed with %d", (int)r); return NM_ERR_DRIVER; }
     cuuint64_t wdims[3] = {ct, (cuuint64_t)Cout, 27};
     cuuint64_t wstrides[2] = {ct * 2, ct * Cout * 2};
-    cuuint32_t wbox[3] = {(cuuint32_t)bk, (cuuint32_t)pn, 1};
+    cuuint32_t wbox[3] = {(cuuint32_t)bk, (cuuint32_t)(pl.pair ? pn / 2 : pn), 1};
     cuuint32_t westr[3] = {1, 1, 1};
     r = encode(&q.tmap_b, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, (void*)packed_w, wdims, wstrides, wbox, westr,
                CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
@@ -1331,32 +1570,74 @@ int conv3d_tc_impl(const void* x, const void* packed_w, const float* bias, void*
                               (cuuint64_t)D * H * W * Cout * 2};
     cuuint32_t obox[5] = {(cuuint32_t)pn, 8, 16, 1, 1};
     r = encode(&q.tmap_o, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 5, out, odims, ostrides, obox, estr,
-               CU_TENSOR_MAP_INTERLEAVE_NONE, pn == 32 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B,
+               CU_TENSOR_MAP_INTERLEAVE_NONE,
+               pn == 64 ? CU_TENSOR_MAP_SWIZZLE_128B : (pn == 32 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B),
                CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) { nm_set_error("nm_conv3d_tc(slab3): cuTensorMapEncodeTiled(out) failed with %d", (int)r); return NM_ERR_DRIVER; }
     const int cols = n * q.nh * q.nw;
     const int parts = ntile / pn;
-    const int grid = cols * parts < nm_num_sms() ? cols * parts : (nm_num_sms() / parts) * parts;
     NM_PER_DEVICE_ONCE({
+      NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab3_kernel<64, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
       NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab3_kernel<64, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
       NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab3_kernel<32, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-      NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab3_kernel<64, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
       NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab3_kernel<64, 32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
       NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab3_kernel<64, 32, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
       NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab3_kernel<64, 32, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+      NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab3_kernel<64, 32, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+      NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab3_kernel<32, 32, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+      NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab3_kernel<64, 64, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+      NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab3_kernel<32, 64, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+      NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab3_kernel<64, 32, true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+      NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab3_kernel<64, 32, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+      NM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab3_kernel<64, 32, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
     });
     // the up-sampling producer runs on 4 warps (3 working): with 6 (5 working, 144 finer items) dec.8 got slower
     // [measured, same GPU: 20.4 -> 24.6 ms per 640 frames] - more producer threads take issue slots and shared-memory
     // bandwidth from the MMA / epilogue warps; the in-place transform gains from 6 (13.2 -> 11.6 ms)
     const int threads3 = kSlab3Threads + (up ? 32 * kUpWarps : (in_scale ? 32 * kSlab3XformWarps : 0));
-    if (accum) {
-      NM_CHECK_ARG(bk == 64 && pn == 32 && !in_scale, "nm_conv3d_tc: split-K accumulation needs slab3<64, 32>");
-      if (up) conv3d_slab3_kernel<64, 32, true, true><<<grid, threads3, need, (cudaStream_t)stream>>>(q);
-      else conv3d_slab3_kernel<64, 32, false, true><<<grid, threads3, need, (cudaStream_t)stream>>>(q);
-    } else if (up) conv3d_slab3_kernel<64, 32, true><<<grid, threads3, need, (cudaStream_t)stream>>>(q);
-    else if (pn == 16) conv3d_slab3_kernel<64, 16><<<grid, threads3, need, (cudaStream_t)stream>>>(q);
-    else if (bk == 64) conv3d_slab3_kernel<64, 32><<<grid, threads3, need, (cudaStream_t)stream>>>(q);
-    else conv3d_slab3_kernel<32, 32><<<grid, threads3, need, (cudaStream_t)stream>>>(q);
+    NM_CHECK_ARG(!accum || (bk == 64 && pn == 32 && !in_scale), "nm_conv3d_tc: split-K accumulation needs slab3<64, 32>");
+    cudaLaunchConfig_t cfg = {};
+    cfg.blockDim = dim3(threads3);
+    cfg.dynamicSmemBytes = need;
+    cfg.stream = (cudaStream_t)stream;
+    cudaLaunchAttribute cluster;
+    cluster.id = cudaLaunchAttributeClusterDimension;
+    cluster.val.clusterDim.x = 2; cluster.val.clusterDim.y = 1; cluster.val.clusterDim.z = 1;
+    // persistent grid: one unit (CTA or CTA pair) per column and part, at most as many as can be resident
+    auto launch = [&](auto kern, bool pair) -> int {
+      if (!pair) {
+        cfg.gridDim = dim3(cols * parts < nm_num_sms() ? cols * parts : (nm_num_sms() / parts) * parts);
+        NM_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kern, q));
+        return NM_OK;
+      }
+      cfg.attrs = &cluster;
+      cfg.numAttrs = 1;
+      int max_pairs = 0;
+      NM_CHECK_ARG(max_resident_pairs((const void*)kern, cfg, &max_pairs) == cudaSuccess && max_pairs >= parts,
+                   "nm_conv3d_tc(slab3): no resident CTA pairs for %d parts", parts);
+      const int units = (cols / 2) * parts;
+      cfg.gridDim = dim3(2 * (units < max_pairs ? units : (max_pairs / parts) * parts));
+      NM_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kern, q));
+      return NM_OK;
+    };
+    int rc;
+    if (pl.pair) {
+      if (accum && up) rc = launch(conv3d_slab3_kernel<64, 32, true, true, true>, true);
+      else if (accum) rc = launch(conv3d_slab3_kernel<64, 32, false, true, true>, true);
+      else if (up) rc = launch(conv3d_slab3_kernel<64, 32, true, false, true>, true);
+      else if (pn == 64 && bk == 64) rc = launch(conv3d_slab3_kernel<64, 64, false, false, true>, true);
+      else if (pn == 64) rc = launch(conv3d_slab3_kernel<32, 64, false, false, true>, true);
+      else if (bk == 64) rc = launch(conv3d_slab3_kernel<64, 32, false, false, true>, true);
+      else rc = launch(conv3d_slab3_kernel<32, 32, false, false, true>, true);
+    } else {
+      if (accum && up) rc = launch(conv3d_slab3_kernel<64, 32, true, true>, false);
+      else if (accum) rc = launch(conv3d_slab3_kernel<64, 32, false, true>, false);
+      else if (up) rc = launch(conv3d_slab3_kernel<64, 32, true>, false);
+      else if (pn == 16) rc = launch(conv3d_slab3_kernel<64, 16>, false);
+      else if (bk == 64) rc = launch(conv3d_slab3_kernel<64, 32>, false);
+      else rc = launch(conv3d_slab3_kernel<32, 32>, false);
+    }
+    if (rc != NM_OK) return rc;
     NM_CHECK_LAUNCH("conv3d_slab3");
     return NM_OK;
   }
