@@ -208,6 +208,8 @@ struct WgPlan {
   size_t smem, ws_bytes;
 };
 
+constexpr long long kWgMaxUnits = 2048;  // units (256 voxels) one CTA accumulates at most
+
 bool wg_plan(int N, int D, int H, int W, int Cin, int Cout, WgPlan* q) {
   if (N <= 0 || D <= 0 || H <= 0 || Cin % 32 || Cout % 32 || Cin > 256 || Cout > 256 || Cin <= 0 || Cout <= 0) return false;
   if (!(W == 16 || W == 32 || W == 64 || W == 128)) return false;
@@ -234,8 +236,12 @@ bool wg_plan(int N, int D, int H, int W, int Cin, int Cout, WgPlan* q) {
   q->tmem_cols = cols;
   const long long units = (long long)N * D * (H / ht);
   if (units >= (1LL << 31)) return false;
+  // one wave of CTAs, repeated until no CTA sums more than kWgMaxUnits units: the tensor cores do not round the fp32
+  // accumulator to nearest, so a chain's error grows with its length (~1e-9 of the largest dW entry per voxel - 1.3e-3
+  // at the 64^3 layers of a 240-frame step with one wave); the splits are summed in fixed order by the reduce kernel
   long long splits = nm_num_sms() / q->groups;
   if (splits < 1) splits = 1;
+  splits *= (units + splits * kWgMaxUnits - 1) / (splits * kWgMaxUnits);
   if (splits > units) splits = units;
   q->splits = (int)splits;
   q->ws_bytes = (size_t)q->splits * q->groups * q->gm * 128 * q->ncols * sizeof(float);

@@ -584,13 +584,18 @@ def test_conv3d_weight_grad(ops, n, grid, cin, cout):
     assert rel_err(got24, ref[:, :24]) < 1e-3
 
 
-@pytest.mark.parametrize("n,grid,C,groups,leaky", [(2, 16, 32, 2, True), (3, 8, 64, 4, True), (1, 32, 32, 2, False),
-                                                  (2, 8, 128, 8, True), (3, 4, 48, 3, True), (2, 2, 72, 4, False),
-                                                  (2, 4, 48, 3, False), (5, 2, 72, 4, True)])
-def test_groupnorm_backward(ops, n, grid, C, groups, leaky):
+_GNB_CASES = [(2, 16, 32, 2, True), (3, 8, 64, 4, True), (1, 32, 32, 2, False), (2, 8, 128, 8, True), (3, 4, 48, 3, True),
+              (2, 2, 72, 4, False), (2, 4, 48, 3, False), (5, 2, 72, 4, True)]
+
+
+@pytest.mark.parametrize("n,grid,C,groups,leaky,stats",
+                         [pytest.param(*c, False, id="-".join(map(str, c))) for c in _GNB_CASES] +
+                         [pytest.param(*c, True, id="-".join(map(str, c)) + "-fwdstats") for c in _GNB_CASES])
+def test_groupnorm_backward(ops, n, grid, C, groups, leaky, stats):
     """dL/dx, dL/dgamma, dL/dbeta of LeakyReLU(GroupNorm(x)) against torch.autograd on the CPU (fp32 on the fp16-rounded
     tensors).  An element whose pre-activation sits within rounding of 0 may take the other LeakyReLU branch: the check
-    allows 1e-5 of the elements to differ and bounds the mean error."""
+    allows 1e-5 of the elements to differ and bounds the mean error.  `stats`: x is the output of a conv3d forward and
+    the backward takes the statistics that forward kept (`capture_gn_stats`), as the training step does."""
     g = torch.Generator().manual_seed(grid + C + groups)
     gn = torch.nn.GroupNorm(groups, C)
     with torch.no_grad():
@@ -598,12 +603,23 @@ def test_groupnorm_backward(ops, n, grid, C, groups, leaky):
         gn.bias.copy_(0.3 * torch.randn(C, generator=g))
     x = (torch.randn(n, C, grid, grid, grid, generator=g) * 1.5 + 0.3).half().float().requires_grad_(True)
     dz = torch.randn(n, C, grid, grid, grid, generator=g).half().float()
+    gn_cuda = torch.nn.GroupNorm(groups, C).cuda()
+    gn_cuda.load_state_dict(gn.state_dict())
+    st = None
+    if stats:
+        conv = torch.nn.Conv3d(C, C, 1)
+        with torch.no_grad():
+            conv.weight.copy_(torch.randn(conv.weight.shape, generator=g) * 1.5 / C ** 0.5)
+            conv.bias.fill_(0.3)
+        with ops.capture_gn_stats() as sink:
+            raw, _, _ = ops.conv3d(to_act(x.detach()), conv.cuda(), gn_cuda)
+        assert len(sink) == 1
+        st = tuple(sink[0])
+        x = from_act(raw).requires_grad_(True)
     y = gn(x)
     z = F.leaky_relu(y, 0.01) if leaky else y
     (z * dz).sum().backward()
-    gn_cuda = torch.nn.GroupNorm(groups, C).cuda()
-    gn_cuda.load_state_dict(gn.state_dict())
-    dx, dg, db, dxs = ops.groupnorm_backward(to_act(x.detach()), to_act(dz), gn_cuda, leaky=leaky)
+    dx, dg, db, dxs = ops.groupnorm_backward(to_act(x.detach()), to_act(dz), gn_cuda, leaky=leaky, stats=st)
     dx = from_act(dx)
     # dxsum = gradient of a bias added to x (the producing conv's bias): per-channel sum of dL/dx
     ref_bias = x.grad.sum(dim=(0, 2, 3, 4))
@@ -614,8 +630,9 @@ def test_groupnorm_backward(ops, n, grid, C, groups, leaky):
     assert float(diff.mean()) <= 3e-4 * scale
     assert float((dg.cpu() - gn.weight.grad).abs().max()) <= 2e-3 * float(gn.weight.grad.abs().max())
     assert float((db.cpu() - gn.bias.grad).abs().max()) <= 2e-3 * float(gn.bias.grad.abs().max())
-    dx2, dg2, db2, dxs2 = ops.groupnorm_backward(to_act(x.detach()), to_act(dz), gn_cuda, leaky=leaky)
+    dx2, dg2, db2, dxs2 = ops.groupnorm_backward(to_act(x.detach()), to_act(dz), gn_cuda, leaky=leaky, stats=st)
     assert torch.equal(from_act(dx2), dx) and torch.equal(dg2, dg) and torch.equal(db2, db) and torch.equal(dxs2, dxs)
     # out_scale multiplies the fp32 outputs only
-    _, dg3, db3, dxs3 = ops.groupnorm_backward(to_act(x.detach()), to_act(dz), gn_cuda, leaky=leaky, out_scale=0.25)
+    _, dg3, db3, dxs3 = ops.groupnorm_backward(to_act(x.detach()), to_act(dz), gn_cuda, leaky=leaky, out_scale=0.25,
+                                                stats=st)
     assert torch.allclose(dg3, dg * 0.25, rtol=1e-6, atol=0) and torch.allclose(db3, db * 0.25, rtol=1e-6, atol=0)
